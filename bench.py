@@ -11,6 +11,14 @@ all-reduce when N > 1 (weak scaling: every rank owns B sequences).  Workload at 
 
 Timing: W warm-up steps, then K steps each bracketed by CUDA events on the launching stream, an L2 flush (a 256 MiB
 memset, outside the events) between steps, barrier + synchronize on both sides, max over ranks.
+
+--dump-outputs DIR writes what the headline workload's last timed step returned to its caller as DIR/<name>.npy
+(float32; item ids as float64), at most 64 MiB in all, so that two builds can be compared output for output on the
+same seeded inputs.  Training: the step's loss and the weights after it (U and b whole; the rows of W_in and the
+columns of W_out of a fixed item sample, DIR/sample_items.npy).  Scoring (cfg5): the top-k ids and probabilities of
+the last step and p(true next item) at every step.  Gradient sums are accumulated with atomics, so two runs of the same
+build differ slightly: compare with a tolerance.  Measured on a B200 at 1000 W, cfg4, 20 steps: loss to 1.3e-7
+relative, W_out to 1.2e-5, b to 2.7e-4, U to 7.3e-4, W_in rows to 2.2e-3.
 """
 import argparse
 import json
@@ -27,6 +35,45 @@ sys.path.insert(0, ROOT)
 
 METRIC = "training sequences/sec"
 DEFAULT_CONFIG = "cfg4_gru256_1m"
+DUMP_SAMPLE_ITEMS = 8192
+DUMP_SAMPLE_BYTES = 48 << 20           # item-indexed weight slices; U and b add at most a few MiB on top
+
+
+def save_outputs(out_dir, arrays):
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64 if a.dtype.kind in "iu" else np.float32))
+
+
+def sample_items(V, n, seed=0):
+    """The items whose W_in rows / W_out columns --dump-outputs writes: the n/2 lowest ids (the most frequent under
+    the Zipf workload, so rows that every step updates) and a seeded uniform draw of n/2 from the rest."""
+    if V <= n:
+        return np.arange(V, dtype=np.int64)
+    rng = np.random.default_rng(seed)
+    tail = n // 2 + rng.choice(V - n // 2, size=n - n // 2, replace=False)
+    return np.sort(np.concatenate([np.arange(n // 2), tail])).astype(np.int64)
+
+
+def dump_training_outputs(hot, loss, out_dir, rank):
+    """The loss of the last timed step and the weights it left.  Under vocabulary parallelism every rank contributes
+    the sampled W_out columns of its own shard (one all-reduce of an (H, n) block), so every rank must call; rank 0
+    writes."""
+    import torch
+    n = min(DUMP_SAMPLE_ITEMS, max(1, DUMP_SAMPLE_BYTES // (4 * (hot.GH + hot.H))))
+    items = sample_items(hot.V_total, n)
+    idx = torch.from_numpy(items).to(hot.device)
+    own = (idx >= hot.v_lo) & (idx < hot.v_lo + hot.V)
+    cols = torch.zeros((hot.H, len(items)), dtype=torch.float32, device=hot.device)
+    cols[:, own] = hot.W_out.index_select(1, idx[own] - hot.v_lo)
+    if hot.vocab_parallel:
+        hot.comm.all_reduce_sum(cols)
+    arrays = {"loss": loss.detach().float().cpu().numpy(), "sample_items": items,
+              "W_in_rows": hot.W_in.index_select(0, idx).cpu().numpy(), "U": hot.U.cpu().numpy(),
+              "b": hot.b.cpu().numpy(), "W_out_cols": cols.cpu().numpy()}
+    if rank == 0:
+        save_outputs(out_dir, arrays)
 
 
 def load_peaks():
@@ -176,11 +223,13 @@ def cpu_oracle_step_fn(cfg, ids, tgt, seed):
     return step
 
 
-def time_cpu(cfg, steps, warmup, budget_s=25.0, sample_b=None):
-    """The oracle port timed on the host cores.  When the workload's batch fits (sample_b == B) the median step time
-    is the result.  Otherwise (cfg3 / cfg4: the (N, V) logits of the full batch do not fit host memory) the step time
-    is fitted as t(B) = a + b*B on two reduced batches -- the reference updates the whole (V, G*H) table densely
-    every step, a cost that does not shrink with the batch -- and the value is B_full / t(B_full)."""
+def time_cpu(cfg, steps, warmup, budget_s=None, sample_b=None):
+    """The oracle port timed on the host cores, `steps` steps at every timed batch size (fewer only when a budget_s in
+    seconds is given and runs out; `timed_steps` reports the counts).  When the workload's batch fits (sample_b == B)
+    the median step time is the result.  Otherwise (cfg3 / cfg4: the (N, V) logits of the full batch do not fit host
+    memory) the step time is fitted as t(B) = a + b*B on two reduced batches -- the reference updates the whole
+    (V, G*H) table densely every step, a cost that does not shrink with the batch -- and the value is
+    B_full / t(B_full)."""
     import torch
     from seq_recommendations_b200 import synthetic
     cores = os.cpu_count() or 1
@@ -199,7 +248,7 @@ def time_cpu(cfg, steps, warmup, budget_s=25.0, sample_b=None):
             t0 = time.perf_counter()
             step()
             times.append(time.perf_counter() - t0)
-            if time.perf_counter() - t_all > budget:
+            if budget is not None and time.perf_counter() - t_all > budget:
                 break
         return float(np.median(times)) * 1e3, len(times)
 
@@ -207,17 +256,19 @@ def time_cpu(cfg, steps, warmup, budget_s=25.0, sample_b=None):
         ms, n = median_step_ms(B_full, steps, warmup, budget_s)
         return dict(value=B_full / (ms / 1e3), unit="sequences/sec", cores=torch.get_num_threads(), kind="port",
                     sample="%d steps of fwd+bwd+clip+Adagrad on B=%d,T=%d,V=%d (oracle/keras_semantics.py, torch-CPU "
-                           "fp32, median)" % (n, B_full, cfg["T"], cfg["V"]), ms_per_step=ms)
+                           "fp32, median)" % (n, B_full, cfg["T"], cfg["V"]), ms_per_step=ms, timed_steps=[n])
     b1, b2 = max(1, sample_b // 2), max(2, sample_b // 2 * 3)
-    ms1, n1 = median_step_ms(b1, max(1, min(steps, 2)), min(warmup, 1), budget_s / 2)
-    ms2, n2 = median_step_ms(b2, max(1, min(steps, 2)), 0, budget_s / 2)
+    half = None if budget_s is None else budget_s / 2
+    ms1, n1 = median_step_ms(b1, steps, min(warmup, 1), half)
+    ms2, n2 = median_step_ms(b2, steps, 0, half)
     slope = max((ms2 - ms1) / (b2 - b1), 0.0)
     fixed = max(ms1 - slope * b1, 0.0)
     ms = fixed + slope * B_full
     return dict(value=B_full / (ms / 1e3), unit="sequences/sec", cores=torch.get_num_threads(), kind="port",
                 sample="fwd+bwd+clip+Adagrad (oracle/keras_semantics.py, torch-CPU fp32) at T=%d,V=%d on B=%d (%.0f ms, "
                        "%d steps) and B=%d (%.0f ms, %d steps); t(B) = %.0f ms + %.1f ms*B extrapolated to B=%d" % (
-                           cfg["T"], cfg["V"], b1, ms1, n1, b2, ms2, n2, fixed, slope, B_full), ms_per_step=ms)
+                           cfg["T"], cfg["V"], b1, ms1, n1, b2, ms2, n2, fixed, slope, B_full), ms_per_step=ms,
+                timed_steps=[n1, n2])
 
 
 def scan_info(cfg, B):
@@ -262,7 +313,7 @@ def run_reference(args, cfg, name):
         return
     world = max(1, args.gpus)
     sample_b = cpu_sample_batch(cfg, cfg["B"])
-    r = time_cpu(cfg, max(1, args.steps), max(1, min(args.warmup, 2)), budget_s=90.0, sample_b=sample_b)
+    r = time_cpu(cfg, args.steps, max(1, min(args.warmup, 2)), sample_b=sample_b)
     vp = (args.vocab_parallel == 1 or (args.vocab_parallel < 0 and name.startswith("cfg4"))) and world > 1 \
         and cfg["V"] % world == 0
     line = {
@@ -270,7 +321,7 @@ def run_reference(args, cfg, name):
         "steps": args.steps, "warmup": args.warmup, "ms_per_step": r["ms_per_step"], "higher_is_better": True,
         "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
         "config": config_dict(args, name, cfg, world, cfg["B"], vp, True),
-        "cpu_baseline": {k: r[k] for k in ("value", "unit", "cores", "kind", "sample")},
+        "cpu_baseline": {k: r[k] for k in ("value", "unit", "cores", "kind", "sample", "timed_steps")},
         "e2e": {"value": r["value"], "unit": "sequences/sec", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
         "gpu_launches": 0,
     }
@@ -278,9 +329,10 @@ def run_reference(args, cfg, name):
 
 
 # ------------------------------------------------------------------------------------------------------------------
-def run_scoring(args, cfg, name):
+def run_scoring(args, cfg, name, dump=None):
     """configs[4] (inference): sequences scored per second -- recurrent scan over T steps, then top-k next items of the
-    last step (`last`) or p(true next item) at every step (`all`).  One step = one batch of B sequences."""
+    last step (`last`) or p(true next item) at every step (`all`).  One step = one batch of B sequences.  dump: the
+    directory --dump-outputs writes the last timed step's results to."""
     import torch
     from seq_recommendations_b200 import _lib
     from seq_recommendations_b200.engine import HotPath
@@ -293,11 +345,12 @@ def run_scoring(args, cfg, name):
     pin_i, pin_t = torch.from_numpy(ids).pin_memory(), torch.from_numpy(tgt).pin_memory()
     dev_i, dev_t = pin_i.cuda(), pin_t.cuda()
     flush = torch.empty(256 << 20, dtype=torch.uint8, device="cuda")
-    out = {}
+    out, results = {}, {}
     clocks = ClockSampler(0)
     for mode in ("last", "all"):
-        fn = (lambda i, t: hot.topk_batch(i, k, last_step_only=True)[0]) if mode == "last" else (
-            lambda i, t: hot.target_prob_batch(i, t))
+        run = (lambda i, t: hot.topk_batch(i, k, last_step_only=True)) if mode == "last" else (
+            lambda i, t: (hot.target_prob_batch(i, t),))
+        fn = lambda i, t: run(i, t)[0]
         for _ in range(max(args.warmup, 3)):
             fn(dev_i, dev_t)
         torch.cuda.synchronize()
@@ -309,11 +362,14 @@ def run_scoring(args, cfg, name):
             flush.zero_()
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record()
-            fn(dev_i, dev_t)
+            last = run(dev_i, dev_t)
             e1.record()
             evs.append((e0, e1))
         torch.cuda.synchronize()
         launches = _lib.launch_count()
+        if dump:
+            names = ("top_items", "top_probs") if mode == "last" else ("target_probs",)
+            results.update((n, r.cpu().numpy()) for n, r in zip(names, last))
         ms = sum(a.elapsed_time(b) for a, b in evs) / args.steps
         e2e = []
         for _ in range(args.steps):
@@ -325,6 +381,8 @@ def run_scoring(args, cfg, name):
             e2e.append(time.perf_counter() - t0)
         out[mode] = dict(ms=ms, e2e_ms=float(np.mean(e2e)) * 1e3, launches=launches, d2h=int(r.numel() * r.element_size()))
     clk = clocks.stop()
+    if dump:
+        save_outputs(dump, results)
     peaks = load_peaks()
     G = 3 if cfg["cell"] == "GRU" else 4
     flops_all = B * T * (2 * G * H * H + 2 * H * V)
@@ -357,11 +415,12 @@ def run_scoring(args, cfg, name):
     return line
 
 
-def measure_training(args, name, cfg, comm, rank, local, steps, warmup, full=True, batch=None, vp=None):
+def measure_training(args, name, cfg, comm, rank, local, steps, warmup, full=True, batch=None, vp=None, dump=None):
     """One training workload on this process group: K timed steps with resident inputs (CUDA events, L2 flush between
     steps, barrier + synchronize on both sides, max over ranks), the same steps once more with an event at every phase
     boundary (per-kernel times), and the end-to-end leg from pinned host buffers.  `full` adds the reference-facing
-    plugin leg, the CPU baseline and the clock sampler.  Returns the JSON fields of this workload (rank 0) or None."""
+    plugin leg, the CPU baseline and the clock sampler; `dump` is the directory the last timed step's outputs go to.
+    Returns the JSON fields of this workload (rank 0) or None."""
     import torch
     from seq_recommendations_b200 import _lib, synthetic
     from seq_recommendations_b200.engine import HotPath
@@ -411,6 +470,8 @@ def measure_training(args, name, cfg, comm, rank, local, steps, warmup, full=Tru
     wall_s = time.perf_counter() - t_wall
     step_ms = sum(a.elapsed_time(b) for a, b in evs) / steps
     final_loss = float(loss.item())
+    if dump:
+        dump_training_outputs(hot, loss, dump, rank)
     hot.check_errors()
     # ---- the same K steps once more, launched eagerly with an event at every phase boundary: per-kernel times for the
     #      roofline and the launch count (a graph replay runs exactly these launches)
@@ -529,7 +590,8 @@ def measure_training(args, name, cfg, comm, rank, local, steps, warmup, full=Tru
         "e2e_plugin": plugin,
         "gpu_launches": launches,
         "roofline": roofline,
-        "cpu_baseline": ({k: cpu[k] for k in ("value", "unit", "cores", "kind", "sample")} if cpu else None),
+        "cpu_baseline": ({k: cpu[k] for k in ("value", "unit", "cores", "kind", "sample", "timed_steps")}
+                         if cpu else None),
         "phases_ms": per_step,
         "scan": scan_info(cfg, B),
         "wall_s_timed_region": wall_s,
@@ -657,7 +719,13 @@ def main():
     ap.add_argument("--tc", default="x3", choices=["x3", "bf16", "off"], help="logits GEMM mode (x3 = fp32-grade)")
     ap.add_argument("--vocab-parallel", type=int, default=-1,
                     help="1: column-shard W_out over the ranks (default for cfg4 when N > 1), 0: replicate")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the headline workload's last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of --impl b200")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     from seq_recommendations_b200 import synthetic
@@ -665,7 +733,7 @@ def main():
     if args.impl == "reference":
         return run_reference(args, cfg, args.config)
     if args.config.startswith("cfg5"):
-        print(json.dumps(run_scoring(args, cfg, args.config)))
+        print(json.dumps(run_scoring(args, cfg, args.config, dump=args.dump_outputs)))
         return
 
     import torch
@@ -679,7 +747,8 @@ def main():
     torch.cuda.set_device(local)
     comm = dist.init_from_env("nccl") if world > 1 else dist.Comm()
 
-    head = measure_training(args, args.config, cfg, comm, rank, local, args.steps, args.warmup, full=True)
+    head = measure_training(args, args.config, cfg, comm, rank, local, args.steps, args.warmup, full=True,
+                            dump=args.dump_outputs)
     extra = {}
     if world > 1:
         # strong scaling of the same workload: the GLOBAL batch stays cfg B, every rank takes B / N sequences
@@ -695,11 +764,10 @@ def main():
         # the other BASELINE configurations, same measurement (weak scaling at N > 1), brief: value, ms/step, e2e,
         # roofline, clocks each
         sub = {}
-        steps_sub = max(10, args.steps)
         for name in ("cfg1_msnbc_lstm100", "cfg2_reddit_gru128", "cfg3_lstm256_50k"):
             if name == args.config:
                 continue
-            r = measure_training(args, name, dict(synthetic.CONFIGS[name]), comm, rank, local, steps_sub, args.warmup,
+            r = measure_training(args, name, dict(synthetic.CONFIGS[name]), comm, rank, local, args.steps, args.warmup,
                                  full=False)
             if r is not None:
                 sub[name] = {k: r[k] for k in ("value", "unit", "ms_per_step", "config", "clocks", "phases_ms",

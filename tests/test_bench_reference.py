@@ -26,6 +26,21 @@ def test_reference_arm_prints_contract_line():
     assert d["cpu_baseline"]["kind"] == "port" and d["cpu_baseline"]["cores"] >= 1
     assert d["e2e"]["h2d_bytes_per_step"] == 0 and d["e2e"]["d2h_bytes_per_step"] == 0
     assert d["config"]["workload"] == "cfg1_msnbc_gru100"
+    assert d["steps"] == 2 and d["cpu_baseline"]["timed_steps"] == [2]
+
+
+def test_reference_timing_runs_exactly_the_requested_steps():
+    """Both the full-batch timing and the two-batch fit (taken when the logits of the full batch are too large) time
+    exactly `steps` steps at every batch size."""
+    import torch
+    import bench
+    cfg = dict(cell="GRU", act="tanh", V=50, H=8, T=6, B=64)
+    threads = torch.get_num_threads()                     # time_cpu takes every host core; later tests keep theirs
+    try:
+        for sample_b, want in ((64, [5]), (8, [5, 5])):
+            assert bench.time_cpu(cfg, 5, 1, sample_b=sample_b)["timed_steps"] == want
+    finally:
+        torch.set_num_threads(threads)
 
 
 def test_reference_arm_other_ranks_stay_silent():
