@@ -205,6 +205,30 @@ int seqrec_ce_tc_backward(const uint16_t* A_hi, const uint16_t* A_lo, const uint
                           int H, int Hk, int V, int Vp, int64_t Np, int v_begin, int v_end, int ldw,
                           int accumulate_dh, int x3, const float* b_out, float* db_out, const int32_t* n_tokens_dev,
                           void* stream);
+/* ---- rank of the true next item (Recall@k / MRR@k / NDCG@k without the logits) ------------------------------------
+ * For a token with target y >= 0 and logits z (bias included):
+ *     rank = 1 + #{v != y : z_v > z_y} + #{v < y : z_v == z_y}
+ * i.e. the 1-based position of y in the stable descending order, ties to the lower item id (the order of seqrec_topk:
+ * rank <= k <=> y is the top-k entry rank-1).  Pads (y < 0) have rank 0.
+ * seqrec_ce_tc_forward_rank is seqrec_ce_tc_forward (same operands, same ws_m / ws_s partials, bit for bit) that also
+ * counts, per token, the items of [v_begin, v_end) that precede y against the reference logit ref[n] (the exact fp32
+ * target logit of seqrec_target_logit; the tensor-core logits are compared with it, so the count is exact outside a
+ * band of the split-product error around z_y).  tgt holds GLOBAL item ids: item v of this launch is id_offset + v, so
+ * a vocabulary shard (id_offset = its first item) counts its items under the catalog-wide tie rule.
+ * Both rank entry points ADD their count to rank[n] with integer atomics (deterministic): the caller initialises
+ * rank[] -- 0 to receive the bare count (vocabulary shards, whose counts are then summed), or 1 on valid tokens and 0
+ * on pads to receive the 1-based rank directly (what the engine does; the +1 is never added by these kernels). */
+int seqrec_ce_tc_forward_rank(const uint16_t* A_hi, const uint16_t* A_lo, const uint16_t* Bt_hi, const uint16_t* Bt_lo,
+                              const float* b_out, float* ws_m, float* ws_s, const float* ref, const int32_t* tgt,
+                              int id_offset, int32_t* rank, int64_t n_tokens, int Hk, int V, int v_begin, int v_end,
+                              int x3, void* stream);
+/* the same count on the exact-fp32 SIMT logits of seqrec_ce_forward (hout (N,H), W_out (H, ldw), b_out may be NULL).
+ * ref NULL: z_y is computed with the same arithmetic as every z_v (an item whose W_out column equals the target's ties
+ * exactly and the tie rule decides); every target must then lie in this launch's items. */
+int seqrec_target_rank(const float* hout, const float* W_out, const float* b_out, const float* ref, const int32_t* tgt,
+                       int id_offset, int32_t* rank, int64_t n_tokens, int H, int V, int v_begin, int v_end, int ldw,
+                       void* stream);
+
 /* ---- K5 + K6 (dH half) from ONE logits pass (csrc/ce_tc.cu, TS_FUSED) -----------------------------------------
  * The softmax is evaluated against a per-token REFERENCE logit ref[n] (the exact fp32 target logit from
  * seqrec_target_logit) instead of the running row maximum -- exp(z - ref) needs no rescaling (ref is one of the row's
@@ -274,6 +298,9 @@ int seqrec_softmax_rows_stats(const float* Z, const int32_t* tgt, float* m, floa
 /* Z <- (exp(Z - m)/s - onehot(tgt)) * coef, in place (un-normalised, like K6; rows with coef == 0 become zeros) */
 int seqrec_softmax_rows_dlogit(float* Z, const int32_t* tgt, const float* m, const float* s, const float* coef,
                                int64_t n_tokens, int V, void* stream);
+/* rank[n] (overwritten) = the 1-based rank of tgt[n] in row n of materialised logits Z (n_rows, V), 0 for pads; the
+ * reference value is Z[n, tgt[n]] itself, so ties are exact (definition at seqrec_ce_tc_forward_rank) */
+int seqrec_rows_rank(const float* Z, const int32_t* tgt, int32_t* rank, int64_t n_rows, int V, void* stream);
 /* model.predict from materialised time-major logits (T,B,V): batch-major probabilities (B,T,V) */
 int seqrec_softmax_rows_probs(const float* Z, const float* m, const float* s, float* probs_btv, int T, int B, int V,
                               void* stream);
@@ -298,6 +325,12 @@ int seqrec_likelihood(const float* P, const int32_t* lengths, int64_t n_seqs, in
  * {sum, count} of the val parts (pre-zeroed). */
 int seqrec_likelihood_cut(const float* P, const int32_t* lengths, int64_t n_seqs, int T, int skip_first,
                           double train_percent, double* out4, void* stream);
+
+/* ranking metrics from per-token ranks (n, 0 = pad): for q < n_ks, out[3q..3q+2] += {#(rank <= ks[q]), sum 1/rank,
+ * sum 1/log2(rank+1)} over the ranks <= ks[q]; out[3 n_ks..3 n_ks+2] += the same sums over every rank > 0 (the first is
+ * the number of scored tokens, the second the uncut MRR sum).  ks: n_ks int32 on the device, each >= 1; out (3 n_ks + 3
+ * doubles) pre-zeroed.  Recall@k = out[3q] / n, MRR@k = out[3q+1] / n, NDCG@k = out[3q+2] / n. */
+int seqrec_rank_metrics(const int32_t* rank, int64_t n, const int32_t* ks, int n_ks, double* out, void* stream);
 
 /* ---- K8: global-norm clip + Adagrad (experiments_methods.py:41) -------------------------------------------------
  * sumsq[0] (double, pre-zeroed) += sum g^2 */

@@ -50,6 +50,8 @@ SIGNATURES = {
     "seqrec_ce_finalize_mean": [_p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _l, _i, _p, _p],
     "seqrec_ce_backward": [_p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _l, _i, _i, _i, _i, _i, _i, _p],
     "seqrec_ce_tc_forward": [_p, _p, _p, _p, _p, _p, _p, _l, _i, _i, _i, _i, _i, _p],
+    "seqrec_ce_tc_forward_rank": [_p] * 9 + [_i, _p, _l, _i, _i, _i, _i, _i, _p],
+    "seqrec_target_rank": [_p, _p, _p, _p, _p, _i, _p, _l, _i, _i, _i, _i, _i, _p],
     "seqrec_ce_tc_partials": [_l, _i, _i],
     "seqrec_ce_tc_backward": [_p] * 16 + [_l, _i, _i, _i, _i, _l, _i, _i, _i, _i, _i, _p, _p, _p, _p],
     "seqrec_ce_tc_fused": [_p] * 11 + [_l, _i, _i, _i, _i, _i, _i, _i, _p, _p],
@@ -65,11 +67,13 @@ SIGNATURES = {
     "seqrec_softmax_rows_stats": [_p, _p, _p, _p, _p, _l, _i, _p],
     "seqrec_softmax_rows_dlogit": [_p, _p, _p, _p, _p, _l, _i, _p],
     "seqrec_softmax_rows_probs": [_p, _p, _p, _p, _i, _i, _i, _p],
+    "seqrec_rows_rank": [_p, _p, _p, _l, _i, _p],
     "seqrec_gemm_nt": [_p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _p],
     "seqrec_colsum": [_p, _p, _l, _i, _i, _p],
     "seqrec_diag_constraint": [_p, _i, _i, _p],
     "seqrec_likelihood": [_p, _p, _l, _i, _i, _p, _p],
     "seqrec_likelihood_cut": [_p, _p, _l, _i, _i, ctypes.c_double, _p, _p],
+    "seqrec_rank_metrics": [_p, _l, _p, _i, _p, _p],
     "seqrec_sumsq": [_p, _l, _p, _p],
     "seqrec_sumsq_rows": [_p, _p, _p, _i, _i, _p, _p],
     "seqrec_adagrad": [_p, _p, _p, _l, _f, _f, _f, _p, _p, _p],

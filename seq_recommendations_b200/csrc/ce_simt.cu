@@ -78,6 +78,9 @@ __device__ __forceinline__ void merge_ms(float& m, float& s, float m2, float s2)
   m = mn;
 }
 
+static size_t ce_smem_bytes(int H, bool with_d) { return sizeof(float) * ((size_t)2 * H * CP + (with_d ? CT * CP : 0)); }
+static size_t ce_smem_bytes_rank(int H) { return sizeof(float) * ((size_t)2 * H * CP + CT); }
+
 // ---------------------------------------------------------------------------------------------------------------
 // forward: per-token running (max, sum-exp) over this CTA's item range, and the target logit
 __global__ void __launch_bounds__(CE_THREADS)
@@ -152,6 +155,101 @@ ce_forward_simt_kernel(const float* __restrict__ hout, const float* __restrict__
       ws_s[(int64_t)blockIdx.y * n_tokens + n] = s[i];
     }
   }
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// rank of the target: adds #{v in this CTA's item range, id != y : z_v > z_y  or  (z_v == z_y and id < y)} to rank[n]
+// (id = id_offset + v, y = tgt[n] a global id; pads, y < 0, add nothing).  The logits are the 4x4 micro-tiles of the
+// forward kernel above; without `ref` the reference z_y is the same fmaf chain over h plus the bias, so an item whose
+// W_out column equals the target's ties with it EXACTLY and the tie rule (lower id first) decides.
+__global__ void __launch_bounds__(CE_THREADS)
+target_rank_simt_kernel(const float* __restrict__ hout, const float* __restrict__ W_out,
+                        const float* __restrict__ b_out, const float* __restrict__ ref,
+                        const int32_t* __restrict__ tgt, int id_offset, int32_t* __restrict__ rank, int64_t n_tokens,
+                        int H, int v_begin, int v_end, int ldw, int items_per_split) {
+  extern __shared__ __align__(16) float smem[];
+  CeSmem sm = carve(smem, H);
+  float* zy_s = sm.W_s + (size_t)H * CP;                     // [CT] reference logits of the tile's tokens
+  const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4;
+  const int64_t n0 = (int64_t)blockIdx.x * CT;
+  const int vb = v_begin + blockIdx.y * items_per_split;
+  const int ve = min(v_end, vb + items_per_split);
+  load_token_tile(sm.A_s, hout, nullptr, n0, n_tokens, H);
+  __syncthreads();
+  if (tid < CT) {
+    const int64_t n = n0 + tid;
+    const int32_t y = n < n_tokens ? tgt[n] : -1;
+    float z = 0.f;
+    const int yl = y - id_offset;                          // column of W_out (ref == NULL: the target is local)
+    if (ref && y >= 0) {
+      z = ref[n];
+    } else if (y >= 0 && yl < ldw) {
+      for (int h = 0; h < H; ++h) z = fmaf(sm.A_s[h * CP + tid], W_out[(size_t)h * ldw + yl], z);
+      z = z + (b_out ? b_out[yl] : 0.f);
+    }
+    zy_s[tid] = z;
+  }
+  __syncthreads();
+  float rz[4];
+  int32_t tg[4], cnt[4];
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const int64_t n = n0 + ty * 4 + i;
+    tg[i] = n < n_tokens ? tgt[n] : -1;
+    rz[i] = zy_s[ty * 4 + i];
+    cnt[i] = 0;
+  }
+  for (int v0 = vb; v0 < ve; v0 += CT) {
+    __syncthreads();
+    load_item_tile(sm.W_s, W_out, ldw, v0, ve, H);
+    __syncthreads();
+    float acc[4][4];
+    logits_tile(acc, sm.A_s, sm.W_s, H, tx, ty);
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      const int v = v0 + tx * 4 + j;
+      if (v >= ve) continue;
+      const float b = b_out ? b_out[v] : 0.f;
+      const int id = id_offset + v;
+#pragma unroll
+      for (int i = 0; i < 4; ++i) {
+        const float z = acc[i][j] + b;
+        cnt[i] += tg[i] >= 0 && id != tg[i] && (z > rz[i] || (z == rz[i] && id < tg[i]));
+      }
+    }
+  }
+  // the 16 column-threads of a row are lanes differing in bits 0..3
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    int c = cnt[i];
+#pragma unroll
+    for (int o = 8; o > 0; o >>= 1) c += __shfl_xor_sync(0xffffffffu, c, o);
+    if (tx == 0 && c > 0) atomicAdd(rank + n0 + ty * 4 + i, c);
+  }
+}
+
+extern "C" int seqrec_target_rank(const float* hout, const float* W_out, const float* b_out, const float* ref,
+                                  const int32_t* tgt, int id_offset, int32_t* rank, int64_t n_tokens, int H, int V,
+                                  int v_begin, int v_end, int ldw, void* stream) {
+  SEQREC_ARG(hout && W_out && tgt && rank && n_tokens > 0 && H > 0 && V > 0, 1);
+  SEQREC_ARG(v_begin >= 0 && v_end <= V && v_begin < v_end && ldw >= v_end && id_offset >= 0, 2);
+  const size_t smem = ce_smem_bytes_rank(H);
+  if (smem > 227 * 1024) return -1010;
+  cudaError_t e = cudaFuncSetAttribute(target_rank_simt_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e != cudaSuccess) return -(int)e;
+  // enough CTAs to fill the SMs: the item range is split over blockIdx.y (each split adds its own count)
+  const int64_t n_tiles = (n_tokens + CT - 1) / CT;
+  const int v_tiles = ceil_div(v_end - v_begin, CT);
+  int splits = (int)((2 * SEQREC_NUM_SMS + n_tiles - 1) / n_tiles);
+  if (splits > v_tiles) splits = v_tiles;
+  if (splits < 1) splits = 1;
+  const int ips = ceil_div(v_tiles, splits) * CT;
+  splits = ceil_div(v_end - v_begin, ips);
+  dim3 grid((unsigned)n_tiles, splits);
+  target_rank_simt_kernel<<<grid, CE_THREADS, smem, as_stream(stream)>>>(hout, W_out, b_out, ref, tgt, id_offset, rank,
+                                                                         n_tokens, H, v_begin, v_end, ldw, ips);
+  SEQREC_CHECK_LAUNCH();
+  return 0;
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -457,7 +555,6 @@ predict_probs_simt_kernel(const float* __restrict__ hout, const float* __restric
 
 // ---------------------------------------------------------------------------------------------------------------
 // host side
-static size_t ce_smem_bytes(int H, bool with_d) { return sizeof(float) * ((size_t)2 * H * CP + (with_d ? CT * CP : 0)); }
 
 int ce_forward_simt(const float* hout, const float* hscale, const float* W_out, const float* b_out,
                     const int32_t* tgt, float* ws_m, float* ws_s, float* zy, int64_t n_tokens, int H, int V,

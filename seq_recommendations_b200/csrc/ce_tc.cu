@@ -314,12 +314,17 @@ using Walk = WaveShare::Walk;
 // outer = token tile (A resident per segment), inner = item tile (Bt streamed in 64-wide K blocks, NS stages).
 // Every segment writes one partial per 64-column half into ws[(slot*2 + half)][n], slot = position of the CTA among
 // the CTAs sharing that token tile; slots a token tile does not use are filled with (-inf, 0).
-template <int KB, int NS, bool X3, bool BIAS>
+// RANK: the same pass also counts, per token with target y = tgt[n] >= 0 (a GLOBAL item id; item v of this launch is
+// id_offset + v), the items that precede y in the stable descending order of the logits against the exact reference
+// logit ref[n]:  #{v != y : z_v > ref  or  (z_v == ref and id < y)}, added to rank[n] with one integer atomicAdd per
+// (segment, half) -- integer sums, so the result does not depend on the order of the CTAs.
+template <int KB, int NS, bool X3, bool BIAS, bool RANK>
 __global__ void __launch_bounds__(TCF_THREADS, 1)
 ce_tc_forward_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_constant__ CUtensorMap tmA_lo,
                      const __grid_constant__ CUtensorMap tmB_hi, const __grid_constant__ CUtensorMap tmB_lo,
                      const float* __restrict__ b_out, float* __restrict__ ws_m, float* __restrict__ ws_s,
-                     int64_t n_tokens, int v_begin, int v_end, int max_slots) {
+                     int64_t n_tokens, int v_begin, int v_end, int max_slots, const float* __restrict__ ref,
+                     const int32_t* __restrict__ tgt, int id_offset, int32_t* __restrict__ rank) {
   constexpr int NP = X3 ? 2 : 1;  // operand parts (hi, lo)
   extern __shared__ uint8_t smem_raw[];
   const uint32_t base = (ptx::smem_u32(smem_raw) + 1023u) & ~1023u;
@@ -446,11 +451,22 @@ ce_tc_forward_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_co
     const int half = (warp - 3) >> 2;            // which 64-column half of the tile this warp owns
     const int row = q * 32 + lane;
     float m = -INFINITY, s = 0.f;
+    float rz = 0.f, rz_below = 0.f;              // RANK: reference logit and the float just below it
+    int32_t ry = -1, cnt = 0;                    // RANK: target (global id, -1 = no rank) and the running count
     int tc = 0;
     for (int64_t w = sh.w0; w < sh.w1; ++w, ++tc) {
       const int buf = tc & 1;
       const int tt = sh.outer(w), vt = sh.inner(w);
-      if (sh.seg_first(w)) { m = -INFINITY; s = 0.f; }
+      if (sh.seg_first(w)) {
+        m = -INFINITY; s = 0.f;
+        if (RANK) {
+          const int64_t n = (int64_t)tt * BM + row;
+          ry = n < n_tokens ? tgt[n] : -1;
+          rz = ry >= 0 ? ref[n] : 0.f;
+          rz_below = nextafterf(rz, -INFINITY);
+          cnt = 0;
+        }
+      }
       const int vc0 = v_begin + vt * BN + half * 64;             // first item of this warp's columns
       ptx::mbar_wait(bar_tfull + 8 * buf, (tc >> 1) & 1);
       ptx::tc_fence_after_sync();
@@ -466,6 +482,25 @@ ce_tc_forward_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_co
           if (v < v_end) { if (BIAS) z[j] += __ldg(b_out + v); }
           else z[j] = -INFINITY;
         }
+      }
+      if (RANK && ry >= 0) {
+        // Columns wholly below the target id count z >= ref, i.e. z > (the float below ref); columns wholly above it
+        // count z > ref: ONE compare per logit.  Only the 64 columns that hold the target itself (64/V of the column
+        // blocks of a row) take the per-column tie rule, which also leaves the target out.  Columns past v_end are
+        // -inf and never count.
+        const int tl = ry - (id_offset + vc0);   // target column inside this warp's 64 (may lie outside)
+        int c4[4] = {0, 0, 0, 0};
+        if (tl < 0 || tl >= 64) {
+          const float thr = tl >= 64 ? rz_below : rz;
+#pragma unroll
+          for (int j = 0; j < 64; j += 4) {
+            c4[0] += z[j] > thr; c4[1] += z[j + 1] > thr; c4[2] += z[j + 2] > thr; c4[3] += z[j + 3] > thr;
+          }
+        } else {
+#pragma unroll
+          for (int j = 0; j < 64; ++j) c4[j & 3] += (j != tl) && (z[j] > rz || (z[j] == rz && j < tl));
+        }
+        cnt += (c4[0] + c4[1]) + (c4[2] + c4[3]);
       }
       float mx[4] = {-INFINITY, -INFINITY, -INFINITY, -INFINITY};
 #pragma unroll
@@ -491,6 +526,7 @@ ce_tc_forward_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_co
       if (sh.seg_last(w)) {
         // one partial of the vocabulary reduction per (slot, half), merged by seqrec_ce_finalize
         const int64_t n = (int64_t)tt * BM + row;
+        if (RANK && ry >= 0 && cnt > 0) atomicAdd(rank + n, cnt);
         if (n < n_tokens) {
           const int slot = (int)blockIdx.x - cta_of((int64_t)tt * n_vtiles, total);
           ws_m[((int64_t)slot * 2 + half) * n_tokens + n] = m;
@@ -1347,18 +1383,19 @@ int forward_slots(int64_t n_tokens, int v_begin, int v_end) {
   return (int)((n_inner + per - 1) / per + 1);
 }
 
-template <int KB, int NS, bool X3, bool BIAS>
+template <int KB, int NS, bool X3, bool BIAS, bool RANK>
 int launch_fwd(const CUtensorMap& a_hi, const CUtensorMap& a_lo, const CUtensorMap& b_hi, const CUtensorMap& b_lo,
                const float* b_out, float* ws_m, float* ws_s, int64_t n_tokens, int v_begin, int v_end,
-               cudaStream_t st) {
+               const float* ref, const int32_t* tgt, int id_offset, int32_t* rank, cudaStream_t st) {
   constexpr int NP = X3 ? 2 : 1;
   const size_t smem = 1024 + (size_t)NP * KB * TILE_B + (size_t)NS * NP * TILE_B + 256;
-  auto k = ce_tc_forward_kernel<KB, NS, X3, BIAS>;
+  auto k = ce_tc_forward_kernel<KB, NS, X3, BIAS, RANK>;
   cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return -(int)e;
   const int64_t total = ((n_tokens + BM - 1) / BM) * ceil_div(v_end - v_begin, BN);
   k<<<persistent_grid(total), TCF_THREADS, smem, st>>>(a_hi, a_lo, b_hi, b_lo, b_out, ws_m, ws_s, n_tokens, v_begin,
-                                                       v_end, forward_slots(n_tokens, v_begin, v_end));
+                                                       v_end, forward_slots(n_tokens, v_begin, v_end), ref, tgt,
+                                                       id_offset, rank);
   SEQREC_CHECK_LAUNCH();
   return 0;
 }
@@ -1525,12 +1562,16 @@ extern "C" int seqrec_ce_tc_partials(int64_t n_tokens, int v_begin, int v_end) {
   return 2 * forward_slots(n_tokens, v_begin, v_end);
 }
 
-extern "C" int seqrec_ce_tc_forward(const uint16_t* A_hi, const uint16_t* A_lo, const uint16_t* Bt_hi,
-                                    const uint16_t* Bt_lo, const float* b_out, float* ws_m, float* ws_s,
-                                    int64_t n_tokens, int Hk, int V, int v_begin, int v_end, int x3, void* stream) {
+namespace {
+template <bool RANK>
+int ce_tc_forward_impl(const uint16_t* A_hi, const uint16_t* A_lo, const uint16_t* Bt_hi, const uint16_t* Bt_lo,
+                       const float* b_out, float* ws_m, float* ws_s, const float* ref, const int32_t* tgt,
+                       int id_offset, int32_t* rank, int64_t n_tokens, int Hk, int V, int v_begin, int v_end, int x3,
+                       void* stream) {
   SEQREC_ARG(n_tokens > 0 && V > 0 && v_begin >= 0 && v_begin < v_end && v_end <= V, 1);
   SEQREC_ARG(Hk == 64 || Hk == 128 || Hk == 192 || Hk == 256, 2);
   SEQREC_ARG(A_hi && Bt_hi && (!x3 || (A_lo && Bt_lo)), 3);
+  SEQREC_ARG(!RANK || (ref && tgt && rank), 4);
   CUtensorMap a_hi, a_lo, b_hi, b_lo;
   int rc;
   if ((rc = make_tmap(&a_hi, A_hi, n_tokens, Hk, Hk, BM))) return rc;
@@ -1538,8 +1579,9 @@ extern "C" int seqrec_ce_tc_forward(const uint16_t* A_hi, const uint16_t* A_lo, 
   if ((rc = make_tmap(&a_lo, x3 ? A_lo : A_hi, n_tokens, Hk, Hk, BM))) return rc;
   if ((rc = make_tmap(&b_lo, x3 ? Bt_lo : Bt_hi, V, Hk, Hk, BN))) return rc;
   cudaStream_t st = as_stream(stream);
-#define FWD2(KB, NS, X3V, BV) \
-  return launch_fwd<KB, NS, X3V, BV>(a_hi, a_lo, b_hi, b_lo, b_out, ws_m, ws_s, n_tokens, v_begin, v_end, st)
+#define FWD2(KB, NS, X3V, BV)                                                                                      \
+  return launch_fwd<KB, NS, X3V, BV, RANK>(a_hi, a_lo, b_hi, b_lo, b_out, ws_m, ws_s, n_tokens, v_begin, v_end, ref, \
+                                           tgt, id_offset, rank, st)
 #define FWD(KB, NS)                                                                      \
   {                                                                                      \
     if (x3) { if (b_out) FWD2(KB, NS, true, true); else FWD2(KB, NS, true, false); }     \
@@ -1553,6 +1595,23 @@ extern "C" int seqrec_ce_tc_forward(const uint16_t* A_hi, const uint16_t* A_lo, 
   }
 #undef FWD2
 #undef FWD
+}
+}  // namespace
+
+extern "C" int seqrec_ce_tc_forward(const uint16_t* A_hi, const uint16_t* A_lo, const uint16_t* Bt_hi,
+                                    const uint16_t* Bt_lo, const float* b_out, float* ws_m, float* ws_s,
+                                    int64_t n_tokens, int Hk, int V, int v_begin, int v_end, int x3, void* stream) {
+  return ce_tc_forward_impl<false>(A_hi, A_lo, Bt_hi, Bt_lo, b_out, ws_m, ws_s, nullptr, nullptr, 0, nullptr, n_tokens,
+                                   Hk, V, v_begin, v_end, x3, stream);
+}
+
+extern "C" int seqrec_ce_tc_forward_rank(const uint16_t* A_hi, const uint16_t* A_lo, const uint16_t* Bt_hi,
+                                         const uint16_t* Bt_lo, const float* b_out, float* ws_m, float* ws_s,
+                                         const float* ref, const int32_t* tgt, int id_offset, int32_t* rank,
+                                         int64_t n_tokens, int Hk, int V, int v_begin, int v_end, int x3,
+                                         void* stream) {
+  return ce_tc_forward_impl<true>(A_hi, A_lo, Bt_hi, Bt_lo, b_out, ws_m, ws_s, ref, tgt, id_offset, rank, n_tokens, Hk,
+                                  V, v_begin, v_end, x3, stream);
 }
 
 extern "C" int seqrec_ce_tc_backward(const uint16_t* A_hi, const uint16_t* A_lo, const uint16_t* Ht_hi,

@@ -6,6 +6,7 @@
 //   seqrec_softmax_rows_stats    per-row (max, sum-exp) and target logit of materialised logits
 //   seqrec_softmax_rows_dlogit   Z <- (softmax(Z) - onehot(y)) * coef      in place (un-normalised, like K6)
 //   seqrec_softmax_rows_probs    (T,B,V) logits -> (B,T,V) probabilities   (model.predict)
+//   seqrec_rows_rank             1-based rank of the target in each row    (Recall@k / MRR@k / NDCG@k)
 //   seqrec_gemm_nt               C = A . B^T                               dH = dZ . W^T
 //   seqrec_colsum                out[c] += sum_r in[r,c]                   bias gradients
 //   seqrec_diag_constraint       W[skip + i, j] *= [i == j]                Keras constraint, applied after the update
@@ -113,6 +114,40 @@ extern "C" int seqrec_softmax_rows_probs(const float* Z, const float* m, const f
   int64_t blocks = ((int64_t)T * B * V + 255) / 256;
   if (blocks > SEQREC_NUM_SMS * 16) blocks = SEQREC_NUM_SMS * 16;
   softmax_rows_probs_kernel<<<(int)blocks, 256, 0, as_stream(stream)>>>(Z, m, s, probs_btv, T, B, V);
+  SEQREC_CHECK_LAUNCH();
+  return 0;
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// one warp per row: rank[n] = 1 + #{v != y : Z[n,v] > Z[n,y]  or  (Z[n,v] == Z[n,y] and v < y)}, 0 for pads (y < 0).
+// The reference value is read from the row itself, so ties are exact.
+__global__ void __launch_bounds__(256)
+rows_rank_kernel(const float* __restrict__ Z, const int32_t* __restrict__ tgt, int32_t* __restrict__ rank,
+                 int64_t n_rows, int V) {
+  const int lane = threadIdx.x & 31;
+  const int64_t n = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
+  if (n >= n_rows) return;
+  const int32_t y = tgt[n];
+  if (y < 0 || y >= V) {
+    if (lane == 0) rank[n] = 0;
+    return;
+  }
+  const float* row = Z + n * V;
+  const float zy = row[y];
+  int c = 0;
+  for (int v = lane; v < V; v += 32) {
+    const float z = row[v];
+    c += v != y && (z > zy || (z == zy && v < y));
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) c += __shfl_xor_sync(0xffffffffu, c, o);
+  if (lane == 0) rank[n] = 1 + c;
+}
+
+extern "C" int seqrec_rows_rank(const float* Z, const int32_t* tgt, int32_t* rank, int64_t n_rows, int V,
+                                void* stream) {
+  SEQREC_ARG(Z && tgt && rank && n_rows > 0 && V > 0, 1);
+  rows_rank_kernel<<<ceil_div(n_rows * 32, 256), 256, 0, as_stream(stream)>>>(Z, tgt, rank, n_rows, V);
   SEQREC_CHECK_LAUNCH();
   return 0;
 }

@@ -3,6 +3,7 @@
 // consumed by ValLossHistoryCut, model.py:106-112).  Input is the (n, T) matrix of per-step probabilities the scoring
 // kernels produce (right-aligned: a sequence of L steps fills the LAST L columns, like the left-padded batches); one
 // warp reduces one sequence, logs and sums in double.
+// Also the ranking metrics of next-item evaluation (Recall@k, MRR@k, NDCG@k) from the per-token rank of the target.
 #include "common.cuh"
 
 // window of row i: the last L columns (lengths given; L <= 0 or L > T means the whole row, like numpy's pred[-0:]),
@@ -77,6 +78,46 @@ extern "C" int seqrec_likelihood_cut(const float* P, const int32_t* lengths, int
   SEQREC_ARG(P && out4 && n_seqs > 0 && T > 0 && train_percent <= 1.0 && train_percent >= 0.0, 1);
   likelihood_cut_kernel<<<ceil_div(n_seqs * 32, 256), 256, 0, as_stream(stream)>>>(P, lengths, n_seqs, T, skip_first,
                                                                                    train_percent, out4);
+  SEQREC_CHECK_LAUNCH();
+  return 0;
+}
+
+// ranking metrics: for q < n_ks and k = ks[q], out[3q..3q+2] += {#(rank <= k), sum 1/rank, sum 1/log2(rank + 1)} over
+// the tokens with 0 < rank <= k; out[3 n_ks..3 n_ks+2] += the same sums without a cutoff (the first one is the number of
+// scored tokens).  rank 0 (pad) never counts.  Doubles throughout; one warp reduction and three atomics per warp and q.
+__global__ void __launch_bounds__(256)
+rank_metrics_kernel(const int32_t* __restrict__ rank, int64_t n, const int32_t* __restrict__ ks, int n_ks,
+                    double* __restrict__ out) {
+  const int lane = threadIdx.x & 31;
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  for (int q = 0; q <= n_ks; ++q) {
+    const int k = q < n_ks ? ks[q] : 0x7fffffff;
+    double hits = 0.0, rr = 0.0, dg = 0.0;
+    for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += stride) {
+      const int r = rank[i];
+      if (r > 0 && r <= k) {
+        hits += 1.0;
+        rr += 1.0 / (double)r;
+        dg += 1.0 / log2((double)r + 1.0);
+      }
+    }
+    hits = warp_sum_d(hits);
+    rr = warp_sum_d(rr);
+    dg = warp_sum_d(dg);
+    if (lane == 0 && hits > 0.0) {
+      atomicAdd(out + 3 * q, hits);
+      atomicAdd(out + 3 * q + 1, rr);
+      atomicAdd(out + 3 * q + 2, dg);
+    }
+  }
+}
+
+extern "C" int seqrec_rank_metrics(const int32_t* rank, int64_t n, const int32_t* ks, int n_ks, double* out,
+                                   void* stream) {
+  SEQREC_ARG(rank && ks && out && n > 0 && n_ks >= 1, 1);
+  int64_t blocks = (n + 255) / 256;
+  if (blocks > SEQREC_NUM_SMS * 4) blocks = SEQREC_NUM_SMS * 4;
+  rank_metrics_kernel<<<(int)blocks, 256, 0, as_stream(stream)>>>(rank, n, ks, n_ks, out);
   SEQREC_CHECK_LAUNCH();
   return 0;
 }

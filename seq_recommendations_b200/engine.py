@@ -1246,6 +1246,109 @@ class HotPath:
         self._forward_ce(w)
         return w.py.view(w.T, w.B).t().contiguous()
 
+    # ------------------------------------------------------------------------------------------------ target rank
+    def _stage_rows_operands(self, w):
+        """bf16 hi/lo operands of the tensor-core logits pass for the rows of w.hout (inference: no dropout factors)."""
+        self._stage_weight_operands()
+        call("seqrec_split_bf16", ptr(w.hout), None, ptr(w.A_hi), ptr(w.A_lo), w.N, self.H, self.Hk, 0, self.stream)
+        w.tc_operands_fresh = True
+
+    def _rank_rows_count(self, w, ref, rank, id_offset):
+        """Adds to rank[n] the number of THIS model's items that precede the target w.tgt[n] (a global id) in the stable
+        descending logit order, for the N rows of w.hout.  ref: per-token reference logit (None: the SIMT kernel computes
+        z_y itself with the arithmetic of every z_v).  The tensor-core pass also leaves the softmax partials of the rows
+        in w.ws_m / w.ws_s; returns their number of rows (0 on the SIMT kernel, which computes no statistics)."""
+        st = self.stream
+        if w.tc["fwd"]:
+            self._stage_rows_operands(w)
+            call("seqrec_ce_tc_forward_rank", ptr(w.A_hi), ptr(w.A_lo), ptr(self.Bt_hi), ptr(self.Bt_lo),
+                 ptr(self.b_out), ptr(w.ws_m), ptr(w.ws_s), ptr(ref), ptr(w.tgt), int(id_offset), ptr(rank), w.N,
+                 self.Hk, self.V, 0, self.V, 1 if self.tc_x3 else 0, st)
+            return w.tc["splits"]
+        call("seqrec_target_rank", ptr(w.hout), ptr(self.W_out), ptr(self.b_out), ptr(ref), ptr(w.tgt), int(id_offset),
+             ptr(rank), w.N, self.H, self.V, 0, self.V, self.V, st)
+        return 0
+
+    def _target_rank(self, w):
+        """(N,) int32 1-based rank of w.tgt in the logits of w.hout's rows, 0 on pads."""
+        st = self.stream
+        N = w.N
+        tg = w.tgt.view(-1)
+        if w.tc["panel"]:
+            # hidden sizes above 256: panels of materialised logits (never the (N,V) matrix), ranked row by row
+            rank = torch.empty(N, dtype=torch.int32, device=self.device)
+            nb_max = max(128, ((256 << 20) // (4 * self.V)) // 128 * 128)
+            rows = w.hout.view(N, self.H)
+            Z = torch.empty((min(nb_max, N), self.V), dtype=torch.float32, device=self.device)
+            for n0 in range(0, N, nb_max):
+                nb = min(nb_max, N - n0)
+                gemm(self, rows[n0:n0 + nb], self.W_out, Z[:nb], "nn", bias=self.b_out)
+                call("seqrec_rows_rank", ptr(Z[:nb]), ptr(tg[n0:n0 + nb]), ptr(rank[n0:n0 + nb]), nb, self.V, st)
+            return rank
+        rank = (tg >= 0).to(torch.int32)                 # the 1 of the 1-based rank; the kernels add the count
+        if w.tc["fwd"]:
+            # the exact fp32 target logit is the reference of the count: it must be complete BEFORE the pass (the
+            # statistics pass overlaps it, because there it is only needed by the finalize kernel)
+            call("seqrec_target_logit", ptr(w.hout), None, ptr(self.W_out), ptr(self.b_out), ptr(w.tgt), ptr(w.zy), N,
+                 self.H, self.V, None, None, st)
+            n_splits = self._rank_rows_count(w, w.zy, rank, 0)
+            # the pass wrote the softmax partials too: p(target) of the same rows comes for one finalize kernel
+            self._finalize_ce(w, w.ws_m, w.ws_s, n_splits)
+        else:
+            self._rank_rows_count(w, None, rank, 0)
+        return rank
+
+    def _rank_vp(self, w, last_step_only):
+        """Vocabulary-parallel rank: every rank counts, for all ranks' rows, the items of ITS shard that precede the
+        target (global ids, id_offset = the shard's first item) against the catalog-wide reference logit (computed on
+        the target's owner shard, summed over the shards); the integer counts are summed over the shards."""
+        comm = self.comm
+        if last_step_only:
+            rows, tg, nb, nt = w.hout[w.T - 1], w.tgt[w.T - 1], w.B, 1
+        else:
+            rows, tg, nb, nt = w.hout.view(w.N, self.H), w.tgt.view(-1), w.B, w.T
+        n_loc = rows.shape[0]
+        wg = self.work(nb * comm.world, nt)
+        wg.hout.view(wg.N, self.H).copy_(comm.all_gather_cat(rows.contiguous()))
+        wg.hscale = None
+        tgt_all = comm.all_gather_cat(tg.contiguous().view(-1))
+        local = (tgt_all >= self.v_lo) & (tgt_all < self.v_lo + self.V)
+        wg.tgt.view(-1).copy_(torch.where(local, tgt_all - self.v_lo, torch.full_like(tgt_all, -1)))
+        wg.zy.zero_()
+        call("seqrec_target_logit", ptr(wg.hout), None, ptr(self.W_out), ptr(self.b_out), ptr(wg.tgt), ptr(wg.zy),
+             wg.N, self.H, self.V, None, None, self.stream)
+        comm.all_reduce_sum(wg.zy)                        # only the owner shard contributes: the exact fp32 z_y
+        wg.tgt.view(-1).copy_(tgt_all)                    # global ids from here on
+        counts = torch.zeros(wg.N, dtype=torch.int32, device=self.device)
+        self._rank_rows_count(wg, wg.zy, counts, self.v_lo)
+        comm.all_reduce_sum(counts)
+        lo = comm.rank * n_loc
+        rank = counts[lo:lo + n_loc] + (tg.reshape(-1) >= 0).to(torch.int32)
+        return rank if last_step_only else rank.view(w.T, w.B).t().contiguous()
+
+    def target_rank_batch(self, ids, tgt, x_dense=None, last_step_only=False):
+        """Rank of the true next item per step: (B,T) int32 device tensor, or (B,) for the last step only.
+        rank = 1 + #{v != y : z_v > z_y} + #{v < y : z_v == z_y} (stable descending order, ties to the lower item id:
+        rank <= k <=> topk_batch holds y at index rank-1); pads have rank 0.  On the tensor cores the logits are compared
+        with the exact fp32 target logit, so the rank is exact outside the band of the split-product error around z_y,
+        and p(target) of the same rows is left in the work object's `py` by the same pass."""
+        B, T = (ids.shape if ids is not None else x_dense.shape[:2])
+        w = self.work(int(B), int(T))
+        self._stage(w, ids, tgt, x_dense)
+        self._forward_hidden(w, training=False)
+        if self.vocab_parallel:
+            return self._rank_vp(w, last_step_only)
+        if last_step_only:
+            # a (B, 1) problem over the rows hout[T-1], like topk_batch(last_step_only=True)
+            wl = self.work(int(B), 1)
+            if wl is not w:
+                wl.hout.copy_(w.hout[w.T - 1:w.T])
+                wl.mask.copy_(w.mask[w.T - 1:w.T])
+                wl.tgt.copy_(w.tgt[w.T - 1:w.T])
+            wl.hscale = None
+            return self._target_rank(wl)
+        return self._target_rank(w).view(w.T, w.B).t().contiguous()
+
     def _wide_logits(self, rows):
         """Hidden sizes above 256: logits of `rows` (n, H) materialised through the plain GEMM (tcgen05 when it fills
         tiles) with their per-row softmax statistics.  Scoring helper: n is a batch of rows, never the training set."""

@@ -12,7 +12,8 @@ Adagrad kernels are the ones of the hot path; the dense products run on the tcge
 experiment scripts for these variants drive one device).
 
 Same public methods as engine.HotPath (train_batch / loss_batch / grad_batch / predict_batch / target_prob_batch /
-topk_batch / hidden_batch, get_weight / set_weight, trainable, set_optimizer), so model._Net drives either.
+target_rank_batch / topk_batch / hidden_batch, get_weight / set_weight, trainable, set_optimizer), so model._Net drives
+either.
 """
 import ctypes
 
@@ -428,6 +429,17 @@ class DensePath:
         self._forward_logits(w, training=False)
         self._stats(w, train=False)
         return w.py.view(w.T, w.B).t().contiguous()
+
+    def target_rank_batch(self, ids, tgt, x_dense=None, last_step_only=False):
+        """Rank of the true next item in the materialised logits (stable descending order, ties to the lower item id;
+        pads 0): (B,T) int32 device tensor, or (B,) for the last step only."""
+        w = self.work(*self._shape(ids, x_dense))
+        self._stage(w, ids, tgt, x_dense)
+        self._forward_logits(w, training=False)
+        rank = torch.empty(w.N, dtype=torch.int32, device=self.device)
+        call("seqrec_rows_rank", ptr(w.Z), ptr(w.tgt), ptr(rank), w.N, self.V, self.stream)
+        rank = rank.view(w.T, w.B)
+        return rank[w.T - 1].contiguous() if last_step_only else rank.t().contiguous()
 
     def topk_batch(self, ids, k, last_step_only=True, x_dense=None):
         """Top-k next items from the materialised probabilities: stable descending order, ties to the lower item id."""

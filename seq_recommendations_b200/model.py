@@ -10,7 +10,8 @@ Scope (SURVEY §8): RNNFullModel -- the `y_to_z`-only form ("ytoz", experiments_
 RNNBaseline and NoRecurrenceModel; cells simpleRNN / LSTM (the reference's) and GRU (north-star).
 
 Additive (not in the reference): id-format batches ((N,T) / (N,T,1) integer arrays, pad < 0), `predict_target_prob`,
-`predict_topk`.
+`predict_topk`, `predict_target_rank` / `evaluate_ranking` (rank of the true next item; Recall@k, MRR@k, NDCG@k) and the
+`RankingMetrics` callback.
 """
 import os
 
@@ -23,6 +24,7 @@ from .engine import GATES, HotPath
 from .engine_dense import DensePath
 from .likelihood import compute_likelihood, compute_likelihood_cut  # noqa: F401  (utils.py:145-178, on the device)
 from .preprocessor import is_one_hot, to_id_batch
+from .ranking import check_ks, metrics_from_sums, rank_sums
 
 
 
@@ -53,6 +55,28 @@ class ValLossHistoryCut(cb.Callback):
         self.val_lossses.append(val_neg_ll)
         if logs is not None:
             logs["my_loss"] = val_neg_ll
+
+
+class RankingMetrics(cb.Callback):
+    """Additive: per-epoch ranking metrics of the true next item on the validation set, written into `logs` as
+    val_recall@k, val_mrr@k and val_ndcg@k -- placed before them in the callback list, EarlyStopping(monitor='val_mrr@20',
+    mode='max') and ModelCheckpoint see them.  The ranks come from the fused on-device scoring pass."""
+
+    def __init__(self, val_data, ks=(20,), last_step_only=False):
+        cb.Callback.__init__(self)
+        self.val_data = val_data
+        self.ks = check_ks(ks)
+        self.last_step_only = bool(last_step_only)
+        self.history = []
+
+    def on_epoch_end(self, epoch, logs=None):
+        res = self.model.evaluate_ranking(self.val_data[0], self.val_data[1], ks=self.ks,
+                                          last_step_only=self.last_step_only)
+        self.history.append(res)
+        if logs is not None:
+            for k in self.ks:
+                for name in ("recall", "mrr", "ndcg"):
+                    logs["val_%s@%d" % (name, k)] = float(res["%s@%d" % (name, k)])
 
 
 class BaseModel():
@@ -435,6 +459,35 @@ class _Net(object):
             op.append(b.cpu().numpy())
         return np.concatenate(oi, axis=0), np.concatenate(op, axis=0)
 
+    def _target_ranks(self, x, y, batch_size, last_step_only):
+        ids, xd = self._inputs(x)
+        tgt = to_id_batch(y)
+        out = []
+        for lo in range(0, len(tgt), batch_size):
+            hi = min(len(tgt), lo + batch_size)
+            i, d = self._slice(ids, xd, slice(lo, hi))
+            out.append(self.hot.target_rank_batch(i, tgt[lo:hi], d, last_step_only=last_step_only).clone())
+        out = torch.cat(out, dim=0)
+        self.hot.check_errors()
+        return out
+
+    def predict_target_rank(self, x, y, batch_size=1024, device=False):
+        """(N,T) int32 rank of the true next item among all items: 1 + the items with a higher logit + the lower-id
+        items with an equal one (so rank <= k <=> predict_topk holds it at index rank-1); pads give 0.
+        device=True returns the device tensor (ranking.ranking_metrics reduces it in HBM)."""
+        out = self._target_ranks(x, y, batch_size, False)
+        return out if device else out.cpu().numpy()
+
+    def evaluate_ranking(self, x, y, ks=(1, 5, 10, 20), last_step_only=False, batch_size=1024):
+        """Recall@k, MRR@k, NDCG@k for every k, the uncut MRR and n over the scored steps: every valid step, or with
+        last_step_only the last step of each non-empty sequence.  Data-parallel processes each score their own rows;
+        the sums are added over the processes."""
+        ks = check_ks(ks)
+        sums = rank_sums(self._target_ranks(x, y, batch_size, last_step_only), ks)
+        if self.hot.comm.enabled:
+            self.hot.comm.all_reduce_sum(sums)
+        return metrics_from_sums(sums, ks)
+
     def hidden_states(self, x, batch_size=1024):
         ids, xd = self._inputs(x)
         n = len(ids) if ids is not None else len(xd)
@@ -513,6 +566,12 @@ class BaseRNNModel(BaseModel):
 
     def predict_topk(self, x_test, k=20, last_step_only=True, batch_size=1024):
         return self.model.predict_topk(x_test, k=k, last_step_only=last_step_only, batch_size=batch_size)
+
+    def predict_target_rank(self, x_test, y_test, batch_size=1024):
+        return self.model.predict_target_rank(x_test, y_test, batch_size=batch_size)
+
+    def evaluate_ranking(self, x_test, y_test, ks=(1, 5, 10, 20), last_step_only=False, batch_size=1024):
+        return self.model.evaluate_ranking(x_test, y_test, ks=ks, last_step_only=last_step_only, batch_size=batch_size)
 
 
 def _glorot_uniform(rng, shape):
