@@ -96,6 +96,15 @@ int seqrec_gemm_tn_atomic(const float* A, const float* Bm, float* C, int M, int 
 int seqrec_rnn_forward(int cell, int act, float* xg, const float* U, const uint8_t* mask, float* hout, float* cst,
                        int T, int B, int H, void* stream);
 
+/* seqrec_rnn_forward from an initial state: h0 (B,H) and c0 (B,H, LSTM only) fp32, either may be NULL (= zeros;
+ * then the result is bit-identical to seqrec_rnn_forward).  The final state is hout[T-1] (and cst[T-1] for LSTM): every family
+ * (generic, register-resident and tensor-core scans) writes the held h and c on masked steps, so an all-pad row ends
+ * bit for bit where it started.  A scan continued from hout[T-1] / cst[T-1] of an earlier call gives bit-identical
+ * results to one call over both chunks at the same B (the per-step arithmetic does not depend on t).  c0 for a
+ * GRU / SimpleRNN cell is an argument error.  Inference only: there is no backward from a non-zero state. */
+int seqrec_rnn_forward_state(int cell, int act, float* xg, const float* U, const float* h0, const float* c0,
+                             const uint8_t* mask, float* hout, float* cst, int T, int B, int H, void* stream);
+
 /* ---- K4: recurrent scan backward (Theano scan gradient) ----------------------------------------------------------
  * dhout [T][B][H] = dLoss/dHout.  xg: in = saved gates, out = dxp (pre-activation gradients, in place).
  * U (H, G*H) and Ut = U^T (G*H, H).  For GRU, cst receives r*h_{t-1} (operand of dU's candidate block). */
@@ -126,6 +135,12 @@ int seqrec_rnn_tc_applicable(int cell, int H);
 int seqrec_rnn_tc_max_clusters(int cell, int H);
 int seqrec_rnn_tc_forward(int cell, int act, float* xg, const uint16_t* Ut_hi, const uint16_t* Ut_lo,
                           const uint8_t* mask, float* hout, float* cst, int T, int B, int H, void* stream);
+/* seqrec_rnn_tc_forward from an initial state, with the contract of seqrec_rnn_forward_state (h0 / c0 16-byte
+ * aligned).  Every CTA builds the h_{-1} operand from h0 with the same bf16 hi/lo split the scan applies to its own
+ * h_t, so continuing from hout[T-1] is bit-identical to one longer scan. */
+int seqrec_rnn_tc_forward_state(int cell, int act, float* xg, const uint16_t* Ut_hi, const uint16_t* Ut_lo,
+                                const float* h0, const float* c0, const uint8_t* mask, float* hout, float* cst,
+                                int T, int B, int H, void* stream);
 /* K4 on the tensor cores, same contract as seqrec_rnn_backward: each CTA forms the K-split partial product of ITS gate
  * columns with U[:, cols] (bf16 hi/lo, resident in shared memory) and dL/dh_{t-1} is reduce-scattered through
  * distributed shared memory.  U_hi / U_lo = seqrec_split_bf16(U, transpose = 0): (H, G*H), leading dimension G*H. */

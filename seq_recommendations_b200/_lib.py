@@ -32,6 +32,7 @@ SIGNATURES = {
     "seqrec_gemm_tc": [_p, _p, _p, _p, _p, _p, _l, _i, _i, _l, _l, _l, _i, _i, _p],
     "seqrec_gemm_tn_atomic": [_p, _p, _p, _i, _i, _i, _p],
     "seqrec_rnn_forward": [_i, _i, _p, _p, _p, _p, _p, _i, _i, _i, _p],
+    "seqrec_rnn_forward_state": [_i, _i, _p, _p, _p, _p, _p, _p, _p, _i, _i, _i, _p],
     "seqrec_rnn_backward": [_i, _i, _p, _p, _p, _p, _p, _p, _p, _i, _i, _i, _p],
     "seqrec_rnn_forward_rd": [_i, _i, _p, _p, _p, _p, _p, _p, _i, _i, _i, _p],
     "seqrec_rnn_backward_rd": [_i, _i, _p, _p, _p, _p, _p, _p, _p, _i, _i, _i, _p],
@@ -40,6 +41,7 @@ SIGNATURES = {
     "seqrec_rnn_tc_applicable": [_i, _i],
     "seqrec_rnn_tc_max_clusters": [_i, _i],
     "seqrec_rnn_tc_forward": [_i, _i, _p, _p, _p, _p, _p, _p, _i, _i, _i, _p],
+    "seqrec_rnn_tc_forward_state": [_i, _i, _p, _p, _p, _p, _p, _p, _p, _p, _i, _i, _i, _p],
     "seqrec_rnn_tc_backward": [_i, _i, _p, _p, _p, _p, _p, _p, _p, _i, _i, _i, _p],
     "seqrec_rnn_tc_debug_buffer": [_p],
     "seqrec_rnn_weight_grad": [_i, _p, _p, _p, _p, _p, _i, _i, _i, _p],

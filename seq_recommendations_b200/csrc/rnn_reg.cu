@@ -22,10 +22,11 @@ template <int CELL>
 struct Gates { static constexpr int G = (CELL == SEQREC_CELL_GRU) ? 3 : 1; };
 
 // ---------------------------------------------------------------------------------------------------------------
-template <int CELL, int ACT, int RB, int KPT>
+// INIT: h_{-1} is loaded from h0 (B,H) instead of zeros (rh_s is recomputed every step)
+template <int CELL, int ACT, int RB, int KPT, bool INIT>
 __global__ void __launch_bounds__(KS * 128, 1)
 rnn_forward_reg_kernel(float* __restrict__ xg, const float* __restrict__ U, const uint8_t* __restrict__ mask,
-                       float* __restrict__ hout, int T, int B, int H) {
+                       float* __restrict__ hout, int T, int B, int H, const float* __restrict__ h0) {
   constexpr int G = Gates<CELL>::G;
   constexpr int G1 = (CELL == SEQREC_CELL_GRU) ? 2 : 1;   // gates whose recurrent product uses h_{t-1} itself
   constexpr int KP = KS * KPT;                 // padded hidden size seen by the dot products
@@ -55,7 +56,14 @@ rnn_forward_reg_kernel(float* __restrict__ xg, const float* __restrict__ U, cons
       const int k = s * KPT + i;
       u[g][i] = (k < H && c < H) ? U[(size_t)k * GH + g * H + c] : 0.f;
     }
-  for (int i = tid; i < 2 * RB * KP; i += blockDim.x) h_s[i] = 0.f;   // h_s and rh_s
+  if constexpr (INIT) {
+    for (int i = tid; i < 2 * RB * KP; i += blockDim.x) {
+      const int r = i / KP, k = i - r * KP;    // r >= RB: rh_s
+      h_s[i] = (r < RB && k < H && b0 + r < B) ? h0[(size_t)(b0 + r) * H + k] : 0.f;
+    }
+  } else {
+    for (int i = tid; i < 2 * RB * KP; i += blockDim.x) h_s[i] = 0.f;   // h_s and rh_s
+  }
 
   auto prefetch_x = [&](int t) {               // owners: xp of step t -> x_s[t & 1]
     if (owner && t < T) {
@@ -324,7 +332,7 @@ rnn_backward_reg_kernel(float* __restrict__ xg, const float* __restrict__ U, con
 
 template <int CELL, int ACT, int RB, int KPT>
 int launch_pair(bool fwd, float* xg, const float* U, const uint8_t* mask, float* hout, float* cst, const float* dhout,
-                int T, int B, int H, cudaStream_t st) {
+                int T, int B, int H, cudaStream_t st, const float* h0) {
   constexpr int G = Gates<CELL>::G;
   constexpr int NI = (CELL == SEQREC_CELL_GRU) ? 5 : 2;
   const int CG = (H + 31) / 32 * 32;
@@ -334,12 +342,12 @@ int launch_pair(bool fwd, float* xg, const float* U, const uint8_t* mask, float*
   if (fwd) {
     const size_t smem = sizeof(float) * (size_t)(2 * RB * KP + KS * RB * G * CG + 2 * RB * G * CG + RB * 2 * CG) +
                         sizeof(int) * 2 * RB;
-    auto k = rnn_forward_reg_kernel<CELL, ACT, RB, KPT>;
+    auto k = h0 ? rnn_forward_reg_kernel<CELL, ACT, RB, KPT, true> : rnn_forward_reg_kernel<CELL, ACT, RB, KPT, false>;
     if (smem > 48 * 1024) {
       cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
       if (e != cudaSuccess) return -(int)e;
     }
-    k<<<grid, threads, smem, st>>>(xg, U, mask, hout, T, B, H);
+    k<<<grid, threads, smem, st>>>(xg, U, mask, hout, T, B, H, h0);
   } else {
     const size_t smem_step = sizeof(float) * (size_t)(G * RB * KP + KS * RB * CG + 2 * RB * NI * CG + 2 * RB * CG) +
                              sizeof(int) * 2 * RB;
@@ -358,36 +366,36 @@ int launch_pair(bool fwd, float* xg, const float* U, const uint8_t* mask, float*
 
 template <int CELL, int ACT, int RB>
 int dispatch_kpt(bool fwd, float* xg, const float* U, const uint8_t* mask, float* hout, float* cst,
-                 const float* dhout, int T, int B, int H, cudaStream_t st) {
+                 const float* dhout, int T, int B, int H, cudaStream_t st, const float* h0) {
   const int kpt = (((H + KS - 1) / KS) + 7) / 8 * 8;   // K-slice length, multiple of 8
   switch (kpt) {
-    case 8: return launch_pair<CELL, ACT, RB, 8>(fwd, xg, U, mask, hout, cst, dhout, T, B, H, st);
-    case 16: return launch_pair<CELL, ACT, RB, 16>(fwd, xg, U, mask, hout, cst, dhout, T, B, H, st);
-    case 24: return launch_pair<CELL, ACT, RB, 24>(fwd, xg, U, mask, hout, cst, dhout, T, B, H, st);
-    default: return launch_pair<CELL, ACT, RB, 32>(fwd, xg, U, mask, hout, cst, dhout, T, B, H, st);
+    case 8: return launch_pair<CELL, ACT, RB, 8>(fwd, xg, U, mask, hout, cst, dhout, T, B, H, st, h0);
+    case 16: return launch_pair<CELL, ACT, RB, 16>(fwd, xg, U, mask, hout, cst, dhout, T, B, H, st, h0);
+    case 24: return launch_pair<CELL, ACT, RB, 24>(fwd, xg, U, mask, hout, cst, dhout, T, B, H, st, h0);
+    default: return launch_pair<CELL, ACT, RB, 32>(fwd, xg, U, mask, hout, cst, dhout, T, B, H, st, h0);
   }
 }
 
 template <int CELL, int ACT>
 int dispatch_rb(int rb, bool fwd, float* xg, const float* U, const uint8_t* mask, float* hout, float* cst,
-                const float* dhout, int T, int B, int H, cudaStream_t st) {
+                const float* dhout, int T, int B, int H, cudaStream_t st, const float* h0) {
   switch (rb) {
-    case 1: return dispatch_kpt<CELL, ACT, 1>(fwd, xg, U, mask, hout, cst, dhout, T, B, H, st);
-    case 2: return dispatch_kpt<CELL, ACT, 2>(fwd, xg, U, mask, hout, cst, dhout, T, B, H, st);
-    default: return dispatch_kpt<CELL, ACT, 4>(fwd, xg, U, mask, hout, cst, dhout, T, B, H, st);
+    case 1: return dispatch_kpt<CELL, ACT, 1>(fwd, xg, U, mask, hout, cst, dhout, T, B, H, st, h0);
+    case 2: return dispatch_kpt<CELL, ACT, 2>(fwd, xg, U, mask, hout, cst, dhout, T, B, H, st, h0);
+    default: return dispatch_kpt<CELL, ACT, 4>(fwd, xg, U, mask, hout, cst, dhout, T, B, H, st, h0);
   }
 }
 
 template <int CELL>
 int dispatch_act(int act, int rb, bool fwd, float* xg, const float* U, const uint8_t* mask, float* hout, float* cst,
-                 const float* dhout, int T, int B, int H, cudaStream_t st) {
+                 const float* dhout, int T, int B, int H, cudaStream_t st, const float* h0) {
   switch (act) {
     case SEQREC_ACT_RELU:
-      return dispatch_rb<CELL, SEQREC_ACT_RELU>(rb, fwd, xg, U, mask, hout, cst, dhout, T, B, H, st);
+      return dispatch_rb<CELL, SEQREC_ACT_RELU>(rb, fwd, xg, U, mask, hout, cst, dhout, T, B, H, st, h0);
     case SEQREC_ACT_TANH:
-      return dispatch_rb<CELL, SEQREC_ACT_TANH>(rb, fwd, xg, U, mask, hout, cst, dhout, T, B, H, st);
+      return dispatch_rb<CELL, SEQREC_ACT_TANH>(rb, fwd, xg, U, mask, hout, cst, dhout, T, B, H, st, h0);
     case SEQREC_ACT_LINEAR:
-      return dispatch_rb<CELL, SEQREC_ACT_LINEAR>(rb, fwd, xg, U, mask, hout, cst, dhout, T, B, H, st);
+      return dispatch_rb<CELL, SEQREC_ACT_LINEAR>(rb, fwd, xg, U, mask, hout, cst, dhout, T, B, H, st, h0);
     default: return -1002;
   }
 }
@@ -397,7 +405,7 @@ int dispatch_act(int act, int rb, bool fwd, float* xg, const float* U, const uin
 // LSTM variant (rnn_reg_lstm.cu)
 bool lstm_reg_applicable(int H);
 int lstm_reg_launch(int act, int rb, bool fwd, float* xg, const float* U, const uint8_t* mask, float* hout, float* cst,
-                    const float* dhout, int T, int B, int H, cudaStream_t st);
+                    const float* dhout, int T, int B, int H, cudaStream_t st, const float* h0, const float* c0);
 
 // Is the register-resident scan applicable?  (GRU / SimpleRNN with H <= 128, LSTM with H <= 100)
 bool rnn_reg_applicable(int cell, int H) {
@@ -406,11 +414,13 @@ bool rnn_reg_applicable(int cell, int H) {
 }
 
 // rb: batch rows per CTA (1, 2 or 4).  U is the untransposed recurrent kernel (H, G*H) for BOTH directions.
+// h0 / c0 (forward only): initial state, NULL = zeros; c0 is read by the LSTM only.
 int rnn_reg_launch(int cell, int act, int rb, bool fwd, float* xg, const float* U, const uint8_t* mask, float* hout,
-                   float* cst, const float* dhout, int T, int B, int H, cudaStream_t st) {
+                   float* cst, const float* dhout, int T, int B, int H, cudaStream_t st, const float* h0,
+                   const float* c0) {
   if (cell == SEQREC_CELL_LSTM)
-    return lstm_reg_launch(act, rb > 2 ? 2 : rb, fwd, xg, U, mask, hout, cst, dhout, T, B, H, st);
+    return lstm_reg_launch(act, rb > 2 ? 2 : rb, fwd, xg, U, mask, hout, cst, dhout, T, B, H, st, h0, c0);
   if (cell == SEQREC_CELL_GRU)
-    return dispatch_act<SEQREC_CELL_GRU>(act, rb, fwd, xg, U, mask, hout, cst, dhout, T, B, H, st);
-  return dispatch_act<SEQREC_CELL_SIMPLE>(act, rb, fwd, xg, U, mask, hout, cst, dhout, T, B, H, st);
+    return dispatch_act<SEQREC_CELL_GRU>(act, rb, fwd, xg, U, mask, hout, cst, dhout, T, B, H, st, h0);
+  return dispatch_act<SEQREC_CELL_SIMPLE>(act, rb, fwd, xg, U, mask, hout, cst, dhout, T, B, H, st, h0);
 }

@@ -27,10 +27,12 @@ struct Shape {
 };
 
 // ---------------------------------------------------------------------------------------------------------------
-template <int ACT, int RB, int KS, int KPT>
+// INIT: h_{-1} and c_{-1} are loaded from h0 and c0 (B,H) instead of zeros; a NULL pointer stands for zeros
+template <int ACT, int RB, int KS, int KPT, bool INIT>
 __global__ void __launch_bounds__(Shape<KS, KPT>::MAXT, 1)
 lstm_forward_reg_kernel(float* __restrict__ xg, const float* __restrict__ U, const uint8_t* __restrict__ mask,
-                        float* __restrict__ hout, float* __restrict__ cst, int T, int B, int H, int CG) {
+                        float* __restrict__ hout, float* __restrict__ cst, int T, int B, int H, int CG,
+                        const float* __restrict__ h0, const float* __restrict__ c0) {
   static_assert(RB <= KS, "one owner thread per (row, unit) needs RB <= KS");
   constexpr int KP = Shape<KS, KPT>::KP;
   const int GH = G * H;
@@ -52,7 +54,14 @@ lstm_forward_reg_kernel(float* __restrict__ xg, const float* __restrict__ U, con
       const int k = s * KPT + i;
       u[g][i] = (k < H && c < H && s < KS) ? U[(size_t)k * GH + g * H + c] : 0.f;
     }
-  for (int i = tid; i < RB * KP; i += blockDim.x) h_s[i] = 0.f;
+  if constexpr (INIT) {
+    for (int i = tid; i < RB * KP; i += blockDim.x) {
+      const int q = i / KP, k = i - q * KP;
+      h_s[i] = (h0 && k < H && b0 + q < B) ? h0[(size_t)(b0 + q) * H + k] : 0.f;
+    }
+  } else {
+    for (int i = tid; i < RB * KP; i += blockDim.x) h_s[i] = 0.f;
+  }
 
   auto prefetch_x = [&](int t) {
     if (owner && t < T) {
@@ -69,6 +78,10 @@ lstm_forward_reg_kernel(float* __restrict__ xg, const float* __restrict__ U, con
     m1 = (1 < T) ? (mask[(size_t)B + b0 + r] != 0) : false;
   }
   float hp = 0.f, cp = 0.f;                     // owner: h_{t-1}, c_{t-1} of (row r, unit c)
+  if (INIT && owner) {
+    if (h0) hp = h0[(size_t)(b0 + r) * H + c];
+    if (c0) cp = c0[(size_t)(b0 + r) * H + c];
+  }
   prefetch_x(0);
   __syncthreads();
 
@@ -253,19 +266,20 @@ lstm_backward_reg_kernel(float* __restrict__ xg, const float* __restrict__ U, co
 
 template <int ACT, int RB, int KS, int KPT>
 int launch_lstm(bool fwd, float* xg, const float* U, const uint8_t* mask, float* hout, float* cst, const float* dhout,
-                int T, int B, int H, cudaStream_t st) {
+                int T, int B, int H, cudaStream_t st, const float* h0, const float* c0) {
   constexpr int KP = Shape<KS, KPT>::KP;
   const int CG = (H + 3) / 4 * 4;
   const int threads = (KS * CG + 31) / 32 * 32;
   const int grid = ceil_div(B, RB);
   if (fwd) {
     const size_t smem = sizeof(float) * (size_t)(RB * KP + KS * RB * G * CG + 2 * RB * G * CG);
-    auto k = lstm_forward_reg_kernel<ACT, RB, KS, KPT>;
+    auto k = (h0 || c0) ? lstm_forward_reg_kernel<ACT, RB, KS, KPT, true>
+                        : lstm_forward_reg_kernel<ACT, RB, KS, KPT, false>;
     if (smem > 48 * 1024) {
       cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
       if (e != cudaSuccess) return -(int)e;
     }
-    k<<<grid, threads, smem, st>>>(xg, U, mask, hout, cst, T, B, H, CG);
+    k<<<grid, threads, smem, st>>>(xg, U, mask, hout, cst, T, B, H, CG, h0, c0);
   } else {
     const size_t smem_step = sizeof(float) * (size_t)(G * RB * KP + KS * RB * CG + 2 * RB * 7 * CG);
     const size_t smem_load = sizeof(float) * (size_t)H * (H + 1);
@@ -283,19 +297,19 @@ int launch_lstm(bool fwd, float* xg, const float* U, const uint8_t* mask, float*
 
 template <int ACT, int RB>
 int dispatch_shape(bool fwd, float* xg, const float* U, const uint8_t* mask, float* hout, float* cst,
-                   const float* dhout, int T, int B, int H, cudaStream_t st) {
+                   const float* dhout, int T, int B, int H, cudaStream_t st, const float* h0, const float* c0) {
   // (KS, KPT): KS*KPT >= H, KPT a multiple of 4 (float4 reads of the K-slice), 4*KPT registers of U per thread
-  if (H <= 32) return launch_lstm<ACT, RB, 4, 8>(fwd, xg, U, mask, hout, cst, dhout, T, B, H, st);
-  if (H <= 64) return launch_lstm<ACT, RB, 4, 16>(fwd, xg, U, mask, hout, cst, dhout, T, B, H, st);
-  if (H <= 80) return launch_lstm<ACT, RB, 4, 20>(fwd, xg, U, mask, hout, cst, dhout, T, B, H, st);
-  return launch_lstm<ACT, RB, 5, 20>(fwd, xg, U, mask, hout, cst, dhout, T, B, H, st);
+  if (H <= 32) return launch_lstm<ACT, RB, 4, 8>(fwd, xg, U, mask, hout, cst, dhout, T, B, H, st, h0, c0);
+  if (H <= 64) return launch_lstm<ACT, RB, 4, 16>(fwd, xg, U, mask, hout, cst, dhout, T, B, H, st, h0, c0);
+  if (H <= 80) return launch_lstm<ACT, RB, 4, 20>(fwd, xg, U, mask, hout, cst, dhout, T, B, H, st, h0, c0);
+  return launch_lstm<ACT, RB, 5, 20>(fwd, xg, U, mask, hout, cst, dhout, T, B, H, st, h0, c0);
 }
 
 template <int ACT>
 int dispatch_rb(int rb, bool fwd, float* xg, const float* U, const uint8_t* mask, float* hout, float* cst,
-                const float* dhout, int T, int B, int H, cudaStream_t st) {
-  if (rb <= 1) return dispatch_shape<ACT, 1>(fwd, xg, U, mask, hout, cst, dhout, T, B, H, st);
-  return dispatch_shape<ACT, 2>(fwd, xg, U, mask, hout, cst, dhout, T, B, H, st);
+                const float* dhout, int T, int B, int H, cudaStream_t st, const float* h0, const float* c0) {
+  if (rb <= 1) return dispatch_shape<ACT, 1>(fwd, xg, U, mask, hout, cst, dhout, T, B, H, st, h0, c0);
+  return dispatch_shape<ACT, 2>(fwd, xg, U, mask, hout, cst, dhout, T, B, H, st, h0, c0);
 }
 
 }  // namespace
@@ -304,14 +318,14 @@ bool lstm_reg_applicable(int H) { return H <= 100; }
 
 // rb: batch rows per CTA (clamped to 2).  U is the untransposed recurrent kernel (H, 4H) for BOTH directions.
 int lstm_reg_launch(int act, int rb, bool fwd, float* xg, const float* U, const uint8_t* mask, float* hout, float* cst,
-                    const float* dhout, int T, int B, int H, cudaStream_t st) {
+                    const float* dhout, int T, int B, int H, cudaStream_t st, const float* h0, const float* c0) {
   switch (act) {
     case SEQREC_ACT_RELU:
-      return dispatch_rb<SEQREC_ACT_RELU>(rb, fwd, xg, U, mask, hout, cst, dhout, T, B, H, st);
+      return dispatch_rb<SEQREC_ACT_RELU>(rb, fwd, xg, U, mask, hout, cst, dhout, T, B, H, st, h0, c0);
     case SEQREC_ACT_TANH:
-      return dispatch_rb<SEQREC_ACT_TANH>(rb, fwd, xg, U, mask, hout, cst, dhout, T, B, H, st);
+      return dispatch_rb<SEQREC_ACT_TANH>(rb, fwd, xg, U, mask, hout, cst, dhout, T, B, H, st, h0, c0);
     case SEQREC_ACT_LINEAR:
-      return dispatch_rb<SEQREC_ACT_LINEAR>(rb, fwd, xg, U, mask, hout, cst, dhout, T, B, H, st);
+      return dispatch_rb<SEQREC_ACT_LINEAR>(rb, fwd, xg, U, mask, hout, cst, dhout, T, B, H, st, h0, c0);
     default: return -1002;
   }
 }

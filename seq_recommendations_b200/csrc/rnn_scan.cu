@@ -49,11 +49,13 @@ __host__ __device__ inline int round_up4(int x) { return (x + 3) & ~3; }
 // RD = recurrent dropout (Keras `recurrent_dropout`, model.py:346,351): G inverted-dropout masks rm[g] (B,H), constant
 // over time, multiply h_{t-1} before the recurrent product of gate block g (GRU candidate: r * h_{t-1} * rm[2]).  The
 // masked copies hm[g] = h * rm[g] are kept in shared memory next to h.
-template <int CELL, int ACT, int RB, bool USMEM, bool RD>
+// INIT: the scan starts from h0 (B,H) and, for LSTM, c0 (B,H) instead of zeros; a NULL pointer stands for zeros.
+template <int CELL, int ACT, int RB, bool USMEM, bool RD, bool INIT>
 __global__ void __launch_bounds__(RNN_THREADS, 1)
 rnn_forward_kernel(float* __restrict__ xg, const float* __restrict__ U, const uint8_t* __restrict__ mask,
                    float* __restrict__ hout, float* __restrict__ cst, int T, int B, int H,
-                   const float* __restrict__ rm) {
+                   const float* __restrict__ rm, const float* __restrict__ h0, const float* __restrict__ c0) {
+  static_assert(!(RD && INIT), "recurrent dropout is training only; the carried state is inference only");
   constexpr int G = (CELL == SEQREC_CELL_LSTM) ? 4 : (CELL == SEQREC_CELL_GRU ? 3 : 1);
   const int GH = G * H;
   const int Hp = round_up4(H);
@@ -67,7 +69,18 @@ rnn_forward_kernel(float* __restrict__ xg, const float* __restrict__ U, const ui
   const int tid = threadIdx.x;
   const int b0 = blockIdx.x * RB;
 
-  for (int i = tid; i < RB * Hp; i += RNN_THREADS) { h_s[i] = 0.f; c_s[i] = 0.f; }
+  if constexpr (INIT) {
+    // padding columns u >= H and rows past B stay zero; GRU's c_s (r*h) is recomputed every step
+    for (int i = tid; i < RB * Hp; i += RNN_THREADS) {
+      const int r = i / Hp, u = i - r * Hp;
+      const bool ok = b0 + r < B && u < H;
+      const size_t e = (size_t)(b0 + r) * H + u;
+      h_s[i] = (ok && h0) ? h0[e] : 0.f;
+      c_s[i] = (ok && c0 && CELL == SEQREC_CELL_LSTM) ? c0[e] : 0.f;
+    }
+  } else {
+    for (int i = tid; i < RB * Hp; i += RNN_THREADS) { h_s[i] = 0.f; c_s[i] = 0.f; }
+  }
   if (RD) {
     for (int i = tid; i < G * RB * Hp; i += RNN_THREADS) hm_s[i] = 0.f;
   }
@@ -302,33 +315,34 @@ static int pick_rb(int B) {
 
 static const size_t kMaxDynSmem = 227 * 1024;
 
-template <int CELL, int ACT, int RB, bool RD>
+template <int CELL, int ACT, int RB, bool RD, bool INIT>
 static int launch_fwd_rd(float* xg, const float* U, const uint8_t* mask, float* hout, float* cst, int T, int B, int H,
-                         const float* rm, cudaStream_t st) {
+                         const float* rm, const float* h0, const float* c0, cudaStream_t st) {
   constexpr int G = (CELL == SEQREC_CELL_LSTM) ? 4 : (CELL == SEQREC_CELL_GRU ? 3 : 1);
   const int GH = G * H, Hp = round_up4(H), GHp = round_up4(GH);
   const size_t base = sizeof(float) * (size_t)(2 * RB * Hp + RB * GHp + (RD ? G * RB * Hp : 0));
   const size_t with_u = base + sizeof(float) * (size_t)H * GH;
   const int grid = ceil_div(B, RB);
   if (with_u <= kMaxDynSmem) {
-    auto k = rnn_forward_kernel<CELL, ACT, RB, true, RD>;
+    auto k = rnn_forward_kernel<CELL, ACT, RB, true, RD, INIT>;
     cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)with_u);
     if (e != cudaSuccess) return -(int)e;
-    k<<<grid, RNN_THREADS, with_u, st>>>(xg, U, mask, hout, cst, T, B, H, rm);
+    k<<<grid, RNN_THREADS, with_u, st>>>(xg, U, mask, hout, cst, T, B, H, rm, h0, c0);
   } else {
-    auto k = rnn_forward_kernel<CELL, ACT, RB, false, RD>;
+    auto k = rnn_forward_kernel<CELL, ACT, RB, false, RD, INIT>;
     cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)base);
     if (e != cudaSuccess) return -(int)e;
-    k<<<grid, RNN_THREADS, base, st>>>(xg, U, mask, hout, cst, T, B, H, rm);
+    k<<<grid, RNN_THREADS, base, st>>>(xg, U, mask, hout, cst, T, B, H, rm, h0, c0);
   }
   SEQREC_CHECK_LAUNCH();
   return 0;
 }
 template <int CELL, int ACT, int RB>
 static int launch_fwd(float* xg, const float* U, const uint8_t* mask, float* hout, float* cst, int T, int B, int H,
-                      const float* rm, cudaStream_t st) {
-  return rm ? launch_fwd_rd<CELL, ACT, RB, true>(xg, U, mask, hout, cst, T, B, H, rm, st)
-            : launch_fwd_rd<CELL, ACT, RB, false>(xg, U, mask, hout, cst, T, B, H, nullptr, st);
+                      const float* rm, const float* h0, const float* c0, cudaStream_t st) {
+  if (h0 || c0) return launch_fwd_rd<CELL, ACT, RB, false, true>(xg, U, mask, hout, cst, T, B, H, nullptr, h0, c0, st);
+  if (rm) return launch_fwd_rd<CELL, ACT, RB, true, false>(xg, U, mask, hout, cst, T, B, H, rm, nullptr, nullptr, st);
+  return launch_fwd_rd<CELL, ACT, RB, false, false>(xg, U, mask, hout, cst, T, B, H, nullptr, nullptr, nullptr, st);
 }
 
 template <int CELL, int ACT, int RB, bool RD>
@@ -379,22 +393,26 @@ static int launch_bwd(float* xg, const float* Ut, const uint8_t* mask, const flo
 // register-resident fast path (rnn_reg.cu)
 bool rnn_reg_applicable(int cell, int H);
 int rnn_reg_launch(int cell, int act, int rb, bool fwd, float* xg, const float* U, const uint8_t* mask, float* hout,
-                   float* cst, const float* dhout, int T, int B, int H, cudaStream_t st);
+                   float* cst, const float* dhout, int T, int B, int H, cudaStream_t st, const float* h0 = nullptr,
+                   const float* c0 = nullptr);
 
 // rows per CTA of the register-resident scan: 96 of the 128 registers hold U when H > 96, leaving room for 2 rows
 static int reg_rb(int rb, int H) { return H > 96 ? (rb > 2 ? 2 : rb) : (rb > 4 ? 4 : rb); }
 
 extern "C" int seqrec_rnn_needs_ut(int cell, int H) { return rnn_reg_applicable(cell, H) ? 0 : 1; }
 
+// h0 / c0: initial state (NULL = zeros; never together with rm)
 static int rnn_forward_any(int cell, int act, float* xg, const float* U, const uint8_t* mask, float* hout, float* cst,
-                           int T, int B, int H, const float* rm, cudaStream_t st) {
+                           int T, int B, int H, const float* rm, cudaStream_t st, const float* h0 = nullptr,
+                           const float* c0 = nullptr) {
   const int rb = pick_rb(B);
   if (!rm && rnn_reg_applicable(cell, H))
-    return rnn_reg_launch(cell, act, reg_rb(rb, H), true, xg, U, mask, hout, cst, nullptr, T, B, H, st);
+    return rnn_reg_launch(cell, act, reg_rb(rb, H), true, xg, U, mask, hout, cst, nullptr, T, B, H, st, h0, c0);
   switch (cell) {
-    case SEQREC_CELL_SIMPLE: DISPATCH_ACT(launch_fwd, SEQREC_CELL_SIMPLE, xg, U, mask, hout, cst, T, B, H, rm, st)
-    case SEQREC_CELL_LSTM: DISPATCH_ACT(launch_fwd, SEQREC_CELL_LSTM, xg, U, mask, hout, cst, T, B, H, rm, st)
-    case SEQREC_CELL_GRU: DISPATCH_ACT(launch_fwd, SEQREC_CELL_GRU, xg, U, mask, hout, cst, T, B, H, rm, st)
+    case SEQREC_CELL_SIMPLE:
+      DISPATCH_ACT(launch_fwd, SEQREC_CELL_SIMPLE, xg, U, mask, hout, cst, T, B, H, rm, h0, c0, st)
+    case SEQREC_CELL_LSTM: DISPATCH_ACT(launch_fwd, SEQREC_CELL_LSTM, xg, U, mask, hout, cst, T, B, H, rm, h0, c0, st)
+    case SEQREC_CELL_GRU: DISPATCH_ACT(launch_fwd, SEQREC_CELL_GRU, xg, U, mask, hout, cst, T, B, H, rm, h0, c0, st)
     default: return -1003;
   }
 }
@@ -423,6 +441,14 @@ extern "C" int seqrec_rnn_forward(int cell, int act, float* xg, const float* U, 
                                   float* cst, int T, int B, int H, void* stream) {
   SEQREC_ARG(T > 0 && B > 0 && H > 0, 1);
   return rnn_forward_any(cell, act, xg, U, mask, hout, cst, T, B, H, nullptr, as_stream(stream));
+}
+
+extern "C" int seqrec_rnn_forward_state(int cell, int act, float* xg, const float* U, const float* h0,
+                                        const float* c0, const uint8_t* mask, float* hout, float* cst, int T, int B,
+                                        int H, void* stream) {
+  SEQREC_ARG(T > 0 && B > 0 && H > 0, 1);
+  SEQREC_ARG(c0 == nullptr || cell == SEQREC_CELL_LSTM, 2);
+  return rnn_forward_any(cell, act, xg, U, mask, hout, cst, T, B, H, nullptr, as_stream(stream), h0, c0);
 }
 
 extern "C" int seqrec_rnn_backward(int cell, int act, float* xg, const float* U, const float* Ut,

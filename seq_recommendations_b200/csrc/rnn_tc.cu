@@ -110,11 +110,15 @@ struct FwdCfg {
   static constexpr uint32_t SMEM = 2 * U_PART + 2 * H_PART + 4 * STG + 128 + 1024;
 };
 
-template <int CELL, int ACT, int CS>
+// INIT: the scan starts from h0 (B,H) and, for LSTM, c0 (B,H) instead of zeros (a NULL pointer stands for zeros).
+// Every CTA builds the whole h_{-1} operand from h0 with the split and swizzle of stage_slice, so a scan continued
+// from hout[T-1] (and cst[T-1]) computes bit for bit what one longer scan computes.
+template <int CELL, int ACT, int CS, bool INIT>
 __global__ void __launch_bounds__(RT_THREADS, 1)
 rnn_tc_forward_kernel(const __grid_constant__ CUtensorMap tmU_hi, const __grid_constant__ CUtensorMap tmU_lo,
                       float* __restrict__ xg, const uint8_t* __restrict__ mask, float* __restrict__ hout,
-                      float* __restrict__ cst, int T, int B, long long* __restrict__ dbg) {
+                      float* __restrict__ cst, int T, int B, long long* __restrict__ dbg,
+                      const float* __restrict__ h0, const float* __restrict__ c0) {
   using C = FwdCfg<CELL, CS>;
   constexpr int H = C::H, G = C::G, GH = G * H, RPS = C::RPS, KB = C::KB;
   constexpr bool LSTM = CELL == SEQREC_CELL_LSTM;
@@ -142,8 +146,21 @@ rnn_tc_forward_kernel(const __grid_constant__ CUtensorMap tmU_hi, const __grid_c
     ptx::mbar_init(bar_free, CS);
     ptx::fence_barrier_init();
   }
-  for (uint32_t i = threadIdx.x * 16u; i < 2 * C::H_PART; i += RT_THREADS * 16u) st_shared_u4(sH + i, 0, 0, 0, 0);
-  ptx::fence_proxy_async_smem();                             // h_{-1} = 0 is read by the tensor core (async proxy)
+  if constexpr (INIT) {
+    // the epilogue threads' (row, half) layout: each stages its 16 units of every unit slice p (rows past B: zeros)
+    if (warp < 4) {
+      const int row = 16 * warp + (lane & 15), hh = lane >> 4;
+      const bool ok = h0 != nullptr && b0 + row < B;
+      for (int p = 0; p < CS; ++p) {
+        float v[16];
+        load16(v, h0 + (size_t)(ok ? b0 + row : 0) * H + p * UPC + hh * 16, ok);
+        stage_slice(sH + (uint32_t)p * 4096u, sH + C::H_PART + (uint32_t)p * 4096u, row, hh, v);
+      }
+    }
+  } else {
+    for (uint32_t i = threadIdx.x * 16u; i < 2 * C::H_PART; i += RT_THREADS * 16u) st_shared_u4(sH + i, 0, 0, 0, 0);
+  }
+  ptx::fence_proxy_async_smem();                             // h_{-1} is read by the tensor core (async proxy)
   if (warp == 4) {
     ptx::tmem_alloc(tmem_slot, 64);
     ptx::tmem_relinquish();
@@ -263,6 +280,10 @@ rnn_tc_forward_kernel(const __grid_constant__ CUtensorMap tmU_hi, const __grid_c
     float hprev[16], cs[16], zg[16];
 #pragma unroll
     for (int j = 0; j < 16; ++j) { hprev[j] = 0.f; cs[j] = 0.f; zg[j] = 0.f; }
+    if constexpr (INIT) {
+      load16(hprev, h0 + (size_t)(valid ? b : 0) * H + u0, valid && h0 != nullptr);
+      if (LSTM) load16(cs, c0 + (size_t)(valid ? b : 0) * H + u0, valid && c0 != nullptr);
+    }
 
     auto after_acc = [&](int r) {                            // MMA of round r is complete
       ptx::mbar_wait(bar_acc, (uint32_t)r & 1u);
@@ -368,7 +389,7 @@ rnn_tc_forward_kernel(const __grid_constant__ CUtensorMap tmU_hi, const __grid_c
 
 template <int CELL, int ACT, int CS>
 int launch_fwd(float* xg, const uint16_t* Ut_hi, const uint16_t* Ut_lo, const uint8_t* mask, float* hout, float* cst,
-               int T, int B, cudaStream_t st) {
+               int T, int B, cudaStream_t st, const float* h0, const float* c0) {
   using C = FwdCfg<CELL, CS>;
   CUtensorMap tm_hi, tm_lo;
   int rc;
@@ -377,7 +398,7 @@ int launch_fwd(float* xg, const uint16_t* Ut_hi, const uint16_t* Ut_lo, const ui
     return rc;
   if ((rc = tma::make_2d_bf16(&tm_lo, Ut_lo, (uint64_t)C::G * C::H, C::H, C::H, 64, 16, CU_TENSOR_MAP_SWIZZLE_128B)))
     return rc;
-  auto k = rnn_tc_forward_kernel<CELL, ACT, CS>;
+  auto k = (h0 || c0) ? rnn_tc_forward_kernel<CELL, ACT, CS, true> : rnn_tc_forward_kernel<CELL, ACT, CS, false>;
   cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM);
   if (e != cudaSuccess) return -(int)e;
   cudaLaunchConfig_t cfg = {};
@@ -392,7 +413,7 @@ int launch_fwd(float* xg, const uint16_t* Ut_hi, const uint16_t* Ut_lo, const ui
   attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-  e = cudaLaunchKernelEx(&cfg, k, tm_hi, tm_lo, xg, mask, hout, cst, T, B, g_rnn_tc_dbg);
+  e = cudaLaunchKernelEx(&cfg, k, tm_hi, tm_lo, xg, mask, hout, cst, T, B, g_rnn_tc_dbg, h0, c0);
   if (e != cudaSuccess) return -(int)e;
   SEQREC_CHECK_LAUNCH();
   return 0;
@@ -400,12 +421,14 @@ int launch_fwd(float* xg, const uint16_t* Ut_hi, const uint16_t* Ut_lo, const ui
 
 template <int CELL, int CS>
 int dispatch_act_fwd(int act, float* xg, const uint16_t* Ut_hi, const uint16_t* Ut_lo, const uint8_t* mask,
-                     float* hout, float* cst, int T, int B, cudaStream_t st) {
+                     float* hout, float* cst, int T, int B, cudaStream_t st, const float* h0, const float* c0) {
   switch (act) {
-    case SEQREC_ACT_RELU: return launch_fwd<CELL, SEQREC_ACT_RELU, CS>(xg, Ut_hi, Ut_lo, mask, hout, cst, T, B, st);
-    case SEQREC_ACT_TANH: return launch_fwd<CELL, SEQREC_ACT_TANH, CS>(xg, Ut_hi, Ut_lo, mask, hout, cst, T, B, st);
+    case SEQREC_ACT_RELU:
+      return launch_fwd<CELL, SEQREC_ACT_RELU, CS>(xg, Ut_hi, Ut_lo, mask, hout, cst, T, B, st, h0, c0);
+    case SEQREC_ACT_TANH:
+      return launch_fwd<CELL, SEQREC_ACT_TANH, CS>(xg, Ut_hi, Ut_lo, mask, hout, cst, T, B, st, h0, c0);
     case SEQREC_ACT_LINEAR:
-      return launch_fwd<CELL, SEQREC_ACT_LINEAR, CS>(xg, Ut_hi, Ut_lo, mask, hout, cst, T, B, st);
+      return launch_fwd<CELL, SEQREC_ACT_LINEAR, CS>(xg, Ut_hi, Ut_lo, mask, hout, cst, T, B, st, h0, c0);
     default: return -1002;
   }
 }
@@ -770,7 +793,7 @@ namespace {
 template <int CELL, int CS>
 int max_clusters_fwd() {
   using C = FwdCfg<CELL, CS>;
-  auto k = rnn_tc_forward_kernel<CELL, SEQREC_ACT_TANH, CS>;
+  auto k = rnn_tc_forward_kernel<CELL, SEQREC_ACT_TANH, CS, false>;
   cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM);
   if (e != cudaSuccess) return -(int)e;
   cudaLaunchConfig_t cfg = {};
@@ -802,18 +825,28 @@ extern "C" int seqrec_rnn_tc_applicable(int cell, int H) {
   return ((cell == SEQREC_CELL_LSTM || cell == SEQREC_CELL_GRU) && (H == 128 || H == 256)) ? 1 : 0;
 }
 
+extern "C" int seqrec_rnn_tc_forward_state(int cell, int act, float* xg, const uint16_t* Ut_hi,
+                                           const uint16_t* Ut_lo, const float* h0, const float* c0,
+                                           const uint8_t* mask, float* hout, float* cst, int T, int B, int H,
+                                           void* stream) {
+  SEQREC_ARG(T > 0 && B > 0 && seqrec_rnn_tc_applicable(cell, H), 1);
+  SEQREC_ARG(xg && Ut_hi && Ut_lo && mask && hout && (cell != SEQREC_CELL_LSTM || cst), 2);
+  SEQREC_ARG(c0 == nullptr || cell == SEQREC_CELL_LSTM, 2);
+  SEQREC_ARG(((uintptr_t)h0 & 15) == 0 && ((uintptr_t)c0 & 15) == 0, 2);   // read as float4
+  cudaStream_t st = as_stream(stream);
+  if (cell == SEQREC_CELL_LSTM) {
+    if (H == 256)
+      return dispatch_act_fwd<SEQREC_CELL_LSTM, 8>(act, xg, Ut_hi, Ut_lo, mask, hout, cst, T, B, st, h0, c0);
+    return dispatch_act_fwd<SEQREC_CELL_LSTM, 4>(act, xg, Ut_hi, Ut_lo, mask, hout, cst, T, B, st, h0, c0);
+  }
+  if (H == 256) return dispatch_act_fwd<SEQREC_CELL_GRU, 8>(act, xg, Ut_hi, Ut_lo, mask, hout, cst, T, B, st, h0, c0);
+  return dispatch_act_fwd<SEQREC_CELL_GRU, 4>(act, xg, Ut_hi, Ut_lo, mask, hout, cst, T, B, st, h0, c0);
+}
+
 extern "C" int seqrec_rnn_tc_forward(int cell, int act, float* xg, const uint16_t* Ut_hi, const uint16_t* Ut_lo,
                                      const uint8_t* mask, float* hout, float* cst, int T, int B, int H,
                                      void* stream) {
-  SEQREC_ARG(T > 0 && B > 0 && seqrec_rnn_tc_applicable(cell, H), 1);
-  SEQREC_ARG(xg && Ut_hi && Ut_lo && mask && hout && (cell != SEQREC_CELL_LSTM || cst), 2);
-  cudaStream_t st = as_stream(stream);
-  if (cell == SEQREC_CELL_LSTM) {
-    if (H == 256) return dispatch_act_fwd<SEQREC_CELL_LSTM, 8>(act, xg, Ut_hi, Ut_lo, mask, hout, cst, T, B, st);
-    return dispatch_act_fwd<SEQREC_CELL_LSTM, 4>(act, xg, Ut_hi, Ut_lo, mask, hout, cst, T, B, st);
-  }
-  if (H == 256) return dispatch_act_fwd<SEQREC_CELL_GRU, 8>(act, xg, Ut_hi, Ut_lo, mask, hout, cst, T, B, st);
-  return dispatch_act_fwd<SEQREC_CELL_GRU, 4>(act, xg, Ut_hi, Ut_lo, mask, hout, cst, T, B, st);
+  return seqrec_rnn_tc_forward_state(cell, act, xg, Ut_hi, Ut_lo, nullptr, nullptr, mask, hout, cst, T, B, H, stream);
 }
 
 extern "C" int seqrec_rnn_tc_backward(int cell, int act, float* xg, const uint16_t* U_hi, const uint16_t* U_lo,

@@ -30,6 +30,7 @@ from . import _lib
 from ._lib import ACT, CELL, call, ptr
 from .dist import Comm, embedding_grad_mode
 from .gemm import gemm
+from .state import RecurrentState
 
 GATES = {"simpleRNN": 1, "LSTM": 4, "GRU": 3}
 NUM_SMS = 148
@@ -482,7 +483,8 @@ class HotPath:
         return t
 
     # ------------------------------------------------------------------------------------------------ forward
-    def _forward_hidden(self, w, training):
+    def _forward_hidden(self, w, training, state=None):
+        """state: RecurrentState the scan starts from (inference only); None = zeros."""
         st = self.stream
         w.in_scale = None
         w.hscale = None
@@ -508,6 +510,16 @@ class HotPath:
             w.rec_mask = self._dropout((self.G, w.B, self.H), self.dropout_rec)
             call("seqrec_rnn_forward_rd", CELL[self.cell], ACT[self.act], ptr(w.xg), ptr(self.U), ptr(w.rec_mask),
                  ptr(w.mask), ptr(w.hout), ptr(w.cst), w.T, w.B, self.H, st)
+        elif state is not None:
+            h0, c0 = self._state_operands(state, w.B)
+            if self.rnn_tc:
+                call("seqrec_split_bf16", ptr(self.U), None, ptr(self.Ut_hi), ptr(self.Ut_lo), self.H, self.GH, self.H,
+                     1, st)
+                call("seqrec_rnn_tc_forward_state", CELL[self.cell], ACT[self.act], ptr(w.xg), ptr(self.Ut_hi),
+                     ptr(self.Ut_lo), ptr(h0), ptr(c0), ptr(w.mask), ptr(w.hout), ptr(w.cst), w.T, w.B, self.H, st)
+            else:
+                call("seqrec_rnn_forward_state", CELL[self.cell], ACT[self.act], ptr(w.xg), ptr(self.U), ptr(h0),
+                     ptr(c0), ptr(w.mask), ptr(w.hout), ptr(w.cst), w.T, w.B, self.H, st)
         elif self.rnn_tc:
             call("seqrec_split_bf16", ptr(self.U), None, ptr(self.Ut_hi), ptr(self.Ut_lo), self.H, self.GH, self.H, 1,
                  st)
@@ -1203,13 +1215,78 @@ class HotPath:
         return loss, out, dict(dh=(dh / n_valid).cpu().numpy(), rows=rows,
                                dxp=(w.xg.detach() / n_valid).cpu().numpy())
 
+    # ------------------------------------------------------------------------------------------------ carried state
+    def initial_state(self, n):
+        """The zero state of n sessions: what every scan of a whole window starts from."""
+        return RecurrentState.zeros(n, self.cell, self.H, self.device)
+
+    def _state_operands(self, state, n):
+        """(h0, c0) device pointers' tensors of a state of n sessions (c0 None unless LSTM)."""
+        state.check(self.cell, self.H, n)
+        h = state.h.to(self.device, torch.float32).contiguous()
+        c = None if state.c is None else state.c.to(self.device, torch.float32).contiguous()
+        return h, c
+
+    def advance_state(self, ids, state=None, x_dense=None):
+        """Continues the masked recurrence of a batch of sessions over a left-padded chunk of new events (B,T') and
+        returns the state after it (fresh tensors).  state None = the zero state.  A pad step holds h and c, so an
+        all-pad row keeps its state bit for bit; advancing by a and then by b equals advancing by a|b bit for bit."""
+        B, T = (ids.shape if ids is not None else x_dense.shape[:2])
+        w = self.work(int(B), int(T))
+        self._stage(w, ids, None, x_dense)
+        self._forward_hidden(w, training=False, state=state)
+        return RecurrentState(w.hout[w.T - 1].clone(), w.cst[w.T - 1].clone() if self.cell == "LSTM" else None,
+                              self.cell, self.H)
+
+    def _state_work(self, state, tgt=None):
+        """The (n, 1) work object of the last_step_only scorers with hout = state.h.  Every row is scored (a state
+        always has a next item); with targets, a target < 0 is a pad (p = 1e-7, rank 0)."""
+        h, _ = self._state_operands(state, len(state))
+        wl = self.work(len(state), 1)
+        wl.hout[0].copy_(h)
+        wl.hscale = None
+        if tgt is None:
+            wl.mask.fill_(1)
+        else:
+            self._check_host_ids(None, tgt)
+            t = torch.as_tensor(tgt).to(self.device, torch.int32).reshape(-1)
+            if t.numel() != wl.B:
+                raise ValueError("%d targets for %d sessions" % (t.numel(), wl.B))
+            if bool((t >= self.V_total).any()):
+                raise ValueError("target id outside the catalog (%d items)" % self.V_total)
+            wl.tgt[0].copy_(t)
+            wl.mask[0].copy_(t >= 0)
+        return wl
+
+    def topk_from_state(self, state, k):
+        """Top-k next items after each session's state: (n,k) ids and probabilities, computed by the kernels of
+        topk_batch(last_step_only=True)."""
+        return self._topk_scored(self._state_work(state), int(k), True)
+
+    def target_prob_from_state(self, state, tgt):
+        """p(tgt[i] is the next item of session i), (n,) clipped like target_prob_batch."""
+        wl = self._state_work(state, tgt)
+        if self.vocab_parallel:
+            wg = self._vp_forward(wl, training=False)
+            lo = self.comm.rank * wl.N
+            return wg.py[lo:lo + wl.N].clone()
+        self._forward_ce(wl)
+        return wl.py.clone()
+
+    def target_rank_from_state(self, state, tgt):
+        """(n,) int32 rank of tgt[i] after session i's state, as target_rank_batch(last_step_only=True)."""
+        wl = self._state_work(state, tgt)
+        if self.vocab_parallel:
+            return self._rank_vp(wl, True)
+        return self._target_rank(wl)
+
     # ------------------------------------------------------------------------------------------------ scoring
-    def hidden_batch(self, ids, x_dense=None):
+    def hidden_batch(self, ids, x_dense=None, initial_state=None):
         """(B,T,H) hidden outputs (z_to_z_output activations), inference phase."""
         B, T = (ids.shape if ids is not None else x_dense.shape[:2])
         w = self.work(int(B), int(T))
         self._stage(w, ids, None, x_dense)
-        self._forward_hidden(w, training=False)
+        self._forward_hidden(w, training=False, state=initial_state)
         return w.hout.permute(1, 0, 2).contiguous()
 
     def predict_batch(self, ids, x_dense=None):
@@ -1232,12 +1309,13 @@ class HotPath:
              w.T, w.B, self.H, self.V, self.stream)
         return probs
 
-    def target_prob_batch(self, ids, tgt, x_dense=None):
-        """p(true next item) per step, clipped to [1e-7, 1-1e-7] like model.py:108-110; (B,T) device tensor."""
+    def target_prob_batch(self, ids, tgt, x_dense=None, initial_state=None):
+        """p(true next item) per step, clipped to [1e-7, 1-1e-7] like model.py:108-110; (B,T) device tensor.
+        initial_state: the sessions' RecurrentState the chunk continues (None = zeros)."""
         B, T = (ids.shape if ids is not None else x_dense.shape[:2])
         w = self.work(int(B), int(T))
         self._stage(w, ids, tgt, x_dense)
-        self._forward_hidden(w, training=False)
+        self._forward_hidden(w, training=False, state=initial_state)
         if self.vocab_parallel:
             # every rank scores all ranks' tokens against its item shard; the merged statistics cover the whole catalog
             wg = self._vp_forward(w, training=False)
@@ -1326,16 +1404,17 @@ class HotPath:
         rank = counts[lo:lo + n_loc] + (tg.reshape(-1) >= 0).to(torch.int32)
         return rank if last_step_only else rank.view(w.T, w.B).t().contiguous()
 
-    def target_rank_batch(self, ids, tgt, x_dense=None, last_step_only=False):
+    def target_rank_batch(self, ids, tgt, x_dense=None, last_step_only=False, initial_state=None):
         """Rank of the true next item per step: (B,T) int32 device tensor, or (B,) for the last step only.
         rank = 1 + #{v != y : z_v > z_y} + #{v < y : z_v == z_y} (stable descending order, ties to the lower item id:
         rank <= k <=> topk_batch holds y at index rank-1); pads have rank 0.  On the tensor cores the logits are compared
         with the exact fp32 target logit, so the rank is exact outside the band of the split-product error around z_y,
-        and p(target) of the same rows is left in the work object's `py` by the same pass."""
+        and p(target) of the same rows is left in the work object's `py` by the same pass.
+        initial_state: the sessions' RecurrentState the chunk continues (None = zeros)."""
         B, T = (ids.shape if ids is not None else x_dense.shape[:2])
         w = self.work(int(B), int(T))
         self._stage(w, ids, tgt, x_dense)
-        self._forward_hidden(w, training=False)
+        self._forward_hidden(w, training=False, state=initial_state)
         if self.vocab_parallel:
             return self._rank_vp(w, last_step_only)
         if last_step_only:
@@ -1360,12 +1439,18 @@ class HotPath:
         call("seqrec_softmax_rows_stats", ptr(Z), None, ptr(m), ptr(s_), None, n, self.V, self.stream)
         return Z, m, s_
 
-    def topk_batch(self, ids, k, last_step_only=True, x_dense=None):
-        """Top-k next items: (B,k) ids and probabilities for the last step, or (B,T,k) for every step."""
+    def topk_batch(self, ids, k, last_step_only=True, x_dense=None, initial_state=None):
+        """Top-k next items: (B,k) ids and probabilities for the last step, or (B,T,k) for every step.
+        initial_state: the sessions' RecurrentState the chunk continues (None = zeros)."""
         B, T = (ids.shape if ids is not None else x_dense.shape[:2])
         w = self.work(int(B), int(T))
         self._stage(w, ids, None, x_dense)
-        self._forward_hidden(w, training=False)
+        self._forward_hidden(w, training=False, state=initial_state)
+        return self._topk_scored(w, int(k), last_step_only)
+
+    def _topk_scored(self, w, k, last_step_only):
+        """Top-k of the rows of w.hout (all steps, or the last one)."""
+        B = w.B
         if self.vocab_parallel:
             return self._topk_vp(w, int(k), last_step_only)
         if w.tc["panel"]:
@@ -1381,8 +1466,9 @@ class HotPath:
         if last_step_only:
             # softmax statistics of the last step only: a (B, 1) problem over the rows hout[T-1]
             wl = self.work(int(B), 1)
-            wl.hout.copy_(w.hout[w.T - 1:w.T])
-            wl.mask.copy_(w.mask[w.T - 1:w.T])
+            if wl is not w:
+                wl.hout.copy_(w.hout[w.T - 1:w.T])
+                wl.mask.copy_(w.mask[w.T - 1:w.T])
             wl.hscale = None
             self._forward_ce(wl, with_targets=False)
             hrows, m, s, n = wl.hout[0], wl.m, wl.s, wl.B

@@ -22,6 +22,7 @@ from . import callbacks as cb
 from . import optimizers
 from .engine import GATES, HotPath
 from .engine_dense import DensePath
+from .state import RecurrentState, write_npz
 from .likelihood import compute_likelihood, compute_likelihood_cut  # noqa: F401  (utils.py:145-178, on the device)
 from .preprocessor import is_one_hot, to_id_batch
 from .ranking import check_ks, metrics_from_sums, rank_sums
@@ -179,13 +180,7 @@ class _Net(object):
         """Rank 0 writes (temp file + rename: a reader never sees a torn archive), everybody waits."""
         comm = self.hot.comm
         if comm.rank == 0:
-            d = os.path.dirname(filepath)
-            if d and not os.path.exists(d):
-                os.makedirs(d)
-            tmp = "%s.tmp.%d" % (filepath, os.getpid())
-            with open(tmp, "wb") as f:
-                np.savez(f, **arrays)
-            os.replace(tmp, filepath)
+            write_npz(filepath, arrays)
         comm.barrier()
 
     def save_weights(self, filepath, overwrite=True):
@@ -433,49 +428,132 @@ class _Net(object):
         return np.concatenate(out, axis=0)
 
     # ---- additive scoring API --------------------------------------------------------------------------------------
-    def predict_target_prob(self, x, y, batch_size=1024, device=False):
+    def predict_target_prob(self, x, y, batch_size=1024, device=False, initial_state=None):
         """(N,T) p(true next item), clipped to [1e-7, 1-1e-7]; pads give 1e-7 (model.py:108-110 semantics).
-        device=True returns the device tensor (the likelihood metrics reduce it in HBM)."""
+        device=True returns the device tensor (the likelihood metrics reduce it in HBM).  initial_state: the
+        RecurrentState of the N sessions that x continues (None = zeros, the whole-window semantics)."""
         ids, xd = self._inputs(x)
         tgt = to_id_batch(y)
+        self._check_state(initial_state, len(tgt))
         out = []
         for lo in range(0, len(tgt), batch_size):
             hi = min(len(tgt), lo + batch_size)
             i, d = self._slice(ids, xd, slice(lo, hi))
-            out.append(self.hot.target_prob_batch(i, tgt[lo:hi], d).clone())
+            out.append(self.hot.target_prob_batch(i, tgt[lo:hi], d, **self._state_kw(initial_state, lo, hi)).clone())
         out = torch.cat(out, dim=0)
         self.hot.check_errors()
         return out if device else out.cpu().numpy()
 
-    def predict_topk(self, x, k=20, last_step_only=True, batch_size=1024):
-        """Top-k next-item ids (int32) and probabilities; ties broken by the lower item id."""
+    def predict_topk(self, x, k=20, last_step_only=True, batch_size=1024, initial_state=None):
+        """Top-k next-item ids (int32) and probabilities; ties broken by the lower item id.  initial_state: the
+        RecurrentState of the sessions that x continues (None = zeros)."""
         ids, xd = self._inputs(x)
         n = len(ids) if ids is not None else len(xd)
+        self._check_state(initial_state, n)
         oi, op = [], []
         for lo in range(0, n, batch_size):
-            i, d = self._slice(ids, xd, slice(lo, min(n, lo + batch_size)))
-            a, b = self.hot.topk_batch(i, k, last_step_only=last_step_only, x_dense=d)
+            hi = min(n, lo + batch_size)
+            i, d = self._slice(ids, xd, slice(lo, hi))
+            a, b = self.hot.topk_batch(i, k, last_step_only=last_step_only, x_dense=d,
+                                       **self._state_kw(initial_state, lo, hi))
             oi.append(a.cpu().numpy())
             op.append(b.cpu().numpy())
         return np.concatenate(oi, axis=0), np.concatenate(op, axis=0)
 
-    def _target_ranks(self, x, y, batch_size, last_step_only):
+    def _target_ranks(self, x, y, batch_size, last_step_only, initial_state=None):
         ids, xd = self._inputs(x)
         tgt = to_id_batch(y)
+        self._check_state(initial_state, len(tgt))
         out = []
         for lo in range(0, len(tgt), batch_size):
             hi = min(len(tgt), lo + batch_size)
             i, d = self._slice(ids, xd, slice(lo, hi))
-            out.append(self.hot.target_rank_batch(i, tgt[lo:hi], d, last_step_only=last_step_only).clone())
+            out.append(self.hot.target_rank_batch(i, tgt[lo:hi], d, last_step_only=last_step_only,
+                                                  **self._state_kw(initial_state, lo, hi)).clone())
         out = torch.cat(out, dim=0)
         self.hot.check_errors()
         return out
 
-    def predict_target_rank(self, x, y, batch_size=1024, device=False):
+    def predict_target_rank(self, x, y, batch_size=1024, device=False, initial_state=None):
         """(N,T) int32 rank of the true next item among all items: 1 + the items with a higher logit + the lower-id
         items with an equal one (so rank <= k <=> predict_topk holds it at index rank-1); pads give 0.
-        device=True returns the device tensor (ranking.ranking_metrics reduces it in HBM)."""
-        out = self._target_ranks(x, y, batch_size, False)
+        device=True returns the device tensor (ranking.ranking_metrics reduces it in HBM).  initial_state: the
+        RecurrentState of the sessions that x continues (None = zeros)."""
+        out = self._target_ranks(x, y, batch_size, False, initial_state)
+        return out if device else out.cpu().numpy()
+
+    # ---- carried recurrent state (inference) ---------------------------------------------------------------------
+    def _need_state_support(self):
+        if not isinstance(self.hot, HotPath):
+            raise NotImplementedError(
+                "carried state is built for the recurrent hot path (ytoz RNNFullModel, RNNBaseline): the x_to_z / "
+                "x_to_y / y_to_y branches and NoRecurrenceModel also read history features and the previous item, "
+                "which a recurrent state does not carry")
+
+    def _check_state(self, state, n):
+        if state is not None:
+            self._need_state_support()
+            state.check(self.hot.cell, self.hot.H, n)
+
+    @staticmethod
+    def _state_kw(state, lo, hi):
+        return {} if state is None else {"initial_state": state.take(slice(lo, hi))}
+
+    def initial_state(self, n):
+        """The zero state of n sessions (what scoring a whole window starts from)."""
+        self._need_state_support()
+        return self.hot.initial_state(n)
+
+    def advance_state(self, x, state=None, batch_size=1024):
+        """The state of each session after the new events x (any input `predict` takes: ids (n,T'), one-hot, or
+        RNNBaseline's dense input), continuing `state` (None = zeros).  Pads hold the state."""
+        self._need_state_support()
+        ids, xd = self._inputs(x)
+        n = len(ids) if ids is not None else len(xd)
+        self._check_state(state, n)
+        hs, cs = [], []
+        for lo in range(0, n, batch_size):
+            hi = min(n, lo + batch_size)
+            i, d = self._slice(ids, xd, slice(lo, hi))
+            st = self.hot.advance_state(i, None if state is None else state.take(slice(lo, hi)), d)
+            hs.append(st.h)
+            cs.append(st.c)
+        self.hot.check_errors()
+        return RecurrentState(torch.cat(hs), None if cs[0] is None else torch.cat(cs), self.hot.cell, self.hot.H)
+
+    def _from_state(self, state, batch_size, fn):
+        self._need_state_support()
+        self._check_state(state, len(state))
+        out = [fn(state.take(slice(lo, min(len(state), lo + batch_size))), lo, min(len(state), lo + batch_size))
+               for lo in range(0, len(state), batch_size)]
+        self.hot.check_errors()
+        return out
+
+    @staticmethod
+    def _next_ids(y, n):
+        t = y if isinstance(y, torch.Tensor) else torch.from_numpy(np.asarray(y, dtype=np.int64))
+        if t.dim() != 1 or t.numel() != n:
+            raise ValueError("y must be the (%d,) next-item ids of the sessions" % n)
+        return t
+
+    def predict_topk_from_state(self, state, k=20, batch_size=1024):
+        """Top-k next items after each session's state: (n,k) int32 ids and probabilities, equal to predict_topk on
+        the events the state has seen (for histories of at most T events)."""
+        out = self._from_state(state, batch_size, lambda s, lo, hi: self.hot.topk_from_state(s, k))
+        return (np.concatenate([a.cpu().numpy() for a, _ in out]), np.concatenate([b.cpu().numpy() for _, b in out]))
+
+    def predict_target_prob_from_state(self, state, y, batch_size=1024, device=False):
+        """(n,) p(y[i] is the next item of session i); y < 0 is a pad (1e-7)."""
+        t = self._next_ids(y, len(state))
+        out = torch.cat(self._from_state(state, batch_size,
+                                         lambda s, lo, hi: self.hot.target_prob_from_state(s, t[lo:hi])))
+        return out if device else out.cpu().numpy()
+
+    def predict_target_rank_from_state(self, state, y, batch_size=1024, device=False):
+        """(n,) int32 rank of y[i] after session i's state (the rank of predict_target_rank); y < 0 gives 0."""
+        t = self._next_ids(y, len(state))
+        out = torch.cat(self._from_state(state, batch_size,
+                                         lambda s, lo, hi: self.hot.target_rank_from_state(s, t[lo:hi])))
         return out if device else out.cpu().numpy()
 
     def evaluate_ranking(self, x, y, ks=(1, 5, 10, 20), last_step_only=False, batch_size=1024):
@@ -561,14 +639,30 @@ class BaseRNNModel(BaseModel):
         raise NotImplementedError("get_activations is built for the recurrent layer and the output layer only")
 
     # additive
-    def predict_target_prob(self, x_test, y_test, batch_size=1024):
-        return self.model.predict_target_prob(x_test, y_test, batch_size=batch_size)
+    def predict_target_prob(self, x_test, y_test, batch_size=1024, initial_state=None):
+        return self.model.predict_target_prob(x_test, y_test, batch_size=batch_size, initial_state=initial_state)
 
-    def predict_topk(self, x_test, k=20, last_step_only=True, batch_size=1024):
-        return self.model.predict_topk(x_test, k=k, last_step_only=last_step_only, batch_size=batch_size)
+    def predict_topk(self, x_test, k=20, last_step_only=True, batch_size=1024, initial_state=None):
+        return self.model.predict_topk(x_test, k=k, last_step_only=last_step_only, batch_size=batch_size,
+                                       initial_state=initial_state)
 
-    def predict_target_rank(self, x_test, y_test, batch_size=1024):
-        return self.model.predict_target_rank(x_test, y_test, batch_size=batch_size)
+    def predict_target_rank(self, x_test, y_test, batch_size=1024, initial_state=None):
+        return self.model.predict_target_rank(x_test, y_test, batch_size=batch_size, initial_state=initial_state)
+
+    def initial_state(self, n):
+        return self.model.initial_state(n)
+
+    def advance_state(self, x, state=None, batch_size=1024):
+        return self.model.advance_state(x, state=state, batch_size=batch_size)
+
+    def predict_topk_from_state(self, state, k=20, batch_size=1024):
+        return self.model.predict_topk_from_state(state, k=k, batch_size=batch_size)
+
+    def predict_target_prob_from_state(self, state, y, batch_size=1024):
+        return self.model.predict_target_prob_from_state(state, y, batch_size=batch_size)
+
+    def predict_target_rank_from_state(self, state, y, batch_size=1024):
+        return self.model.predict_target_rank_from_state(state, y, batch_size=batch_size)
 
     def evaluate_ranking(self, x_test, y_test, ks=(1, 5, 10, 20), last_step_only=False, batch_size=1024):
         return self.model.evaluate_ranking(x_test, y_test, ks=ks, last_step_only=last_step_only, batch_size=batch_size)
