@@ -803,15 +803,11 @@ class HotPath:
     # ------------------------------------------------------------------------------------------------ public steps
     def loss_batch(self, ids, tgt, x_dense=None):
         """Forward only: returns (loss_sum, n_valid) device tensors of THIS rank's batch (evaluate path)."""
-        B, T = (ids.shape if ids is not None else x_dense.shape[:2])
-        w = self.work(int(B), int(T))
-        self._stage(w, ids, tgt, x_dense)
-        self._forward_hidden(w, training=False)
+        w = self._scan_batch(ids, tgt, x_dense)
         if self.vocab_parallel:
             # loss_sum already covers every rank's tokens: report this rank's share so callers can all-reduce as usual
             wg = self._vp_forward(w, training=False)
-            lo = self.comm.rank * w.N
-            return wg.ce[lo:lo + w.N].sum().reshape(1), w.n_valid_i.to(torch.float32)
+            return self._my_rows(wg.ce).sum().reshape(1), w.n_valid_i.to(torch.float32)
         self._forward_ce(w)
         return w.loss_sum.clone(), w.n_valid_i.to(torch.float32)
 
@@ -979,40 +975,61 @@ class HotPath:
         per-token (max, sum-exp) partials and the target logit are merged across ranks.  Returns the work object that
         holds the global-token buffers (token order: rank-major blocks of each rank's time-major tokens).
         Three collectives: hidden rows, targets (pads are -1, so the mask travels with them), packed (m, s, zy)."""
-        comm = self.comm
-        wg = self.work(w.B * comm.world, w.T)
-        hs = w.hout.view(w.N, self.H)
-        if w.hscale is not None:
-            hs = hs * w.hscale
-        wg.hout.view(wg.N, self.H).copy_(comm.all_gather_cat(hs))
-        wg.hscale = None
-        tgt_all = comm.all_gather_cat(w.tgt.view(-1))
-        valid = tgt_all >= 0
-        wg.mask.view(-1).copy_(valid)
-        local = (tgt_all >= self.v_lo) & (tgt_all < self.v_lo + self.V)
-        wg.tgt.view(-1).copy_(torch.where(local, tgt_all - self.v_lo, torch.full_like(tgt_all, -1)))
-        wg.zy.zero_()
+        wg, _ = self._vp_gather(w)
         if train:
             # n_valid and the loss sum of ALL tokens are known locally (identical on every rank): they go into the step
             # floats directly and stay outside the reduced range
-            self.scal[0:1].copy_(valid.sum().to(torch.int32))
+            self.scal[0:1].copy_(wg.mask.view(-1).sum().to(torch.int32))
         if train and self.ce_fused and wg.tc["bwd"]:
             # fused statistics + dh pass: the target logit (owner's shard) is summed over the shards FIRST and is every
             # rank's reference; the partial sum-exps then add up across shards (same reference) -- two N-float all-reduces
-            self._ce_train_fused(wg, zy_reduce=comm.all_reduce_sum, s_reduce=comm.all_reduce_sum)
+            self._ce_train_fused(wg, zy_reduce=self.comm.all_reduce_sum, s_reduce=self.comm.all_reduce_sum)
             wg.fused = True
             return wg
         wg.fused = False
-        n_splits = self._ce_partials(wg, True, training)
-        # local merge -> (m_r, s_r) per token; ONE exchange of the packed (m, s, zy); global merge (only the owner of a
-        # target contributes a non-zero zy)
+        self._vp_merge(wg, True, training, train)
+        return wg
+
+    def _vp_gather(self, w, last_step_only=False, with_targets=True):
+        """All ranks' rows of w -- every token, or step T-1 of every session -- in this rank's work(B*P, T or 1), rank
+        after rank: the hidden rows (times the output-dropout factors when set) and either the targets (remapped to
+        this shard's item ids, -1 elsewhere; mask = target >= 0) or the mask.  Returns (wg, the gathered global target
+        ids or None)."""
+        comm = self.comm
+        wg = self.work(w.B * comm.world, 1 if last_step_only else w.T)
+        rows = w.hout[w.T - 1] if last_step_only else w.hout.view(w.N, self.H)
+        if w.hscale is not None:              # output dropout of a training step (every step)
+            rows = rows * w.hscale
+        wg.hout.view(wg.N, self.H).copy_(comm.all_gather_cat(rows))
+        wg.hscale = None
+        if not with_targets:
+            wg.mask.view(-1).copy_(comm.all_gather_cat(w.mask[w.T - 1] if last_step_only else w.mask.view(-1)))
+            return wg, None
+        tgt_all = comm.all_gather_cat(w.tgt[w.T - 1] if last_step_only else w.tgt.view(-1))
+        wg.mask.view(-1).copy_(tgt_all >= 0)
+        local = (tgt_all >= self.v_lo) & (tgt_all < self.v_lo + self.V)
+        wg.tgt.view(-1).copy_(torch.where(local, tgt_all - self.v_lo, torch.full_like(tgt_all, -1)))
+        wg.zy.zero_()
+        return wg, tgt_all
+
+    def _vp_merge(self, wg, with_targets, training=False, train=False):
+        """Catalog-wide softmax statistics of wg's rows from this shard's logits: the partials are merged locally to
+        (m_r, s_r) per row, ONE exchange of the packed (m, s[, zy]), then the global merge (only the owner of a target
+        contributes a non-zero zy)."""
+        comm = self.comm
+        n_splits = self._ce_partials(wg, with_targets, training)
         call("seqrec_ce_finalize", ptr(wg.ws_m), ptr(wg.ws_s), None, None, ptr(wg.m), ptr(wg.s), None, None, None, None,
              wg.N, n_splits, self.stream)
-        packed = comm.all_gather_cat(torch.stack([wg.m, wg.s, wg.zy]).unsqueeze(0))      # (P, 3, N)
-        packed = packed.permute(1, 0, 2).contiguous()                                    # (3, P, N)
-        torch.sum(packed[2], dim=0, out=wg.zy)
-        self._finalize_ce(wg, packed[0], packed[1], comm.world, True, train=train)
-        return wg
+        parts = [wg.m, wg.s, wg.zy] if with_targets else [wg.m, wg.s]
+        packed = comm.all_gather_cat(torch.stack(parts).unsqueeze(0)).permute(1, 0, 2).contiguous()   # (2|3, P, N)
+        if with_targets:
+            torch.sum(packed[2], dim=0, out=wg.zy)
+        self._finalize_ce(wg, packed[0], packed[1], comm.world, with_targets, train=train)
+
+    def _my_rows(self, t):
+        """This rank's block of a tensor over all ranks' rows (rank-major blocks)."""
+        n = t.shape[0] // self.comm.world
+        return t[self.comm.rank * n:(self.comm.rank + 1) * n]
 
     def _train_core_vp(self, w):
         """Vocabulary-parallel step (SURVEY 8(e), cfg4): data-parallel scan, logits against the local V/P items for the
@@ -1119,8 +1136,10 @@ class HotPath:
                          ptr(self.flat_a[off:off + sz]), sz, o["lr"], o["eps"], o["clipnorm"], ptr(self.sumsq), den, st)
         self._join()
 
-    def _rank_rows(self, wt, hrows, m, s, n, k):
-        """Top-k of n rows against THIS rank's items (ids are local item indices), probabilities from (m, s)."""
+    def _topk_rows(self, wt, k):
+        """Top-k of the wt.N rows of wt.hout against THIS rank's items (ids are local item indices), probabilities from
+        the softmax statistics (wt.m, wt.s)."""
+        hrows, m, s, n = wt.hout, wt.m, wt.s, wt.N
         out_i = torch.empty((n, k), dtype=torch.int32, device=self.device)
         out_p = torch.empty((n, k), dtype=torch.float32, device=self.device)
         n_lists = wt.tc["splits"] if wt.tc["fwd"] else 0
@@ -1143,21 +1162,10 @@ class HotPath:
         comm = self.comm
         if k > self.V:
             raise ValueError("k must not exceed the items of one shard (%d)" % self.V)
-        if last_step_only:
-            rows, msk, nb, nt = w.hout[w.T - 1], w.mask[w.T - 1], w.B, 1
-        else:
-            rows, msk, nb, nt = w.hout.view(w.N, self.H), w.mask.view(-1), w.B, w.T
-        n_loc = rows.shape[0]
-        wg = self.work(nb * comm.world, nt)
-        wg.hout.view(wg.N, self.H).copy_(comm.all_gather_cat(rows.contiguous()))
-        wg.mask.view(-1).copy_(comm.all_gather_cat(msk.contiguous().view(-1)))
-        wg.hscale = None
-        n_splits = self._ce_partials(wg, False, False)
-        call("seqrec_ce_finalize", ptr(wg.ws_m), ptr(wg.ws_s), None, None, ptr(wg.m), ptr(wg.s), None, None, None, None,
-             wg.N, n_splits, self.stream)
-        packed = comm.all_gather_cat(torch.stack([wg.m, wg.s]).unsqueeze(0)).permute(1, 0, 2).contiguous()
-        self._finalize_ce(wg, packed[0], packed[1], comm.world, False)  # catalog-wide (m, s) of every gathered row
-        loc_i, loc_p = self._rank_rows(wg, wg.hout.view(wg.N, self.H), wg.m, wg.s, wg.N, k)
+        wg, _ = self._vp_gather(w, last_step_only, with_targets=False)
+        n_loc = wg.N // comm.world
+        self._vp_merge(wg, with_targets=False)                           # catalog-wide (m, s) of every gathered row
+        loc_i, loc_p = self._topk_rows(wg, k)
         loc_i = loc_i + self.v_lo                                        # global item ids
         # every rank needs the P candidate lists of ITS rows only: one all-to-all (block j of the local result holds
         # rank j's rows), then the same (probability descending, lower id first) merge kernel the 1-GPU ranking ends with
@@ -1169,10 +1177,7 @@ class HotPath:
         top_p = torch.empty((n_loc, k), dtype=torch.float32, device=self.device)
         call("seqrec_topk_merge", ptr(cand_p), ptr(cand_i), comm.world, n_loc * k, ptr(top_i), ptr(top_p), n_loc, k,
              self.stream)
-        if last_step_only:
-            return top_i, top_p
-        return (top_i.view(w.T, w.B, k).permute(1, 0, 2).contiguous(),
-                top_p.view(w.T, w.B, k).permute(1, 0, 2).contiguous())
+        return top_i, top_p
 
     # ------------------------------------------------------------------------------------------------ gradients only
     def grad_batch(self, ids, tgt, x_dense=None, fused=None):
@@ -1231,10 +1236,7 @@ class HotPath:
         """Continues the masked recurrence of a batch of sessions over a left-padded chunk of new events (B,T') and
         returns the state after it (fresh tensors).  state None = the zero state.  A pad step holds h and c, so an
         all-pad row keeps its state bit for bit; advancing by a and then by b equals advancing by a|b bit for bit."""
-        B, T = (ids.shape if ids is not None else x_dense.shape[:2])
-        w = self.work(int(B), int(T))
-        self._stage(w, ids, None, x_dense)
-        self._forward_hidden(w, training=False, state=state)
+        w = self._scan_batch(ids, None, x_dense, state)
         return RecurrentState(w.hout[w.T - 1].clone(), w.cst[w.T - 1].clone() if self.cell == "LSTM" else None,
                               self.cell, self.H)
 
@@ -1265,39 +1267,53 @@ class HotPath:
 
     def target_prob_from_state(self, state, tgt):
         """p(tgt[i] is the next item of session i), (n,) clipped like target_prob_batch."""
-        wl = self._state_work(state, tgt)
-        if self.vocab_parallel:
-            wg = self._vp_forward(wl, training=False)
-            lo = self.comm.rank * wl.N
-            return wg.py[lo:lo + wl.N].clone()
-        self._forward_ce(wl)
-        return wl.py.clone()
+        return self._target_prob(self._state_work(state, tgt)).clone()
 
     def target_rank_from_state(self, state, tgt):
         """(n,) int32 rank of tgt[i] after session i's state, as target_rank_batch(last_step_only=True)."""
-        wl = self._state_work(state, tgt)
-        if self.vocab_parallel:
-            return self._rank_vp(wl, True)
-        return self._target_rank(wl)
+        return self._rank_scored(self._state_work(state, tgt), True)
 
     # ------------------------------------------------------------------------------------------------ scoring
-    def hidden_batch(self, ids, x_dense=None, initial_state=None):
-        """(B,T,H) hidden outputs (z_to_z_output activations), inference phase."""
+    # Every scorer: stage the batch and scan (_scan_batch; the *_from_state scorers build their (n, 1) problem with
+    # _state_work instead), score every step or the last one (_target_prob, _rank_scored, _topk_scored: the only places
+    # that tell a vocabulary-parallel model from a replicated one), lay the time-major results out per session.
+    def _scan_batch(self, ids, tgt, x_dense=None, initial_state=None):
+        """Stages a (B,T) batch and runs the inference scan from initial_state (None = zeros); returns the work object."""
         B, T = (ids.shape if ids is not None else x_dense.shape[:2])
         w = self.work(int(B), int(T))
-        self._stage(w, ids, None, x_dense)
+        self._stage(w, ids, tgt, x_dense)
         self._forward_hidden(w, training=False, state=initial_state)
-        return w.hout.permute(1, 0, 2).contiguous()
+        return w
+
+    def _per_session(self, x, w):
+        """Time-major results of w's tokens (N, ...) laid out per session, (B, T, ...), in storage of their own.  (When
+        T or B is 1 the transposed view of a work buffer is contiguous already: .contiguous() would return the buffer.)"""
+        x = x.view((w.T, w.B) + tuple(x.shape[1:])).transpose(0, 1)
+        return x.clone(memory_format=torch.contiguous_format)
+
+    def _last_step(self, w, with_targets=False):
+        """The (B, 1) problem over the rows hout[T-1] of w (step T-1 of every session), with their mask and, when the
+        call has targets, their targets."""
+        wl = self.work(w.B, 1)
+        if wl is not w:
+            wl.hout.copy_(w.hout[w.T - 1:w.T])
+            wl.mask.copy_(w.mask[w.T - 1:w.T])
+            if with_targets:
+                wl.tgt.copy_(w.tgt[w.T - 1:w.T])
+        wl.hscale = None
+        return wl
+
+    def hidden_batch(self, ids, x_dense=None, initial_state=None):
+        """(B,T,H) hidden outputs (z_to_z_output activations), inference phase."""
+        w = self._scan_batch(ids, None, x_dense, initial_state)
+        return self._per_session(w.hout.view(w.N, self.H), w)
 
     def predict_batch(self, ids, x_dense=None):
         """model.predict: (B,T,V) float32 softmax probabilities on the device."""
         if self.vocab_parallel:
             raise NotImplementedError("a vocabulary-parallel model never materialises (B,T,V): use topk_batch / "
                                       "target_prob_batch, or gather the weights into a replicated model")
-        B, T = (ids.shape if ids is not None else x_dense.shape[:2])
-        w = self.work(int(B), int(T))
-        self._stage(w, ids, None, x_dense)
-        self._forward_hidden(w, training=False)
+        w = self._scan_batch(ids, None, x_dense)
         probs = torch.empty((w.B, w.T, self.V), dtype=torch.float32, device=self.device)
         if w.tc["panel"]:
             # hidden sizes above 256: logits through the plain GEMM (model.predict materialises (N,V) by definition)
@@ -1312,17 +1328,16 @@ class HotPath:
     def target_prob_batch(self, ids, tgt, x_dense=None, initial_state=None):
         """p(true next item) per step, clipped to [1e-7, 1-1e-7] like model.py:108-110; (B,T) device tensor.
         initial_state: the sessions' RecurrentState the chunk continues (None = zeros)."""
-        B, T = (ids.shape if ids is not None else x_dense.shape[:2])
-        w = self.work(int(B), int(T))
-        self._stage(w, ids, tgt, x_dense)
-        self._forward_hidden(w, training=False, state=initial_state)
+        w = self._scan_batch(ids, tgt, x_dense, initial_state)
+        return self._per_session(self._target_prob(w), w)
+
+    def _target_prob(self, w):
+        """(N,) p(target) of w's tokens, time-major (a view of a work buffer)."""
         if self.vocab_parallel:
             # every rank scores all ranks' tokens against its item shard; the merged statistics cover the whole catalog
-            wg = self._vp_forward(w, training=False)
-            lo = self.comm.rank * w.N
-            return wg.py[lo:lo + w.N].view(w.T, w.B).t().contiguous()
+            return self._my_rows(self._vp_forward(w, training=False).py)
         self._forward_ce(w)
-        return w.py.view(w.T, w.B).t().contiguous()
+        return w.py
 
     # ------------------------------------------------------------------------------------------------ target rank
     def _stage_rows_operands(self, w):
@@ -1381,18 +1396,7 @@ class HotPath:
         target (global ids, id_offset = the shard's first item) against the catalog-wide reference logit (computed on
         the target's owner shard, summed over the shards); the integer counts are summed over the shards."""
         comm = self.comm
-        if last_step_only:
-            rows, tg, nb, nt = w.hout[w.T - 1], w.tgt[w.T - 1], w.B, 1
-        else:
-            rows, tg, nb, nt = w.hout.view(w.N, self.H), w.tgt.view(-1), w.B, w.T
-        n_loc = rows.shape[0]
-        wg = self.work(nb * comm.world, nt)
-        wg.hout.view(wg.N, self.H).copy_(comm.all_gather_cat(rows.contiguous()))
-        wg.hscale = None
-        tgt_all = comm.all_gather_cat(tg.contiguous().view(-1))
-        local = (tgt_all >= self.v_lo) & (tgt_all < self.v_lo + self.V)
-        wg.tgt.view(-1).copy_(torch.where(local, tgt_all - self.v_lo, torch.full_like(tgt_all, -1)))
-        wg.zy.zero_()
+        wg, tgt_all = self._vp_gather(w, last_step_only)
         call("seqrec_target_logit", ptr(wg.hout), None, ptr(self.W_out), ptr(self.b_out), ptr(wg.tgt), ptr(wg.zy),
              wg.N, self.H, self.V, None, None, self.stream)
         comm.all_reduce_sum(wg.zy)                        # only the owner shard contributes: the exact fp32 z_y
@@ -1400,9 +1404,7 @@ class HotPath:
         counts = torch.zeros(wg.N, dtype=torch.int32, device=self.device)
         self._rank_rows_count(wg, wg.zy, counts, self.v_lo)
         comm.all_reduce_sum(counts)
-        lo = comm.rank * n_loc
-        rank = counts[lo:lo + n_loc] + (tg.reshape(-1) >= 0).to(torch.int32)
-        return rank if last_step_only else rank.view(w.T, w.B).t().contiguous()
+        return self._my_rows(counts) + (self._my_rows(tgt_all) >= 0).to(torch.int32)
 
     def target_rank_batch(self, ids, tgt, x_dense=None, last_step_only=False, initial_state=None):
         """Rank of the true next item per step: (B,T) int32 device tensor, or (B,) for the last step only.
@@ -1411,22 +1413,16 @@ class HotPath:
         with the exact fp32 target logit, so the rank is exact outside the band of the split-product error around z_y,
         and p(target) of the same rows is left in the work object's `py` by the same pass.
         initial_state: the sessions' RecurrentState the chunk continues (None = zeros)."""
-        B, T = (ids.shape if ids is not None else x_dense.shape[:2])
-        w = self.work(int(B), int(T))
-        self._stage(w, ids, tgt, x_dense)
-        self._forward_hidden(w, training=False, state=initial_state)
+        w = self._scan_batch(ids, tgt, x_dense, initial_state)
+        return self._rank_scored(w, last_step_only)
+
+    def _rank_scored(self, w, last_step_only):
+        """Target ranks of every step of w, (B,T), or of its last step, (B,)."""
         if self.vocab_parallel:
-            return self._rank_vp(w, last_step_only)
-        if last_step_only:
-            # a (B, 1) problem over the rows hout[T-1], like topk_batch(last_step_only=True)
-            wl = self.work(int(B), 1)
-            if wl is not w:
-                wl.hout.copy_(w.hout[w.T - 1:w.T])
-                wl.mask.copy_(w.mask[w.T - 1:w.T])
-                wl.tgt.copy_(w.tgt[w.T - 1:w.T])
-            wl.hscale = None
-            return self._target_rank(wl)
-        return self._target_rank(w).view(w.T, w.B).t().contiguous()
+            rank = self._rank_vp(w, last_step_only)
+        else:
+            rank = self._target_rank(self._last_step(w, with_targets=True) if last_step_only else w)
+        return rank if last_step_only else self._per_session(rank, w)
 
     def _wide_logits(self, rows):
         """Hidden sizes above 256: logits of `rows` (n, H) materialised through the plain GEMM (tcgen05 when it fills
@@ -1442,41 +1438,24 @@ class HotPath:
     def topk_batch(self, ids, k, last_step_only=True, x_dense=None, initial_state=None):
         """Top-k next items: (B,k) ids and probabilities for the last step, or (B,T,k) for every step.
         initial_state: the sessions' RecurrentState the chunk continues (None = zeros)."""
-        B, T = (ids.shape if ids is not None else x_dense.shape[:2])
-        w = self.work(int(B), int(T))
-        self._stage(w, ids, None, x_dense)
-        self._forward_hidden(w, training=False, state=initial_state)
+        w = self._scan_batch(ids, None, x_dense, initial_state)
         return self._topk_scored(w, int(k), last_step_only)
 
     def _topk_scored(self, w, k, last_step_only):
         """Top-k of the rows of w.hout (all steps, or the last one)."""
-        B = w.B
         if self.vocab_parallel:
-            return self._topk_vp(w, int(k), last_step_only)
-        if w.tc["panel"]:
-            rows = w.hout[w.T - 1] if last_step_only else w.hout.view(w.N, self.H)
-            Z, m, s_ = self._wide_logits(rows)
-            order = torch.sort(Z, dim=1, descending=True, stable=True)      # ties: the lower item id first
-            top_i = order.indices[:, :k].to(torch.int32).contiguous()
-            top_p = torch.exp(order.values[:, :k] - m.unsqueeze(1)) / s_.unsqueeze(1)
-            if last_step_only:
-                return top_i, top_p.contiguous()
-            return (top_i.view(w.T, w.B, k).permute(1, 0, 2).contiguous(),
-                    top_p.view(w.T, w.B, k).permute(1, 0, 2).contiguous())
-        if last_step_only:
-            # softmax statistics of the last step only: a (B, 1) problem over the rows hout[T-1]
-            wl = self.work(int(B), 1)
-            if wl is not w:
-                wl.hout.copy_(w.hout[w.T - 1:w.T])
-                wl.mask.copy_(w.mask[w.T - 1:w.T])
-            wl.hscale = None
-            self._forward_ce(wl, with_targets=False)
-            hrows, m, s, n = wl.hout[0], wl.m, wl.s, wl.B
+            top_i, top_p = self._topk_vp(w, k, last_step_only)
         else:
-            self._forward_ce(w, with_targets=False)
-            hrows, m, s, n = w.hout, w.m, w.s, w.N
-        out_i, out_p = self._rank_rows(wl if last_step_only else w, hrows, m, s, n, int(k))
+            wt = self._last_step(w) if last_step_only else w
+            if wt.tc["panel"]:
+                Z, m, s_ = self._wide_logits(wt.hout.view(wt.N, self.H))
+                order = torch.sort(Z, dim=1, descending=True, stable=True)      # ties: the lower item id first
+                top_i = order.indices[:, :k].to(torch.int32).contiguous()
+                top_p = (torch.exp(order.values[:, :k] - m.unsqueeze(1)) / s_.unsqueeze(1)).contiguous()
+            else:
+                # softmax statistics of the rows to rank (the last step: a (B, 1) problem over the rows hout[T-1])
+                self._forward_ce(wt, with_targets=False)
+                top_i, top_p = self._topk_rows(wt, k)
         if last_step_only:
-            return out_i, out_p
-        return (out_i.view(w.T, w.B, k).permute(1, 0, 2).contiguous(),
-                out_p.view(w.T, w.B, k).permute(1, 0, 2).contiguous())
+            return top_i, top_p
+        return self._per_session(top_i, w), self._per_session(top_p, w)
