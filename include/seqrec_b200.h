@@ -347,7 +347,7 @@ int seqrec_likelihood_cut(const float* P, const int32_t* lengths, int64_t n_seqs
  * doubles) pre-zeroed.  Recall@k = out[3q] / n, MRR@k = out[3q+1] / n, NDCG@k = out[3q+2] / n. */
 int seqrec_rank_metrics(const int32_t* rank, int64_t n, const int32_t* ks, int n_ks, double* out, void* stream);
 
-/* ---- K8: global-norm clip + Adagrad (experiments_methods.py:41) -------------------------------------------------
+/* ---- K8: global-norm clip + Adagrad (experiments_methods.py:41) or Adam -----------------------------------------
  * sumsq[0] (double, pre-zeroed) += sum g^2 */
 int seqrec_sumsq(const float* g, int64_t n, double* sumsq, void* stream);
 int seqrec_sumsq_rows(const float* g, const int32_t* rows, const int32_t* n_rows, int GH, int max_rows,
@@ -362,6 +362,20 @@ int seqrec_adagrad(float* p, const float* g, float* a, int64_t n, float lr, floa
 int seqrec_adagrad_rows(float* p, float* g, float* a, const int32_t* rows, const int32_t* n_rows, int32_t* touched,
                         int GH, int max_rows, float lr, float eps, float clipnorm, const double* sumsq,
                         const float* gdenom, void* stream);
+/* Keras 2.0.x Adam with the same clip and 1/gdenom factor: g' = g * scale (scale as for seqrec_adagrad);
+ * k = iterations[0] (device int64: updates applied before this one, advanced by the caller after the step, so a
+ * launch captured in a CUDA graph uses the current k at every replay; never written here);
+ * lr_e = lr / (1 + decay*k); lr_t = lr_e * sqrt(1 - beta_2^(k+1)) / (1 - beta_1^(k+1)) (double, once per block);
+ * m = beta_1*m + (1-beta_1)*g'; v = beta_2*v + (1-beta_2)*g'^2; p -= lr_t * m / (sqrt(v) + eps) */
+int seqrec_adam(float* p, const float* g, float* m, float* v, int64_t n, float lr, float beta_1, float beta_2,
+                float eps, float decay, float clipnorm, const double* sumsq, const float* gdenom,
+                const int64_t* iterations, void* stream);
+/* the same update over EVERY row of an (F, GH) table (dense semantics: untouched rows take g' = 0, their m and v
+ * decay and p still moves); the gradient row is read only where touched[row] != 0, and those rows of g and their
+ * touched flags are re-zeroed */
+int seqrec_adam_table(float* p, float* g, float* m, float* v, int32_t* touched, int64_t F, int GH, float lr,
+                      float beta_1, float beta_2, float eps, float decay, float clipnorm, const double* sumsq,
+                      const float* gdenom, const int64_t* iterations, void* stream);
 
 /* ---- Dropout (model.py:362-363, :371-372): inverted-dropout factors from a counter-based RNG ---------------------
  * out[i] = (u_i >= rate) ? 1/(1-rate) : 0 */

@@ -80,6 +80,8 @@ SIGNATURES = {
     "seqrec_sumsq_rows": [_p, _p, _p, _i, _i, _p, _p],
     "seqrec_adagrad": [_p, _p, _p, _l, _f, _f, _f, _p, _p, _p],
     "seqrec_adagrad_rows": [_p, _p, _p, _p, _p, _p, _i, _i, _f, _f, _f, _p, _p, _p],
+    "seqrec_adam": [_p, _p, _p, _p, _l, _f, _f, _f, _f, _f, _f, _p, _p, _p, _p],
+    "seqrec_adam_table": [_p, _p, _p, _p, _p, _l, _i, _f, _f, _f, _f, _f, _f, _p, _p, _p, _p],
     "seqrec_dropout_mask": [_p, _l, _f, _u64, _u64, _p],
     "seqrec_dropout_mask_dev": [_p, _l, _f, _u64, _p, _p],
     "seqrec_split_bf16": [_p, _p, _p, _p, _l, _l, _l, _i, _p],

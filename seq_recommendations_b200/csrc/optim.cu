@@ -1,5 +1,6 @@
 // K8: global-norm clip + Adagrad, dense and row-sparse (experiments_methods.py:41:
-// Adagrad(lr, epsilon=1e-08, decay=0.0, clipnorm=1.)), plus the dropout-factor generator and the bf16 hi/lo splitter
+// Adagrad(lr, epsilon=1e-08, decay=0.0, clipnorm=1.)), clip + Keras Adam (compile_model's default optimizer, dense and
+// over a whole embedding table), plus the dropout-factor generator and the bf16 hi/lo splitter
 // that stages operands for the tensor-core logits kernels.  All HBM-bound elementwise passes.
 #include "common.cuh"
 
@@ -176,6 +177,146 @@ extern "C" int seqrec_adagrad_rows(float* p, float* g, float* a, const int32_t* 
   SEQREC_ARG(GH > 0 && max_rows > 0, 1);
   adagrad_rows_kernel<<<grid_for(max_rows, 8), 256, 0, as_stream(stream)>>>(p, g, a, rows, n_rows, touched, GH, lr,
                                                                             eps, clipnorm, sumsq, gdenom);
+  SEQREC_CHECK_LAUNCH();
+  return 0;
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// Keras 2.0.x Adam.  iterations[0] (device int64) = updates applied before this one; it is read here and advanced by
+// the caller after the step, so a launch captured in a CUDA graph uses the current t at every replay.  The bias-
+// corrected rate is computed in double once per block.
+__device__ __forceinline__ float adam_lr_t(float lr, float beta_1, float beta_2, float decay,
+                                           const int64_t* __restrict__ iterations) {
+  __shared__ float lr_t;
+  if (threadIdx.x == 0) {
+    const double k = (double)iterations[0];
+    const double lr_e = decay > 0.f ? (double)lr / (1.0 + (double)decay * k) : (double)lr;
+    lr_t = (float)(lr_e * sqrt(1.0 - pow((double)beta_2, k + 1.0)) / (1.0 - pow((double)beta_1, k + 1.0)));
+  }
+  __syncthreads();
+  return lr_t;
+}
+
+__device__ __forceinline__ void adam_one(float& p, float g, float& m, float& v, float lr_t, float b1, float b2,
+                                         float eps) {
+  m = b1 * m + (1.f - b1) * g;
+  v = b2 * v + (1.f - b2) * (g * g);
+  p -= lr_t * m / (sqrtf(v) + eps);
+}
+
+__device__ __forceinline__ void adam_four(float4& p, float4 g, float4& m, float4& v, float lr_t, float b1, float b2,
+                                          float eps) {
+  adam_one(p.x, g.x, m.x, v.x, lr_t, b1, b2, eps);
+  adam_one(p.y, g.y, m.y, v.y, lr_t, b1, b2, eps);
+  adam_one(p.z, g.z, m.z, v.z, lr_t, b1, b2, eps);
+  adam_one(p.w, g.w, m.w, v.w, lr_t, b1, b2, eps);
+}
+
+__global__ void __launch_bounds__(256)
+adam_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m, float* __restrict__ v, int64_t n,
+            float lr, float b1, float b2, float eps, float decay, float clipnorm, const double* __restrict__ sumsq,
+            const float* __restrict__ gdenom, const int64_t* __restrict__ iterations) {
+  const float lr_t = adam_lr_t(lr, b1, b2, decay, iterations);
+  const float sc = clip_scale(sumsq, clipnorm, gdenom);
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  const int64_t tid = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  const bool vec = ((reinterpret_cast<uintptr_t>(p) | reinterpret_cast<uintptr_t>(g) | reinterpret_cast<uintptr_t>(m) |
+                     reinterpret_cast<uintptr_t>(v)) & 15) == 0;
+  const int64_t n4 = vec ? (n >> 2) : 0;
+  float4* p4 = reinterpret_cast<float4*>(p);
+  const float4* g4 = reinterpret_cast<const float4*>(g);
+  float4* m4 = reinterpret_cast<float4*>(m);
+  float4* v4 = reinterpret_cast<float4*>(v);
+  for (int64_t i = tid; i < n4; i += stride) {
+    float4 gv = g4[i], mv = m4[i], vv = v4[i], pv = p4[i];
+    gv.x *= sc; gv.y *= sc; gv.z *= sc; gv.w *= sc;
+    adam_four(pv, gv, mv, vv, lr_t, b1, b2, eps);
+    m4[i] = mv;
+    v4[i] = vv;
+    p4[i] = pv;
+  }
+  for (int64_t i = (n4 << 2) + tid; i < n; i += stride) {
+    float pv = p[i], mv = m[i], vv = v[i];
+    adam_one(pv, g[i] * sc, mv, vv, lr_t, b1, b2, eps);
+    m[i] = mv;
+    v[i] = vv;
+    p[i] = pv;
+  }
+}
+
+// Every row of the (F, GH) table moves (the reference's one-hot input product has a dense gradient); one warp per row.
+// The gradient row is read only where touched[row] != 0 -- it is all zeros elsewhere -- and is then re-zeroed with its
+// flag, which keeps the zero invariant of the dense gradient buffer that adagrad_rows_kernel keeps.
+__global__ void __launch_bounds__(256)
+adam_table_kernel(float* __restrict__ p, float* __restrict__ g, float* __restrict__ m, float* __restrict__ v,
+                  int32_t* __restrict__ touched, int64_t F, int GH, float lr, float b1, float b2, float eps,
+                  float decay, float clipnorm, const double* __restrict__ sumsq, const float* __restrict__ gdenom,
+                  const int64_t* __restrict__ iterations) {
+  const float lr_t = adam_lr_t(lr, b1, b2, decay, iterations);
+  const float sc = clip_scale(sumsq, clipnorm, gdenom);
+  const int lane = threadIdx.x & 31;
+  const bool vec = (GH & 3) == 0 &&
+                   ((reinterpret_cast<uintptr_t>(p) | reinterpret_cast<uintptr_t>(g) | reinterpret_cast<uintptr_t>(m) |
+                     reinterpret_cast<uintptr_t>(v)) & 15) == 0;
+  const int64_t warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+  for (int64_t row = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5; row < F; row += warps) {
+    int hot = lane == 0 ? touched[row] : 0;
+    hot = __shfl_sync(0xffffffffu, hot, 0);
+    const size_t off = (size_t)row * GH;
+    if (vec) {                                   // 128-bit accesses
+      float4* p4 = reinterpret_cast<float4*>(p + off);
+      float4* g4 = reinterpret_cast<float4*>(g + off);
+      float4* m4 = reinterpret_cast<float4*>(m + off);
+      float4* v4 = reinterpret_cast<float4*>(v + off);
+      for (int c = lane; c < (GH >> 2); c += 32) {
+        float4 gv = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (hot) {
+          gv = g4[c];
+          gv.x *= sc; gv.y *= sc; gv.z *= sc; gv.w *= sc;
+          g4[c] = make_float4(0.f, 0.f, 0.f, 0.f);
+        }
+        float4 mv = m4[c], vv = v4[c], pv = p4[c];
+        adam_four(pv, gv, mv, vv, lr_t, b1, b2, eps);
+        m4[c] = mv;
+        v4[c] = vv;
+        p4[c] = pv;
+      }
+    } else {
+      for (int c = lane; c < GH; c += 32) {
+        float gv = 0.f;
+        if (hot) {
+          gv = g[off + c] * sc;
+          g[off + c] = 0.f;
+        }
+        float pv = p[off + c], mv = m[off + c], vv = v[off + c];
+        adam_one(pv, gv, mv, vv, lr_t, b1, b2, eps);
+        m[off + c] = mv;
+        v[off + c] = vv;
+        p[off + c] = pv;
+      }
+    }
+    if (hot && lane == 0) touched[row] = 0;
+  }
+}
+
+extern "C" int seqrec_adam(float* p, const float* g, float* m, float* v, int64_t n, float lr, float beta_1,
+                           float beta_2, float eps, float decay, float clipnorm, const double* sumsq,
+                           const float* gdenom, const int64_t* iterations, void* stream) {
+  SEQREC_ARG(n > 0, 1);
+  SEQREC_ARG(iterations != nullptr, 14);
+  adam_kernel<<<grid_for(n, 256 * 4), 256, 0, as_stream(stream)>>>(p, g, m, v, n, lr, beta_1, beta_2, eps, decay,
+                                                                     clipnorm, sumsq, gdenom, iterations);
+  SEQREC_CHECK_LAUNCH();
+  return 0;
+}
+
+extern "C" int seqrec_adam_table(float* p, float* g, float* m, float* v, int32_t* touched, int64_t F, int GH,
+                                 float lr, float beta_1, float beta_2, float eps, float decay, float clipnorm,
+                                 const double* sumsq, const float* gdenom, const int64_t* iterations, void* stream) {
+  SEQREC_ARG(F > 0 && GH > 0, 6);
+  SEQREC_ARG(touched != nullptr && iterations != nullptr, 5);
+  adam_table_kernel<<<grid_for(F, 8), 256, 0, as_stream(stream)>>>(p, g, m, v, touched, F, GH, lr, beta_1, beta_2,
+                                                                   eps, decay, clipnorm, sumsq, gdenom, iterations);
   SEQREC_CHECK_LAUNCH();
   return 0;
 }

@@ -14,7 +14,8 @@ HBM layout (all fp32 unless noted; token n = t*B + b, time-major):
             per-step integer scalars (n_valid, touched-row count, squared gradient norm).  One fill clears everything
             behind dW_in at the start of a step; one all-reduce covers [dW_in |] step floats | dU | db.  Gradients are
             stored UN-normalised (sums over tokens); the optimiser kernels divide by the global n_valid
-  accum     Adagrad accumulators, same shapes
+  accum     Adagrad accumulators, same shapes -- or Adam's second moments v, with the first moments m in buffers of
+            the same shapes allocated when Adam is selected, and the update count `iterations` (device int64)
   per batch ids/tgt int32 [T][B], mask u8 [T][B], xg [T][B][G*H] (xp -> gates -> dxp in place),
             hout [T][B][H], cst [T][B][H], dh [T][B][H], per-token stats m,s,zy,ce,py,coef [N], ws [splits][N]
 """
@@ -38,6 +39,19 @@ NUM_SMS = 148
 
 def _align(n, a=64):
     return (n + a - 1) // a * a
+
+
+def _optimizer_spec(kind, lr, epsilon, clipnorm, decay, beta_1, beta_2):
+    """HotPath.opt / DensePath.opt: the hyper-parameters of Adagrad or Keras Adam."""
+    if kind not in ("adagrad", "adam"):
+        raise NotImplementedError("optimizer %r: Adagrad (the reference's, experiments_methods.py:41) and Adam are "
+                                  "built" % (kind,))
+    if kind == "adagrad" and decay:
+        raise NotImplementedError("learning-rate decay is never used by the reference (decay=0.0)")
+    if kind == "adam" and not (0.0 <= beta_1 < 1.0 and 0.0 <= beta_2 < 1.0 and decay >= 0.0):
+        raise ValueError("Adam needs 0 <= beta_1, beta_2 < 1 and decay >= 0")
+    return dict(kind=kind, lr=float(lr), eps=float(epsilon), clipnorm=float(clipnorm or 0.0), decay=float(decay or 0.0),
+                beta_1=float(beta_1), beta_2=float(beta_2))
 
 
 class _Work:
@@ -178,9 +192,14 @@ class HotPath:
 
         self.U, self.b, self.W_out, self.b_out = views(self.flat_p)
         self.dU, self.db, self.dW_out, self.db_out = views(self.flat_g)
-        self.aU, self.ab, self.aW_out, self.ab_out = views(self.flat_a)      # Adagrad accumulators
+        self.aU, self.ab, self.aW_out, self.ab_out = views(self.flat_a)      # Adagrad accumulators / Adam's v
+        self._views = views
         self.W_in = torch.zeros((self.F, self.GH), dtype=f32, device=dev)
         self.aW_in = torch.zeros((self.F, self.GH), dtype=f32, device=dev)
+        # Adam's first moments (flat_m, mW_in and the m* views): allocated when Adam is first selected, then kept, so a
+        # captured step's pointers stay valid.  iterations = updates applied so far, read by the Adam kernels.
+        self.flat_m = self.mU = self.mb = self.mW_out = self.mb_out = self.mW_in = None
+        self.iterations = torch.zeros(1, dtype=torch.int64, device=dev)
         self.Ut = torch.empty((self.GH, self.H), dtype=f32, device=dev)
         self._needs_ut = _lib.load().seqrec_rnn_needs_ut(CELL[cell], self.H) != 0
         # tensor-core recurrent scan (csrc/rnn_tc.cu): LSTM / GRU with H in {128, 256}.  The register-resident SIMT scan
@@ -367,6 +386,21 @@ class HotPath:
     def set_accumulator(self, name, value):
         self.set_weight(name, value, prefix="a")
 
+    def get_moments(self, name):
+        """Adam's (m, v) of one weight, full width (state checkpoints)."""
+        return self.get_weight(name, prefix="m"), self.get_weight(name, prefix="a")
+
+    def set_moments(self, name, m, v):
+        self.set_weight(name, m, prefix="m")
+        self.set_weight(name, v, prefix="a")
+
+    def get_iterations(self):
+        """Optimizer updates applied since set_optimizer (Keras `optimizer.iterations`)."""
+        return int(self.iterations.item())
+
+    def set_iterations(self, k):
+        self.iterations.fill_(int(k))
+
     def get_weight(self, name, prefix=""):
         """One weight by name ('W_in', 'U', 'b', 'W_out', 'b_out') as a full-width float32 numpy array."""
         t = getattr(self, prefix + name)
@@ -391,13 +425,18 @@ class HotPath:
     def reset_optimizer_state(self):
         self.flat_a.zero_()
         self.aW_in.zero_()
+        if self.flat_m is not None:
+            self.flat_m.zero_()
+            self.mW_in.zero_()
+        self.iterations.zero_()
 
-    def set_optimizer(self, kind="adagrad", lr=0.01, epsilon=1e-8, clipnorm=0.0, decay=0.0):
-        if kind != "adagrad":
-            raise NotImplementedError("only Adagrad (the reference's optimizer, experiments_methods.py:41) is built")
-        if decay:
-            raise NotImplementedError("learning-rate decay is never used by the reference (decay=0.0)")
-        self.opt = dict(kind=kind, lr=float(lr), eps=float(epsilon), clipnorm=float(clipnorm or 0.0))
+    def set_optimizer(self, kind="adagrad", lr=0.01, epsilon=1e-8, clipnorm=0.0, decay=0.0, beta_1=0.9, beta_2=0.999):
+        """Adagrad (the reference's optimizer, experiments_methods.py:41) or Keras Adam; resets the optimizer state."""
+        self.opt = _optimizer_spec(kind, lr, epsilon, clipnorm, decay, beta_1, beta_2)
+        if kind == "adam" and self.flat_m is None:
+            self.flat_m = torch.zeros_like(self.flat_a)
+            self.mU, self.mb, self.mW_out, self.mb_out = self._views(self.flat_m)
+            self.mW_in = torch.zeros_like(self.aW_in)
         self.reset_optimizer_state()
 
     # ------------------------------------------------------------------------------------------------ batch ingest
@@ -851,7 +890,8 @@ class HotPath:
         """Everything a captured step bakes in BY VALUE (kernel arguments and which kernels are launched at all)."""
         o = self.opt
         return (o["lr"], o["eps"], o["clipnorm"], tuple(sorted(self.trainable.items())), self.dropout_in,
-                self.dropout_out, self.dropout_rec, self.overlap, self.ce_fused, self.ce_compact, self.rnn_tc, self.wgrad_tc, self.tc_mode, self.tc_x3)
+                self.dropout_out, self.dropout_rec, self.overlap, self.ce_fused, self.ce_compact, self.rnn_tc, self.wgrad_tc, self.tc_mode, self.tc_x3,
+                o["kind"], o["beta_1"], o["beta_2"], o["decay"])
 
     def _train_core(self, w):
         """forward + backward + exchange + update on the staged batch (everything after the host->device copy).
@@ -1072,11 +1112,16 @@ class HotPath:
             call("seqrec_sumsq", ptr(self.flat_g[:head]), head, ptr(self.sumsq), st)
             call("seqrec_sumsq_rows", ptr(self.dW_in), ptr(self.rows), ptr(self.n_rows), self.GH, max_rows,
                  ptr(self.sumsq), st)
-        call("seqrec_adagrad", ptr(self.flat_p), ptr(self.flat_g), ptr(self.flat_a), self.flat_p.numel(), o["lr"],
-             o["eps"], o["clipnorm"], ptr(self.sumsq), ptr(self.n_valid_f), st)
-        call("seqrec_adagrad_rows", ptr(self.W_in), ptr(self.dW_in), ptr(self.aW_in), ptr(self.rows), ptr(self.n_rows),
-             ptr(self.touched), self.GH, max_rows, o["lr"], o["eps"], o["clipnorm"], ptr(self.sumsq),
-             ptr(self.n_valid_f), st)
+        if o["kind"] == "adam":
+            self._adam(self.flat_p, self.flat_g, self.flat_m, self.flat_a, st)
+            self._adam_table(st)
+            self.iterations.add_(1)
+        else:
+            call("seqrec_adagrad", ptr(self.flat_p), ptr(self.flat_g), ptr(self.flat_a), self.flat_p.numel(), o["lr"],
+                 o["eps"], o["clipnorm"], ptr(self.sumsq), ptr(self.n_valid_f), st)
+            call("seqrec_adagrad_rows", ptr(self.W_in), ptr(self.dW_in), ptr(self.aW_in), ptr(self.rows),
+                 ptr(self.n_rows), ptr(self.touched), self.GH, max_rows, o["lr"], o["eps"], o["clipnorm"],
+                 ptr(self.sumsq), ptr(self.n_valid_f), st)
         self._w_version += 1
         loss = wg.loss_mean if torch.cuda.is_current_stream_capturing() else wg.loss_mean.clone()
         self._mark("end")
@@ -1111,30 +1156,60 @@ class HotPath:
                     if self.trainable[n]:
                         call("seqrec_sumsq", ptr(self.flat_g[off:off + sz]), sz, ptr(self.sumsq), st)
             self._join()
+        adam = o["kind"] == "adam"
         with self._branch():
             if w.x_dense is None:
                 if self.trainable["W_in"]:
                     # also re-zeroes the touched rows of dW_in and their flags (zero invariant of the dense buffer)
-                    call("seqrec_adagrad_rows", ptr(self.W_in), ptr(self.dW_in), ptr(self.aW_in), ptr(self.rows),
-                         ptr(self.n_rows), ptr(self.touched), self.GH, max_rows, o["lr"], o["eps"], o["clipnorm"],
-                         ptr(self.sumsq), den, self.stream)
+                    if adam:
+                        self._adam_table(self.stream)
+                    else:
+                        call("seqrec_adagrad_rows", ptr(self.W_in), ptr(self.dW_in), ptr(self.aW_in), ptr(self.rows),
+                             ptr(self.n_rows), ptr(self.touched), self.GH, max_rows, o["lr"], o["eps"], o["clipnorm"],
+                             ptr(self.sumsq), den, self.stream)
                 else:
                     self.dW_in.zero_()
                     self.touched.zero_()
             else:
                 if self.trainable["W_in"]:
-                    call("seqrec_adagrad", ptr(self.W_in), ptr(self.dW_in), ptr(self.aW_in), self.W_in.numel(), o["lr"],
-                         o["eps"], o["clipnorm"], ptr(self.sumsq), den, self.stream)
+                    if adam:
+                        self._adam(self.W_in, self.dW_in, self.mW_in, self.aW_in, self.stream)
+                    else:
+                        call("seqrec_adagrad", ptr(self.W_in), ptr(self.dW_in), ptr(self.aW_in), self.W_in.numel(),
+                             o["lr"], o["eps"], o["clipnorm"], ptr(self.sumsq), den, self.stream)
                 self.dW_in.zero_()
         if all_dense:
-            call("seqrec_adagrad", ptr(self.flat_p), ptr(self.flat_g), ptr(self.flat_a), self.flat_p.numel(), o["lr"],
-                 o["eps"], o["clipnorm"], ptr(self.sumsq), den, st)
+            if adam:
+                self._adam(self.flat_p, self.flat_g, self.flat_m, self.flat_a, st)
+            else:
+                call("seqrec_adagrad", ptr(self.flat_p), ptr(self.flat_g), ptr(self.flat_a), self.flat_p.numel(),
+                     o["lr"], o["eps"], o["clipnorm"], ptr(self.sumsq), den, st)
         else:
             for n, off, sz in segs:
                 if self.trainable[n]:
-                    call("seqrec_adagrad", ptr(self.flat_p[off:off + sz]), ptr(self.flat_g[off:off + sz]),
-                         ptr(self.flat_a[off:off + sz]), sz, o["lr"], o["eps"], o["clipnorm"], ptr(self.sumsq), den, st)
+                    if adam:
+                        self._adam(self.flat_p[off:off + sz], self.flat_g[off:off + sz], self.flat_m[off:off + sz],
+                                   self.flat_a[off:off + sz], st)
+                    else:
+                        call("seqrec_adagrad", ptr(self.flat_p[off:off + sz]), ptr(self.flat_g[off:off + sz]),
+                             ptr(self.flat_a[off:off + sz]), sz, o["lr"], o["eps"], o["clipnorm"], ptr(self.sumsq),
+                             den, st)
         self._join()
+        if adam:
+            self.iterations.add_(1)               # after both halves: each read the count of the updates before it
+
+    def _adam(self, p, g, m, v, st):
+        """Dense Adam over p (the flat buffer, one of its segments or the dense W_in of the x_dense input path)."""
+        o = self.opt
+        call("seqrec_adam", ptr(p), ptr(g), ptr(m), ptr(v), p.numel(), o["lr"], o["beta_1"], o["beta_2"], o["eps"],
+             o["decay"], o["clipnorm"], ptr(self.sumsq), ptr(self.n_valid_f), ptr(self.iterations), st)
+
+    def _adam_table(self, st):
+        """Adam over every row of the W_in table; reads and re-zeroes only the touched rows of dW_in."""
+        o = self.opt
+        call("seqrec_adam_table", ptr(self.W_in), ptr(self.dW_in), ptr(self.mW_in), ptr(self.aW_in), ptr(self.touched),
+             self.F, self.GH, o["lr"], o["beta_1"], o["beta_2"], o["eps"], o["decay"], o["clipnorm"], ptr(self.sumsq),
+             ptr(self.n_valid_f), ptr(self.iterations), st)
 
     def _topk_rows(self, wt, k):
         """Top-k of the wt.N rows of wt.hout against THIS rank's items (ids are local item indices), probabilities from

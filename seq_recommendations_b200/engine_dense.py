@@ -23,7 +23,7 @@ import torch
 from . import _lib
 from ._lib import ACT, CELL, call, ptr
 from .dist import Comm
-from .engine import GATES, _align
+from .engine import GATES, _align, _optimizer_spec
 from .gemm import gemm
 
 NAMES = ["W_in", "U", "b", "W_toy", "b_out", "A", "a_bias"]
@@ -99,6 +99,8 @@ class DensePath:
                 setattr(self, n, None)
                 setattr(self, "d" + n, None)
         self.trainable = {n: True for n in self._seg}
+        self.flat_m = None                        # Adam's first moments (m* views), allocated when Adam is selected
+        self.iterations = torch.zeros(1, dtype=torch.int64, device=dev)
         self.Ut = torch.empty((self.GH, self.H), dtype=f32, device=dev) if cell else None
         # scratch of the row scatter-adds (dense destinations: the flags are cleared after every use)
         nrow = max(self.V, 1)
@@ -136,6 +138,19 @@ class DensePath:
     def set_accumulator(self, name, value):
         self.set_weight(name, value, prefix="a")
 
+    def get_moments(self, name):
+        return self.get_weight(name, prefix="m"), self.get_weight(name, prefix="a")
+
+    def set_moments(self, name, m, v):
+        self.set_weight(name, m, prefix="m")
+        self.set_weight(name, v, prefix="a")
+
+    def get_iterations(self):
+        return int(self.iterations.item())
+
+    def set_iterations(self, k):
+        self.iterations.fill_(int(k))
+
     def get_weights(self):
         return [self.get_weight(n) for n in self.weight_names()]
 
@@ -148,13 +163,17 @@ class DensePath:
 
     def reset_optimizer_state(self):
         self.flat_a.zero_()
+        if self.flat_m is not None:
+            self.flat_m.zero_()
+        self.iterations.zero_()
 
-    def set_optimizer(self, kind="adagrad", lr=0.01, epsilon=1e-8, clipnorm=0.0, decay=0.0):
-        if kind != "adagrad":
-            raise NotImplementedError("only Adagrad (the reference's optimizer, experiments_methods.py:41) is built")
-        if decay:
-            raise NotImplementedError("learning-rate decay is never used by the reference (decay=0.0)")
-        self.opt = dict(kind=kind, lr=float(lr), eps=float(epsilon), clipnorm=float(clipnorm or 0.0))
+    def set_optimizer(self, kind="adagrad", lr=0.01, epsilon=1e-8, clipnorm=0.0, decay=0.0, beta_1=0.9, beta_2=0.999):
+        """Adagrad (the reference's optimizer, experiments_methods.py:41) or Keras Adam; resets the optimizer state."""
+        self.opt = _optimizer_spec(kind, lr, epsilon, clipnorm, decay, beta_1, beta_2)
+        if kind == "adam" and self.flat_m is None:
+            self.flat_m = torch.zeros_like(self.flat_a)
+            for n, (off, size, shp) in self._seg.items():
+                setattr(self, "m" + n, self.flat_m[off:off + size].view(shp))
         self.reset_optimizer_state()
 
     def check_errors(self):
@@ -367,7 +386,13 @@ class DensePath:
                 for n, off, sz in segs:
                     if self.trainable[n]:
                         call("seqrec_sumsq", ptr(self.flat_g[off:off + sz]), sz, ptr(self.sumsq), st)
-        if all_on:
+        if o["kind"] == "adam":
+            for off, sz in ([(0, self.flat_p.numel())] if all_on else
+                            [(off, sz) for n, off, sz in segs if self.trainable[n]]):
+                call("seqrec_adam", ptr(self.flat_p[off:off + sz]), ptr(self.flat_g[off:off + sz]),
+                     ptr(self.flat_m[off:off + sz]), ptr(self.flat_a[off:off + sz]), sz, o["lr"], o["beta_1"],
+                     o["beta_2"], o["eps"], o["decay"], o["clipnorm"], ptr(self.sumsq), den, ptr(self.iterations), st)
+        elif all_on:
             call("seqrec_adagrad", ptr(self.flat_p), ptr(self.flat_g), ptr(self.flat_a), self.flat_p.numel(), o["lr"],
                  o["eps"], o["clipnorm"], ptr(self.sumsq), den, st)
         else:
@@ -378,6 +403,8 @@ class DensePath:
         if self.x_to_y and self.diag_b and self.trainable.get("W_toy", False):
             # Keras applies the kernel constraint to the UPDATED weights (model.py:379, :300-301)
             call("seqrec_diag_constraint", ptr(self.W_toy), self.H, self.V, st)
+        if o["kind"] == "adam":
+            self.iterations.add_(1)
         self._w_version += 1
 
     # ------------------------------------------------------------------------------------------------ public steps

@@ -207,23 +207,45 @@ class _Net(object):
             self.set_weights([z["weight%d" % i] for i in range(n)])
 
     def save_state(self, filepath, epoch=0):
-        """Resumable checkpoint (not in the reference, whose checkpoints restart Adagrad): weights, the Adagrad
-        accumulators of every weight, the optimizer hyper-parameters and the epoch counter."""
+        """Resumable checkpoint (not in the reference, whose checkpoints restart Adagrad): weights, the optimizer state
+        of every weight, the optimizer hyper-parameters and the epoch counter.  Adagrad: `accum{i}` and
+        opt = [lr, epsilon, clipnorm].  Adam: opt_kind = 'adam', opt = [lr, beta_1, beta_2, epsilon, clipnorm, decay],
+        `iterations` and the moments `m{i}`, `v{i}` (i in get_weights() order)."""
         arrays = {"weight%d" % i: w for i, w in enumerate(self.get_weights())}
-        for i, n in enumerate(self._names()):
-            arrays["accum%d" % i] = self.hot.get_accumulator(n)
         o = self.hot.opt or {}
         arrays["epoch"] = np.asarray(int(epoch))
-        arrays["opt"] = np.asarray([o.get("lr", 0.0), o.get("eps", 0.0), o.get("clipnorm", 0.0)], dtype=np.float64)
+        if o.get("kind") == "adam":
+            for i, n in enumerate(self._names()):
+                arrays["m%d" % i], arrays["v%d" % i] = self.hot.get_moments(n)
+            arrays["opt_kind"] = np.asarray("adam")
+            arrays["opt"] = np.asarray([o["lr"], o["beta_1"], o["beta_2"], o["eps"], o["clipnorm"], o["decay"]],
+                                       dtype=np.float64)
+            arrays["iterations"] = np.asarray(self.hot.get_iterations(), dtype=np.int64)
+        else:
+            for i, n in enumerate(self._names()):
+                arrays["accum%d" % i] = self.hot.get_accumulator(n)
+            arrays["opt"] = np.asarray([o.get("lr", 0.0), o.get("eps", 0.0), o.get("clipnorm", 0.0)], dtype=np.float64)
         self._write_npz(self._npz_path(filepath), arrays)
 
     def load_state(self, filepath):
-        """Inverse of save_state; returns the stored epoch.  compile() first (it resets the accumulators)."""
+        """Inverse of save_state; returns the stored epoch.  compile() first (it resets the optimizer state), with the
+        optimizer the checkpoint was written with: a different one raises ValueError.  An archive without `opt_kind`
+        is an Adagrad checkpoint."""
         with self._open_npz(filepath) as z:
+            kind = str(z["opt_kind"]) if "opt_kind" in z.files else "adagrad"
+            compiled = (self.hot.opt or {}).get("kind", "adagrad")
+            if kind != compiled:
+                raise ValueError("%s holds %s optimizer state but the model is compiled with %s: compile it with the "
+                                 "checkpoint's optimizer first" % (filepath, kind, compiled))
             names = self._names()
             self.set_weights([z["weight%d" % i] for i in range(len(names))])
             for i, n in enumerate(names):
-                self.hot.set_accumulator(n, z["accum%d" % i])
+                if kind == "adam":
+                    self.hot.set_moments(n, z["m%d" % i], z["v%d" % i])
+                else:
+                    self.hot.set_accumulator(n, z["accum%d" % i])
+            if kind == "adam":
+                self.hot.set_iterations(int(z["iterations"]))
             return int(z["epoch"])
 
     # ---- compile -------------------------------------------------------------------------------------------------
@@ -235,8 +257,12 @@ class _Net(object):
         self.metrics_names = ["loss"] + [m for m in (metrics or []) if isinstance(m, str)]
         if not isinstance(self.optimizer, str):
             o = self.optimizer
-            self.hot.set_optimizer("adagrad", lr=o.lr, epsilon=o.epsilon, clipnorm=getattr(o, "clipnorm", None) or 0.0,
-                                   decay=getattr(o, "decay", 0.0))
+            if optimizers.kind_of(o) == "adam":
+                self.hot.set_optimizer("adam", lr=o.lr, epsilon=o.epsilon, clipnorm=getattr(o, "clipnorm", None) or 0.0,
+                                       decay=getattr(o, "decay", 0.0), beta_1=o.beta_1, beta_2=o.beta_2)
+            else:
+                self.hot.set_optimizer("adagrad", lr=o.lr, epsilon=o.epsilon,
+                                       clipnorm=getattr(o, "clipnorm", None) or 0.0, decay=getattr(o, "decay", 0.0))
 
     # ---- batches -------------------------------------------------------------------------------------------------
     def _inputs(self, x):
@@ -301,8 +327,8 @@ class _Net(object):
     # ---- Keras Model methods ------------------------------------------------------------------------------------
     def fit(self, x, y, validation_data=None, epochs=10, batch_size=100, verbose=1, callbacks=None, shuffle=True):
         if isinstance(self.optimizer, str) or self.optimizer is None:
-            raise NotImplementedError("training needs an Adagrad optimizer object (experiments_methods.py:41); got %r"
-                                      % (self.optimizer,))
+            raise NotImplementedError("training needs an optimizer object: optimizers.Adagrad(...) (experiments_methods.py:41) "
+                                      "or optimizers.Adam(...); got %r" % (self.optimizer,))
         ids, xd = self._inputs(x)
         tgt = to_id_batch(y)
         self.hot._check_host_ids(ids, tgt)
