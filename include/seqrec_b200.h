@@ -301,6 +301,24 @@ int seqrec_topk_tc(const uint16_t* A_hi, const uint16_t* A_lo, const uint16_t* B
 int seqrec_topk_merge(const float* cand_v, const int32_t* cand_i, int n_lists, int64_t list_stride,
                       int32_t* topk_ids, float* topk_p, int64_t n_rows, int k, void* stream);
 
+/* ---- candidate scoring (csrc/candidates.cu): a given list of C item ids per row (id < 0 = pad) ---------------------
+ * z[n, j] = sum_h hout[n, h] . Wt[c - id_offset, h] (+ b_out[c - id_offset]) for c = cand[n * cand_ld + j], with the
+ * arithmetic of seqrec_target_logit (bit-equal to its zy for target c).  Wt (v_local, H) is the item-major copy of
+ * W_out (seqrec_transpose).  A pad, or an id outside [id_offset, id_offset + v_local) (another vocabulary shard's
+ * item), writes 0.0f: summed over the shards, exactly one addend is non-zero.  z is (n_rows, C); any C >= 1 and H. */
+#define SEQREC_MAX_CANDIDATES 1024
+int seqrec_candidate_logits(const float* hout, const float* Wt, const float* b_out, const int32_t* cand,
+                            int64_t cand_ld, float* z, int64_t n_rows, int C, int H, int id_offset, int v_local,
+                            void* stream);
+/* order of the candidates of each row from their logits z (n_rows, C) and ids cand (n_rows, C): score descending, then
+ * lower item id, then lower list position; pads last, reported as id -1 with score 0.  Positions < k go to out_ids /
+ * out_scores (n_rows, k); scores are z, or exp(z - m[n]) / s[n] when m and s are given.  out_ids NULL: no order.
+ * tgt / zy / rank (n_rows each): rank[n] = 1 + #{j : cand_j >= 0, cand_j != y, z_j > zy[n] or (z_j == zy[n] and
+ * cand_j < y)} for y = tgt[n] >= 0, 0 for y < 0.  tgt NULL: no rank. */
+int seqrec_candidate_order(const float* z, const int32_t* cand, int C, int64_t n_rows, const float* m, const float* s,
+                           int k, int32_t* out_ids, float* out_scores, const float* zy, const int32_t* tgt,
+                           int32_t* rank, void* stream);
+
 /* ---- history-feature / skip branches (csrc/dense_ops.cu): RNNFullModel's x_to_z / x_to_y / y_to_y (model.py:354-358,
  * :376-392) and NoRecurrenceModel (model.py:264-319).  logits z = hs.W + x.B + A[y_{t-1}] (+ biases) carry per-(token,
  * item) terms; the reference runs these models on small catalogs ((V,V) transition kernel A), so Z (N,V) is materialised.

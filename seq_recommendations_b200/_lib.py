@@ -65,6 +65,8 @@ SIGNATURES = {
     "seqrec_topk": [_p, _p, _p, _p, _p, _p, _p, _l, _i, _i, _i, _p],
     "seqrec_topk_tc": [_p] * 11 + [_l, _i, _i, _i, _i, _p],
     "seqrec_topk_merge": [_p, _p, _i, _l, _p, _p, _l, _i, _p],
+    "seqrec_candidate_logits": [_p, _p, _p, _p, _l, _p, _l, _i, _i, _i, _i, _p],
+    "seqrec_candidate_order": [_p, _p, _i, _l, _p, _p, _i, _p, _p, _p, _p, _p, _p],
     "seqrec_add_rows": [_p, _p, _p, _p, _l, _i, _p],
     "seqrec_softmax_rows_stats": [_p, _p, _p, _p, _p, _l, _i, _p],
     "seqrec_softmax_rows_dlogit": [_p, _p, _p, _p, _p, _l, _i, _p],

@@ -21,6 +21,7 @@ HBM layout (all fp32 unless noted; token n = t*B + b, time-major):
 """
 import contextlib
 import ctypes
+import gc
 import math
 import os
 
@@ -31,6 +32,7 @@ from . import _lib
 from ._lib import ACT, CELL, call, ptr
 from .dist import Comm, embedding_grad_mode
 from .gemm import gemm
+from .ranking import check_candidates
 from .state import RecurrentState
 
 GATES = {"simpleRNN": 1, "LSTM": 4, "GRU": 3}
@@ -250,6 +252,8 @@ class HotPath:
         self._w_version = 0
         self._split_version = -1
         self.Bt_hi = self.Bt_lo = self.Wb_hi = self.Wb_lo = None
+        self.Wt_items = None                      # fp32 W_out^T (V, H) of the candidate scorers, made on first use
+        self._wt_version = -1
         if weights is not None:
             self.set_weights(weights)
 
@@ -878,9 +882,17 @@ class HotPath:
                 return core(w)
             torch.cuda.synchronize(self.device)
             g = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(g):
-                self._format(w, grads=True)
-                w.graph_loss = core(w)
+            # no garbage collection inside the capture: collecting an unreachable work object frees its pinned staging
+            # buffers, and the host allocator's event queries then invalidate the capture
+            gc_was_on = gc.isenabled()
+            gc.disable()
+            try:
+                with torch.cuda.graph(g):
+                    self._format(w, grads=True)
+                    w.graph_loss = core(w)
+            finally:
+                if gc_was_on:
+                    gc.enable()
             w.graph, w.graph_key = g, key
         w.graph.replay()
         self._w_version += 1
@@ -1348,6 +1360,17 @@ class HotPath:
         """(n,) int32 rank of tgt[i] after session i's state, as target_rank_batch(last_step_only=True)."""
         return self._rank_scored(self._state_work(state, tgt), True)
 
+    def candidates_from_state(self, state, cand, k=None, probs=False):
+        """The candidate order after each session's state: (n,k) ids and scores, as candidates_batch(last_step_only=
+        True).  cand (n, C)."""
+        lists, k = self._candidate_lists(cand, (len(state),), k)
+        return self._candidates_scored(self._state_work(state), lists, False, k, bool(probs), True)
+
+    def candidate_rank_from_state(self, state, tgt, cand):
+        """(n,) int32 rank of tgt[i] among session i's candidates cand[i] after its state."""
+        lists, _ = self._candidate_lists(cand, (len(state),))
+        return self._candidates_scored(self._state_work(state, tgt), lists, True, None, False, True)
+
     # ------------------------------------------------------------------------------------------------ scoring
     # Every scorer: stage the batch and scan (_scan_batch; the *_from_state scorers build their (n, 1) problem with
     # _state_work instead), score every step or the last one (_target_prob, _rank_scored, _topk_scored: the only places
@@ -1534,3 +1557,92 @@ class HotPath:
         if last_step_only:
             return top_i, top_p
         return self._per_session(top_i, w), self._per_session(top_p, w)
+
+    # ------------------------------------------------------------------------------------------------ candidates
+    def candidates_batch(self, ids, cand, k=None, probs=False, last_step_only=True, x_dense=None, initial_state=None):
+        """Scores a given candidate list per session: cand (B, C) for the last step, (B, T, C) for every step; ids < 0
+        are pads.  Returns (ids int32, scores float32) of the first k (default C) entries of the order -- score
+        descending, then lower item id, then lower list position, pads last as (-1, 0) -- of shape (B, k) or (B, T, k).
+        Scores are the logits, or with probs=True the catalog softmax probabilities (one statistics pass).
+        initial_state: the sessions' RecurrentState the chunk continues (None = zeros)."""
+        B, T = (ids.shape if ids is not None else x_dense.shape[:2])
+        lists, k = self._candidate_lists(cand, (int(B),) if last_step_only else (int(B), int(T)), k)
+        w = self._scan_batch(ids, None, x_dense, initial_state)
+        return self._candidates_scored(w, lists, False, k, bool(probs), last_step_only)
+
+    def candidate_rank_batch(self, ids, tgt, cand, last_step_only=False, x_dense=None, initial_state=None):
+        """Rank of the true next item among the candidates, (B,T) int32 (cand (B, T, C)) or (B,) for the last step
+        (cand (B, C)): 1 + #{j : c_j >= 0, c_j != y, z_j > z_y or (z_j == z_y and c_j < y)}; 0 where y < 0."""
+        B, T = (ids.shape if ids is not None else x_dense.shape[:2])
+        lists, _ = self._candidate_lists(cand, (int(B),) if last_step_only else (int(B), int(T)))
+        w = self._scan_batch(ids, tgt, x_dense, initial_state)
+        return self._candidates_scored(w, lists, True, None, False, last_step_only)
+
+    def _candidate_lists(self, cand, lead, k=None):
+        """Validated candidate lists as a contiguous device int32 tensor (every id < 0 becomes the pad -1), and k."""
+        cand, _, k = check_candidates(cand, lead, self.V_total, k)
+        t = cand if isinstance(cand, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(cand))
+        return t.to(self.device).clamp(min=-1).to(torch.int32).contiguous(), k
+
+    def _stage_item_major(self):
+        """fp32 W_out^T (V, H): the candidate logits read one coalesced row per item instead of a strided column of
+        W_out.  Made on first use and again whenever the weights changed; V*H*4 bytes."""
+        if self._wt_version != self._w_version:
+            if self.Wt_items is None:
+                self.Wt_items = torch.empty((self.V, self.H), dtype=torch.float32, device=self.device)
+            call("seqrec_transpose", ptr(self.W_out), ptr(self.Wt_items), self.H, self.V, self.stream)
+            self._wt_version = self._w_version
+        return self.Wt_items
+
+    def _candidate_logits(self, rows, lists, id_offset):
+        """(n, C) logits of the lists (n, C) of global ids against this model's items (0 for pads and other shards)."""
+        n, C = lists.shape
+        z = torch.empty((n, C), dtype=torch.float32, device=self.device)
+        call("seqrec_candidate_logits", ptr(rows), ptr(self._stage_item_major()), ptr(self.b_out), ptr(lists), C, ptr(z),
+             n, C, self.H, int(id_offset), self.V, self.stream)
+        return z
+
+    def _candidates_scored(self, w, cand, tgt, k, probs, last_step_only):
+        """Candidate scoring of the rows of w.hout (all steps, or the last one).  cand: device int32 lists, (B, C) or
+        (B, T, C).  tgt True: the ranks of w's staged targets among them, (B,) or (B,T); else the first k entries of the
+        order, (ids, scores), with catalog probabilities when probs.  With a target the list is [y | candidates], so z_y
+        comes from the candidate arithmetic (and, on a vocabulary shard, from the same reduction)."""
+        C = cand.shape[-1]
+        lists = cand if last_step_only else cand.transpose(0, 1).reshape(w.N, C)       # time-major rows
+        m = s = None
+        if self.vocab_parallel:
+            comm = self.comm
+            y = (w.tgt[w.T - 1] if last_step_only else w.tgt.view(-1)) if tgt else None
+            scored = torch.cat([y[:, None], lists], 1) if tgt else lists
+            wg, _ = self._vp_gather(w, last_step_only, with_targets=False)
+            part = self._candidate_logits(wg.hout.view(wg.N, self.H), comm.all_gather_cat(scored), self.v_lo)
+            Z = torch.empty(scored.shape, dtype=torch.float32, device=self.device)
+            comm.reduce_scatter_sum(Z, part)                 # one non-zero addend per entry: the owner shard's logit
+            if probs:
+                self._vp_merge(wg, with_targets=False)
+                m, s = self._my_rows(wg.m), self._my_rows(wg.s)
+        else:
+            wt = self._last_step(w, with_targets=tgt) if last_step_only else w
+            rows = wt.hout.view(wt.N, self.H)
+            y = wt.tgt.view(-1) if tgt else None
+            Z = self._candidate_logits(rows, torch.cat([y[:, None], lists], 1) if tgt else lists, 0)
+            if probs:
+                if wt.tc["panel"]:
+                    _, m, s = self._wide_logits(rows)
+                else:
+                    self._forward_ce(wt, with_targets=False)
+                    m, s = wt.m, wt.s
+        n = lists.shape[0]
+        if tgt:
+            rank = torch.empty(n, dtype=torch.int32, device=self.device)
+            z, zy = Z[:, 1:].contiguous(), Z[:, 0].contiguous()
+            call("seqrec_candidate_order", ptr(z), ptr(lists), C, n, None, None, 0, None, None, ptr(zy), ptr(y),
+                 ptr(rank), self.stream)
+            return rank if last_step_only else self._per_session(rank, w)
+        out_i = torch.empty((n, k), dtype=torch.int32, device=self.device)
+        out_s = torch.empty((n, k), dtype=torch.float32, device=self.device)
+        call("seqrec_candidate_order", ptr(Z), ptr(lists), C, n, ptr(m), ptr(s), k, ptr(out_i), ptr(out_s), None, None,
+             None, self.stream)
+        if last_step_only:
+            return out_i, out_s
+        return self._per_session(out_i, w), self._per_session(out_s, w)

@@ -12,8 +12,8 @@ Adagrad kernels are the ones of the hot path; the dense products run on the tcge
 experiment scripts for these variants drive one device).
 
 Same public methods as engine.HotPath (train_batch / loss_batch / grad_batch / predict_batch / target_prob_batch /
-target_rank_batch / topk_batch / hidden_batch, get_weight / set_weight, trainable, set_optimizer), so model._Net drives
-either.
+target_rank_batch / topk_batch / candidates_batch / candidate_rank_batch / hidden_batch, get_weight / set_weight,
+trainable, set_optimizer), so model._Net drives either.
 """
 import ctypes
 
@@ -25,6 +25,7 @@ from ._lib import ACT, CELL, call, ptr
 from .dist import Comm
 from .engine import GATES, _align, _optimizer_spec
 from .gemm import gemm
+from .ranking import check_candidates
 
 NAMES = ["W_in", "U", "b", "W_toy", "b_out", "A", "a_bias"]
 
@@ -475,6 +476,49 @@ class DensePath:
             probs = probs[:, -1]
         order = torch.sort(probs, dim=-1, descending=True, stable=True)
         return order.indices[..., :k].to(torch.int32).contiguous(), order.values[..., :k].contiguous()
+
+    def candidates_batch(self, ids, cand, k=None, probs=False, last_step_only=True, x_dense=None):
+        """The candidate order of engine.HotPath.candidates_batch from the materialised logits."""
+        return self._candidates(ids, None, cand, k, probs, last_step_only, x_dense)
+
+    def candidate_rank_batch(self, ids, tgt, cand, last_step_only=False, x_dense=None):
+        """Rank among the candidates (engine.HotPath.candidate_rank_batch) from the materialised logits: with the list
+        arange(V) it is target_rank_batch."""
+        return self._candidates(ids, tgt, cand, None, False, last_step_only, x_dense)
+
+    def _candidates(self, ids, tgt, cand, k, probs, last_step_only, x_dense):
+        B, T = self._shape(ids, x_dense)
+        cand, C, k = check_candidates(cand, (B,) if last_step_only else (B, T), self.V, k)
+        cand = cand if isinstance(cand, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(cand))
+        cand = cand.to(self.device).clamp(min=-1).to(torch.int32)
+        lists = (cand if last_step_only else cand.transpose(0, 1).reshape(B * T, C)).contiguous()   # time-major rows
+        w = self.work(B, T)
+        self._stage(w, ids, tgt, x_dense)
+        self._forward_logits(w, training=False)
+        Z = w.Z.view(T, B, self.V)[T - 1] if last_step_only else w.Z
+        n = lists.shape[0]
+        # the logits seqrec_rows_rank ranks, gathered (small catalogs: plumbing)
+        z = torch.gather(Z, 1, lists.clamp(min=0).long()).masked_fill_(lists < 0, 0.0).contiguous()
+        st = self.stream
+        if tgt is not None:
+            y = (w.tgt[T - 1] if last_step_only else w.tgt.view(-1)).contiguous()
+            zy = torch.gather(Z, 1, y.clamp(min=0).long()[:, None])[:, 0].contiguous()
+            rank = torch.empty(n, dtype=torch.int32, device=self.device)
+            call("seqrec_candidate_order", ptr(z), ptr(lists), C, n, None, None, 0, None, None, ptr(zy), ptr(y),
+                 ptr(rank), st)
+            return rank if last_step_only else rank.view(T, B).t().contiguous()
+        m = s = None
+        if probs:
+            m = torch.empty(n, dtype=torch.float32, device=self.device)
+            s = torch.empty(n, dtype=torch.float32, device=self.device)
+            call("seqrec_softmax_rows_stats", ptr(Z.contiguous()), None, ptr(m), ptr(s), None, n, self.V, st)
+        out_i = torch.empty((n, k), dtype=torch.int32, device=self.device)
+        out_s = torch.empty((n, k), dtype=torch.float32, device=self.device)
+        call("seqrec_candidate_order", ptr(z), ptr(lists), C, n, ptr(m), ptr(s), k, ptr(out_i), ptr(out_s), None, None,
+             None, st)
+        if last_step_only:
+            return out_i, out_s
+        return (out_i.view(T, B, k).transpose(0, 1).contiguous(), out_s.view(T, B, k).transpose(0, 1).contiguous())
 
     def hidden_batch(self, ids, x_dense=None):
         if not self.cell:

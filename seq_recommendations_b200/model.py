@@ -592,6 +592,69 @@ class _Net(object):
             self.hot.comm.all_reduce_sum(sums)
         return metrics_from_sums(sums, ks)
 
+    # ---- candidate scoring (a given list of items per session) -------------------------------------------------------
+    def predict_candidates(self, x, candidates, k=None, probs=False, last_step_only=True, batch_size=1024,
+                           initial_state=None):
+        """How the model orders a given list of items per session: candidates (N, C) (last step) or (N, T, C) (every
+        step), a numpy array or a device tensor, ids < 0 pads.  Returns (ids int32, scores float32) numpy arrays of the
+        first k (default C) entries: score descending, then lower item id, then lower list position, pads last as
+        (-1, 0).  Scores are logits, or with probs=True the catalog softmax probabilities of predict_topk."""
+        ids, xd = self._inputs(x)
+        n = len(ids) if ids is not None else len(xd)
+        self._check_state(initial_state, n)
+        oi, os_ = [], []
+        for lo in range(0, n, batch_size):
+            hi = min(n, lo + batch_size)
+            i, d = self._slice(ids, xd, slice(lo, hi))
+            a, b = self.hot.candidates_batch(i, candidates[lo:hi], k=k, probs=probs, last_step_only=last_step_only,
+                                             x_dense=d, **self._state_kw(initial_state, lo, hi))
+            oi.append(a.cpu().numpy())
+            os_.append(b.cpu().numpy())
+        return np.concatenate(oi, axis=0), np.concatenate(os_, axis=0)
+
+    def _candidate_ranks(self, x, y, candidates, batch_size, last_step_only, initial_state=None):
+        ids, xd = self._inputs(x)
+        tgt = to_id_batch(y)
+        self._check_state(initial_state, len(tgt))
+        out = []
+        for lo in range(0, len(tgt), batch_size):
+            hi = min(len(tgt), lo + batch_size)
+            i, d = self._slice(ids, xd, slice(lo, hi))
+            out.append(self.hot.candidate_rank_batch(i, tgt[lo:hi], candidates[lo:hi], last_step_only=last_step_only,
+                                                     x_dense=d, **self._state_kw(initial_state, lo, hi)))
+        out = torch.cat(out, dim=0)
+        self.hot.check_errors()
+        return out
+
+    def predict_candidate_rank(self, x, y, candidates, last_step_only=False, batch_size=1024, device=False,
+                               initial_state=None):
+        """(N,T) int32 rank of the true next item among each step's candidates (N, T, C), or (N,) with last_step_only
+        (candidates (N, C)): 1 + the other candidates with a higher logit or an equal one and a lower id; y < 0 gives 0.
+        A list may or may not hold the target."""
+        out = self._candidate_ranks(x, y, candidates, batch_size, last_step_only, initial_state)
+        return out if device else out.cpu().numpy()
+
+    def predict_candidates_from_state(self, state, candidates, k=None, probs=False, batch_size=1024):
+        """predict_candidates after each session's state: candidates (n, C)."""
+        out = self._from_state(state, batch_size, lambda s, lo, hi: self.hot.candidates_from_state(
+            s, candidates[lo:hi], k=k, probs=probs))
+        return (np.concatenate([a.cpu().numpy() for a, _ in out]), np.concatenate([b.cpu().numpy() for _, b in out]))
+
+    def predict_candidate_rank_from_state(self, state, y, candidates, batch_size=1024, device=False):
+        """(n,) int32 rank of y[i] among candidates[i] after session i's state; y < 0 gives 0."""
+        t = self._next_ids(y, len(state))
+        out = torch.cat(self._from_state(state, batch_size, lambda s, lo, hi: self.hot.candidate_rank_from_state(
+            s, t[lo:hi], candidates[lo:hi])))
+        return out if device else out.cpu().numpy()
+
+    def evaluate_candidate_ranking(self, x, y, candidates, ks=(1, 5, 10, 20), last_step_only=False, batch_size=1024):
+        """evaluate_ranking over the ranks among the candidates (predict_candidate_rank)."""
+        ks = check_ks(ks)
+        sums = rank_sums(self._candidate_ranks(x, y, candidates, batch_size, last_step_only), ks)
+        if self.hot.comm.enabled:
+            self.hot.comm.all_reduce_sum(sums)
+        return metrics_from_sums(sums, ks)
+
     def hidden_states(self, x, batch_size=1024):
         ids, xd = self._inputs(x)
         n = len(ids) if ids is not None else len(xd)
@@ -692,6 +755,27 @@ class BaseRNNModel(BaseModel):
 
     def evaluate_ranking(self, x_test, y_test, ks=(1, 5, 10, 20), last_step_only=False, batch_size=1024):
         return self.model.evaluate_ranking(x_test, y_test, ks=ks, last_step_only=last_step_only, batch_size=batch_size)
+
+    def predict_candidates(self, x_test, candidates, k=None, probs=False, last_step_only=True, batch_size=1024,
+                           initial_state=None):
+        return self.model.predict_candidates(x_test, candidates, k=k, probs=probs, last_step_only=last_step_only,
+                                             batch_size=batch_size, initial_state=initial_state)
+
+    def predict_candidates_from_state(self, state, candidates, k=None, probs=False, batch_size=1024):
+        return self.model.predict_candidates_from_state(state, candidates, k=k, probs=probs, batch_size=batch_size)
+
+    def predict_candidate_rank(self, x_test, y_test, candidates, last_step_only=False, batch_size=1024,
+                               initial_state=None):
+        return self.model.predict_candidate_rank(x_test, y_test, candidates, last_step_only=last_step_only,
+                                                 batch_size=batch_size, initial_state=initial_state)
+
+    def predict_candidate_rank_from_state(self, state, y, candidates, batch_size=1024):
+        return self.model.predict_candidate_rank_from_state(state, y, candidates, batch_size=batch_size)
+
+    def evaluate_candidate_ranking(self, x_test, y_test, candidates, ks=(1, 5, 10, 20), last_step_only=False,
+                                   batch_size=1024):
+        return self.model.evaluate_candidate_ranking(x_test, y_test, candidates, ks=ks, last_step_only=last_step_only,
+                                                     batch_size=batch_size)
 
 
 def _glorot_uniform(rng, shape):

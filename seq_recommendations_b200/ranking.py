@@ -27,6 +27,39 @@ def check_ks(ks):
     return tuple(out)
 
 
+MAX_CANDIDATES = 1024          # SEQREC_MAX_CANDIDATES of include/seqrec_b200.h
+
+
+def check_candidates(candidates, lead, n_items, k=None):
+    """Validates the candidate lists of a scoring call: `candidates` (numpy array or torch tensor) of shape lead + (C,)
+    -- lead = (n,) for last-step scoring, (n, T) for every step -- holding integer item ids, id < 0 a pad, every id
+    < n_items, 1 <= C <= MAX_CANDIDATES; k (None = C) must lie in [1, C].  A device tensor's ids are checked with one
+    device reduction and one read.  Returns (candidates, C, k); raises ValueError."""
+    lead = tuple(int(v) for v in lead)
+    if isinstance(candidates, torch.Tensor):
+        integer = not (candidates.dtype.is_floating_point or candidates.dtype.is_complex or
+                       candidates.dtype == torch.bool)
+    else:
+        candidates = np.asarray(candidates)
+        integer = np.issubdtype(candidates.dtype, np.integer)
+    shape = tuple(int(v) for v in candidates.shape)
+    if len(shape) != len(lead) + 1 or shape[:-1] != lead:
+        raise ValueError("candidates must have shape %s + (C,), got %s" % (lead, shape))
+    if not integer:
+        raise ValueError("candidate ids must be integers, got %s" % (candidates.dtype,))
+    C = shape[-1]
+    if not 1 <= C <= MAX_CANDIDATES:
+        raise ValueError("a candidate list holds 1 to %d ids, got C = %d" % (MAX_CANDIDATES, C))
+    k = C if k is None else k
+    if isinstance(k, (bool, np.bool_)) or int(k) != k or not 1 <= int(k) <= C:
+        raise ValueError("k must be an integer in [1, C = %d], got %r" % (C, k))
+    if candidates.size if not isinstance(candidates, torch.Tensor) else candidates.numel():
+        top = int(candidates.max())
+        if top >= n_items:
+            raise ValueError("candidate id %d is outside the catalog (%d items)" % (top, n_items))
+    return candidates, C, int(k)
+
+
 def rank_sums(rank, ks):
     """(3 len(ks) + 3) float64 device tensor of seqrec_rank_metrics: per k {hits, sum 1/rank, sum 1/log2(rank+1)}, then
     the same sums without a cutoff ({n scored, sum 1/rank, ...}).  Sums, so that shards of the data can be added."""
