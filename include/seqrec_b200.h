@@ -319,6 +319,39 @@ int seqrec_candidate_order(const float* z, const int32_t* cand, int C, int64_t n
                            int k, int32_t* out_ids, float* out_scores, const float* zy, const int32_t* tgt,
                            int32_t* rank, void* stream);
 
+/* ---- sampled softmax with log-Q correction (csrc/sampled.cu) -----------------------------------------------------
+ * A training step draws S item ids with replacement from q and scores every token against its target y and those S
+ * shared items: with log Q(v) = log(S q(v)) and o_v = h . W_out[:, v] + b_out[v],
+ *     l_0 = o_y - log Q(y),  l_j = o_{s_j} - log Q(s_j) (removed where s_j == y),  loss = -l_0 + log sum_j exp(l_j).
+ * seqrec_sample_items: ids (S,) from draw i = state[0] + i of r_i = splitmix64(splitmix64(seed) ^ i): column
+ * c = ((r >> 32) * V) >> 32, kept if (uint32)r < thr[c], else alias[c] (a Vose alias table; thr and alias NULL =
+ * uniform).  state (2 x uint64) as for seqrec_dropout_mask_dev: advanced by S when the launch completes. */
+#define SEQREC_MAX_SAMPLED 32768
+int seqrec_sample_items(int32_t* ids, int S, const uint32_t* thr, const int32_t* alias, int V, uint64_t seed,
+                        uint64_t* state, void* stream);
+/* W_S (H, S) = W_out[:, ids] (W_out leading dimension ldw) and bias_S[j] = b_out[ids[j]] (b_out may be NULL = 0) minus
+ * logQ[ids[j]]; logQ (V,) = log(S q(v)).  A strided gather: S*H 32-byte sectors read. */
+int seqrec_gather_columns(const float* W_out, int64_t ldw, const float* b_out, const float* logQ, const int32_t* ids,
+                          int S, int H, float* W_S, float* bias_S, void* stream);
+/* one panel of materialised sampled logits Z (n_rows, S), Z = o + b - log Q of the sampled columns.  Per row n with
+ * target y = tgt[n] and mask[n] != 0: l_0 = zy[n] - logQ[y] (zy: the exact fp32 target logit, bias included), columns
+ * with ids[j] == y removed; ce[n] (may be NULL) = the row's loss, Z[n, j] <- p_j (0 on removed columns),
+ * g_tgt[n] = p_0 - 1.  Pad rows: Z, ce and g_tgt become 0.  loss_part[0] = sum of the rows' losses, deterministic (no
+ * float atomics).  S <= SEQREC_MAX_SAMPLED: the ids are held in shared memory for the accidental-hit test. */
+int seqrec_sampled_softmax_rows(float* Z, int S, const int32_t* ids, const float* zy, const int32_t* tgt,
+                                const float* logQ, const uint8_t* mask, float* ce, float* g_tgt, float* loss_part,
+                                int64_t n_rows, void* stream);
+/* the target column of each token: dh[n,:] += g_tgt[n] W_out[:, y_n], dW_out[:, y_n] += g_tgt[n] hs[n,:] (hs = hout, times
+ * hscale when not NULL) and db_out[y_n] += g_tgt[n]; dh, dW_out, db_out may each be NULL (frozen weights); pads
+ * (y_n < 0) are skipped.  Atomics. */
+int seqrec_target_columns(const float* hout, const float* hscale, const float* W_out, int64_t ldw, const int32_t* tgt,
+                          const float* g_tgt, float* dh, float* dW_out, float* db_out, int64_t n_tokens, int H,
+                          void* stream);
+/* dW_out[:, ids[j]] += dW_S[:, j] (dW_S (H, S)) and db_out[ids[j]] += db_S[j]; duplicate ids add up (atomics).  dW_out
+ * or db_out may be NULL. */
+int seqrec_scatter_add_columns(const float* dW_S, const float* db_S, const int32_t* ids, int S, int H, float* dW_out,
+                               int64_t ldw, float* db_out, void* stream);
+
 /* ---- history-feature / skip branches (csrc/dense_ops.cu): RNNFullModel's x_to_z / x_to_y / y_to_y (model.py:354-358,
  * :376-392) and NoRecurrenceModel (model.py:264-319).  logits z = hs.W + x.B + A[y_{t-1}] (+ biases) carry per-(token,
  * item) terms; the reference runs these models on small catalogs ((V,V) transition kernel A), so Z (N,V) is materialised.

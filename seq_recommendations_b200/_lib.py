@@ -67,6 +67,11 @@ SIGNATURES = {
     "seqrec_topk_merge": [_p, _p, _i, _l, _p, _p, _l, _i, _p],
     "seqrec_candidate_logits": [_p, _p, _p, _p, _l, _p, _l, _i, _i, _i, _i, _p],
     "seqrec_candidate_order": [_p, _p, _i, _l, _p, _p, _i, _p, _p, _p, _p, _p, _p],
+    "seqrec_sample_items": [_p, _i, _p, _p, _i, _u64, _p, _p],
+    "seqrec_gather_columns": [_p, _l, _p, _p, _p, _i, _i, _p, _p, _p],
+    "seqrec_sampled_softmax_rows": [_p, _i, _p, _p, _p, _p, _p, _p, _p, _p, _l, _p],
+    "seqrec_target_columns": [_p, _p, _p, _l, _p, _p, _p, _p, _p, _l, _i, _p],
+    "seqrec_scatter_add_columns": [_p, _p, _p, _i, _i, _p, _l, _p, _p],
     "seqrec_add_rows": [_p, _p, _p, _p, _l, _i, _p],
     "seqrec_softmax_rows_stats": [_p, _p, _p, _p, _p, _l, _i, _p],
     "seqrec_softmax_rows_dlogit": [_p, _p, _p, _p, _p, _l, _i, _p],

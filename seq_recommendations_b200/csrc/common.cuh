@@ -47,6 +47,15 @@ __device__ __forceinline__ float act_grad_from_y(float y) {
   return 1.0f;
 }
 
+// counter-based random stream of the dropout factors and the sampled-softmax draws: r_i = splitmix64(splitmix64(seed) ^
+// (offset + i)) -- reproducible and independent of the launch geometry
+__device__ __forceinline__ uint64_t splitmix64(uint64_t x) {
+  x += 0x9E3779B97F4A7C15ull;
+  x = (x ^ (x >> 30)) * 0xBF58476D1CE4E5B9ull;
+  x = (x ^ (x >> 27)) * 0x94D049BB133111EBull;
+  return x ^ (x >> 31);
+}
+
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);

@@ -324,13 +324,7 @@ extern "C" int seqrec_adam_table(float* p, float* g, float* m, float* v, int32_t
 // ---------------------------------------------------------------------------------------------------------------
 // Dropout factors.  Theano's MRG31k3p stream cannot be reproduced (SURVEY a5), so only the distribution is kept:
 // out = 0 with probability `rate`, else 1/(1-rate).  Counter-based (splitmix64 of seed, offset+i): reproducible and
-// independent of the launch geometry.
-__device__ __forceinline__ uint64_t splitmix64(uint64_t x) {
-  x += 0x9E3779B97F4A7C15ull;
-  x = (x ^ (x >> 30)) * 0xBF58476D1CE4E5B9ull;
-  x = (x ^ (x >> 27)) * 0x94D049BB133111EBull;
-  return x ^ (x >> 31);
-}
+// independent of the launch geometry (splitmix64: common.cuh).
 
 __global__ void __launch_bounds__(256)
 dropout_mask_kernel(float* __restrict__ out, int64_t n, float rate, uint64_t seed, uint64_t offset) {

@@ -29,6 +29,7 @@ import numpy as np
 import torch
 
 from . import _lib
+from . import losses
 from ._lib import ACT, CELL, call, ptr
 from .dist import Comm, embedding_grad_mode
 from .gemm import gemm
@@ -119,6 +120,38 @@ class _Work:
         self.pin_tgt = torch.empty((B, T), dtype=i32, pin_memory=True)
 
 
+class _Sampled:
+    """The S-sized operands of the sampled-softmax loss (HotPath.set_loss), allocated once per selection: the draw, the
+    sub-catalog W_S = W_out[:, ids] with its bias, their bf16 hi/lo images for the tensor-core GEMMs, the column
+    gradients, and the device tables of the sampler (alias table, log Q)."""
+
+    def __init__(self, hp, S, q):
+        dev, f32, bf = hp.device, torch.float32, torch.bfloat16
+        H, Hk = hp.H, hp.Hk
+        self.S = S
+        self.Sp = (S + 7) // 8 * 8
+        self.Sk = (S + 63) // 64 * 64
+        self.ids = torch.zeros(S, dtype=torch.int32, device=dev)
+        self.thr = self.alias = None
+        if q is not None:
+            thr, alias = losses.alias_table(q)
+            self.thr = torch.from_numpy(thr.view(np.int32)).to(dev)      # uint32 bits; the kernel reads them unsigned
+            self.alias = torch.from_numpy(alias).to(dev)
+        self.logq = torch.from_numpy(losses.log_q(S, q, hp.V)).to(dev)
+        self.W_S = torch.empty((H, S), dtype=f32, device=dev)
+        self.bias_S = torch.empty(S, dtype=f32, device=dev)
+        self.dW_S = torch.zeros((H, S), dtype=f32, device=dev)
+        self.db_S = torch.zeros(S, dtype=f32, device=dev)
+        self.Bt_hi = self.Bt_lo = self.Wb_hi = self.Wb_lo = None
+        if hp.tc_mode != "off" and S >= 256:
+            # zero padding of Hk / Sp is never written
+            self.Bt_hi = torch.zeros((S, Hk), dtype=bf, device=dev)
+            self.Wb_hi = torch.zeros((Hk, self.Sp), dtype=bf, device=dev)
+            if hp.tc_x3:
+                self.Bt_lo = torch.zeros((S, Hk), dtype=bf, device=dev)
+                self.Wb_lo = torch.zeros((Hk, self.Sp), dtype=bf, device=dev)
+
+
 class HotPath:
     def __init__(self, cell, act, in_dim, hidden, n_items, out_bias=False, input_kind="ids", weights=None,
                  device=None, comm=None, seed=0, tc="x3", vocab_parallel=False):
@@ -155,6 +188,12 @@ class HotPath:
         self.dropout_rec = 0.0                     # Keras recurrent_dropout (z -> z), model.py:346,351
         # identical seeds on every rank would draw identical dropout masks for different shards: fold the rank in
         self.seed = int(seed) * max(1, self.comm.world) + self.comm.rank
+        # the sampled-softmax draws use the UNFOLDED seed: every data-parallel rank draws the same ids, so a P-rank step
+        # equals the one-GPU step on the global batch.  Stream position on the device like rng_state
+        self.sample_seed = int(seed)
+        self.sample_state = torch.zeros(2, dtype=torch.int64, device=self.device)
+        self.sampled = None                        # _Sampled operands while set_loss("sampled_softmax") is selected
+        self._loss_version = 0
         # dropout stream position, on the device ([0] next offset, [1] kernel-internal ticket): a captured step draws
         # fresh factors at every replay
         self.rng_state = torch.zeros(2, dtype=torch.int64, device=self.device)
@@ -442,6 +481,29 @@ class HotPath:
             self.mU, self.mb, self.mW_out, self.mb_out = self._views(self.flat_m)
             self.mW_in = torch.zeros_like(self.aW_in)
         self.reset_optimizer_state()
+
+    def set_loss(self, kind="categorical_crossentropy", num_sampled=None, weights=None):
+        """The training objective of train_batch / grad_batch.  'categorical_crossentropy' (the default): the
+        full-catalog softmax of the reference.  'sampled_softmax': each step draws num_sampled item ids with replacement
+        from q (uniform, or weights / sum(weights) for V finite positive weights) and scores every token against its
+        target and those shared items with log-Q correction (losses.py has the definition).  Scorers, loss_batch and
+        evaluation always use the full softmax.  The sampler's stream position is not part of any checkpoint."""
+        if kind == "categorical_crossentropy":
+            if self.sampled is None:
+                return
+            self.sampled = None
+        elif kind == "sampled_softmax":
+            if self.vocab_parallel:
+                raise NotImplementedError("sampled softmax on a vocabulary-parallel model: train it data parallel")
+            S, q = losses.check_sampled(num_sampled, weights, self.V)
+            self.sampled = _Sampled(self, S, q)
+        else:
+            raise ValueError("loss must be 'categorical_crossentropy' or 'sampled_softmax', got %r" % (kind,))
+        self._loss_version += 1
+
+    def last_samples(self):
+        """The item ids the last sampled-softmax step drew, (S,) int32 numpy (None while the full softmax is selected)."""
+        return None if self.sampled is None else self.sampled.ids.cpu().numpy().copy()
 
     # ------------------------------------------------------------------------------------------------ batch ingest
     def _zero_step_scalars(self, grads=False):
@@ -765,6 +827,99 @@ class HotPath:
             torch.sum(parts, dim=0, keepdim=True, out=w.loss_sum)
         self._mark("misc")
 
+    def _ce_sampled(self, w):
+        """Training-step loss and gradients of the sampled softmax (set_loss): draw the S ids, gather the sub-catalog
+        W_S = W_out[:, ids] (bias b_out - log Q), then panels of  Z = hs . W_S + bias_S  (nb x S fp32, <= 256 MB) as in
+        _ce_panels: the rows kernel turns Z into p in place and leaves the target column's coefficient g_tgt; dh and
+        dW_S come from the same two GEMMs.  The target column's terms and the scatter of dW_S / db_S into the catalog
+        finish dh, dW_out and db_out.  Pads carry no loss and zero gradient rows."""
+        sp = self.sampled
+        st = self.stream
+        N, H, Hk, S = w.N, self.H, self.Hk, sp.S
+        x3 = 1 if self.tc_x3 else 0
+        tc = sp.Bt_hi is not None and N >= 128         # the `big` test of _tc_plan, with S in place of V
+        dW = self.dW_out if self.trainable["W_out"] else None
+        db = self.db_out if self.out_bias and self.trainable["b_out"] else None
+        self._mark("sample")
+        call("seqrec_sample_items", ptr(sp.ids), S, ptr(sp.thr), ptr(sp.alias), self.V, self.sample_seed,
+             ptr(self.sample_state), st)
+        call("seqrec_gather_columns", ptr(self.W_out), self.V, ptr(self.b_out), ptr(sp.logq), ptr(sp.ids), S, H,
+             ptr(sp.W_S), ptr(sp.bias_S), st)
+        hs_all = None
+        if tc:
+            call("seqrec_split_bf16_both", ptr(sp.W_S), None, ptr(sp.Wb_hi), ptr(sp.Wb_lo), ptr(sp.Bt_hi), ptr(sp.Bt_lo),
+                 H, S, sp.Sp, Hk, st)
+            call("seqrec_split_bf16_both", ptr(w.hout), ptr(w.hscale), ptr(w.A_hi), ptr(w.A_lo), ptr(w.Ht_hi),
+                 ptr(w.Ht_lo), N, H, Hk, w.Np, st)
+        else:
+            hs_all = w.hout.view(N, H) if w.hscale is None else w.hout.view(N, H) * w.hscale.view(N, H)
+        w.tc_operands_fresh = False
+        self._join()
+        self._mark("sampled_panels")
+        call("seqrec_target_logit", ptr(w.hout), ptr(w.hscale), ptr(self.W_out), ptr(self.b_out), ptr(w.tgt),
+             ptr(w.zy), N, H, self.V, None, None, st)
+        if dW is not None:
+            sp.dW_S.zero_()
+        if db is not None:
+            sp.db_S.zero_()
+        nb_max = max(128, min((N + 127) // 128 * 128, ((256 << 20) // (4 * S)) // 128 * 128))
+        b = getattr(w, "sampled_bufs", None)
+        if b is None or b["S"] != S or b["tc"] != tc or b["z"].shape[0] < nb_max:
+            bf = torch.bfloat16
+            b = dict(S=S, tc=tc, z=torch.empty((nb_max, S), dtype=torch.float32, device=self.device),
+                     g=torch.zeros(N, dtype=torch.float32, device=self.device))
+            if tc:
+                b["z_hi"] = torch.zeros((nb_max, sp.Sk), dtype=bf, device=self.device)
+                b["z_lo"] = torch.zeros((nb_max, sp.Sk), dtype=bf, device=self.device) if x3 else None
+                b["zt_hi"] = torch.zeros((S, nb_max), dtype=bf, device=self.device)
+                b["zt_lo"] = torch.zeros((S, nb_max), dtype=bf, device=self.device) if x3 else None
+            w.sampled_bufs = b
+        nbk = b["z"].shape[0]
+        n_panels = (N + nb_max - 1) // nb_max
+        parts = torch.zeros(n_panels, dtype=torch.float32, device=self.device)
+        el = 2                                                       # bytes per bf16
+        off = lambda t, elems: ctypes.c_void_p(t.data_ptr() + elems * el) if t is not None else None
+        for p, n0 in enumerate(range(0, N, nb_max)):
+            nb = min(nb_max, N - n0)
+            sl = slice(n0, n0 + nb)
+            Z = b["z"][:nb]
+            if tc:
+                call("seqrec_gemm_tc", off(w.A_hi, n0 * Hk), off(w.A_lo, n0 * Hk), ptr(sp.Bt_hi), ptr(sp.Bt_lo),
+                     ptr(sp.bias_S), ptr(Z), nb, S, Hk, Hk, Hk, S, 0, x3, st)
+            else:
+                call("seqrec_gemm_nn", ptr(hs_all[sl]), ptr(sp.W_S), ptr(sp.bias_S), ptr(Z), nb, S, H, 0, st)
+            call("seqrec_sampled_softmax_rows", ptr(Z), S, ptr(sp.ids), ptr(w.zy[sl]), ptr(w.tgt.view(-1)[sl]),
+                 ptr(sp.logq), ptr(w.mask.view(-1)[sl]), ptr(w.ce[sl]), ptr(b["g"][sl]), ptr(parts[p:p + 1]), nb, st)
+            if db is not None:
+                call("seqrec_colsum", ptr(Z), ptr(sp.db_S), nb, S, S, st)
+            dh = w.dh.view(N, H)[sl]
+            if tc:
+                call("seqrec_split_bf16_both", ptr(Z), None, ptr(b["z_hi"]), ptr(b["z_lo"]), ptr(b["zt_hi"]),
+                     ptr(b["zt_lo"]), nb, S, sp.Sk, nbk, st)
+                # dh[panel] = dZ . W_S^T   (K = S; the Wb_S operand is W_S K-major over the sampled columns)
+                call("seqrec_gemm_tc", ptr(b["z_hi"]), ptr(b["z_lo"]), ptr(sp.Wb_hi), ptr(sp.Wb_lo), None, ptr(dh), nb,
+                     H, S, sp.Sk, sp.Sp, H, 0, x3, st)
+                if dW is not None:
+                    # dW_S += hs[panel]^T . dZ   (K = the panel's tokens)
+                    call("seqrec_gemm_tc", off(w.Ht_hi, n0), off(w.Ht_lo, n0), ptr(b["zt_hi"]), ptr(b["zt_lo"]), None,
+                         ptr(sp.dW_S), H, S, nb, w.Np, nbk, S, 1, x3, st)
+            else:
+                call("seqrec_gemm_nt", ptr(Z), ptr(sp.W_S), ptr(dh), nb, H, S, S, S, H, 0, st)
+                if dW is not None:
+                    call("seqrec_gemm_tn_atomic", ptr(hs_all[sl]), ptr(Z), ptr(sp.dW_S), H, S, nb, st)
+        self._mark("sampled_columns")
+        call("seqrec_target_columns", ptr(w.hout), ptr(w.hscale), ptr(self.W_out), self.V, ptr(w.tgt), ptr(b["g"]),
+             ptr(w.dh), ptr(dW), ptr(db), N, H, st)
+        if w.hscale is not None:
+            w.dh.view(N, H).mul_(w.hscale.view(N, H))
+        if dW is not None or db is not None:
+            call("seqrec_scatter_add_columns", ptr(sp.dW_S), ptr(sp.db_S), ptr(sp.ids), S, H, ptr(dW), self.V, ptr(db),
+                 st)
+        torch.sum(parts, dim=0, keepdim=True, out=self.step_loss_sum)
+        self.n_valid_f.copy_(w.n_valid_i)
+        torch.div(self.step_loss_sum, self.n_valid_f, out=w.loss_mean)
+        self._mark("misc")
+
     def _ce_train_fused(self, w, zy_reduce=None, s_reduce=None):
         """Training-step logits pass on the tensor cores, fused: statistics + dh from ONE logits computation
         (seqrec_ce_tc_fused), finalize, dh finish.  Leaves w.m (= the per-token reference logit), w.s, w.coef ready for
@@ -903,7 +1058,8 @@ class HotPath:
         o = self.opt
         return (o["lr"], o["eps"], o["clipnorm"], tuple(sorted(self.trainable.items())), self.dropout_in,
                 self.dropout_out, self.dropout_rec, self.overlap, self.ce_fused, self.ce_compact, self.rnn_tc, self.wgrad_tc, self.tc_mode, self.tc_x3,
-                o["kind"], o["beta_1"], o["beta_2"], o["decay"])
+                o["kind"], o["beta_1"], o["beta_2"], o["decay"],
+                None if self.sampled is None else self.sampled.S, self._loss_version)
 
     def _train_core(self, w):
         """forward + backward + exchange + update on the staged batch (everything after the host->device copy).
@@ -924,7 +1080,8 @@ class HotPath:
         if ids_handle is not None and self.dp_serial:
             ids_handle.wait()
             ids_handle = None
-        if w.tc["fwd"]:
+        sampled = self.sampled is not None
+        if w.tc["fwd"] and not sampled:
             self._mark("stage_operands")
             with self._branch():                  # bf16 operands of the updated W_out, behind gather + scan
                 self._stage_weight_operands()
@@ -936,7 +1093,9 @@ class HotPath:
             ids_handle.wait()
             ids_handle = None
         fused = self.ce_fused and w.tc["bwd"]
-        if w.tc["panel"]:
+        if sampled:
+            self._ce_sampled(w)                   # loss, dh, dW_out and db_out of the sampled softmax
+        elif w.tc["panel"]:
             self._ce_panels(w, True, train=True, backward=True)      # statistics, dh and dW_out panel by panel
         elif fused:
             self._ce_train_fused(w)
@@ -945,7 +1104,7 @@ class HotPath:
 
         # ---- backward (the gradient buffer was cleared with the step scalars when the batch was staged)
         self._mark("ce_bwd")
-        if not w.tc["panel"]:
+        if not w.tc["panel"] and not sampled:
             self._backward_ce(w, dh=not fused)
         # dW_out / db_out are final here: their all-reduce runs on NCCL's stream behind the recurrent backward pass
         (o_u, s_u), (o_b, s_b) = self._seg[0], self._seg[1]
@@ -1277,13 +1436,16 @@ class HotPath:
         self._stage(w, ids, tgt, x_dense, grads=True)
         self._forward_hidden(w, training=True)
         use_fused = (self.ce_fused if fused is None else bool(fused)) and w.tc["bwd"]
-        if w.tc["panel"]:
+        sampled = self.sampled is not None
+        if sampled:
+            self._ce_sampled(w)
+        elif w.tc["panel"]:
             self._ce_panels(w, True, train=True, backward=True)
         elif use_fused:
             self._ce_train_fused(w)
         else:
             self._forward_ce(w, training=True, train=True)
-        if not w.tc["panel"]:
+        if not w.tc["panel"] and not sampled:
             self._backward_ce(w, dh=not use_fused)
         dh = w.dh.clone()
         self._rnn_backward(w)

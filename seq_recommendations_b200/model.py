@@ -19,6 +19,7 @@ import numpy as np
 import torch
 
 from . import callbacks as cb
+from . import losses
 from . import optimizers
 from .engine import GATES, HotPath
 from .engine_dense import DensePath
@@ -250,8 +251,20 @@ class _Net(object):
 
     # ---- compile -------------------------------------------------------------------------------------------------
     def compile(self, loss="categorical_crossentropy", optimizer="adam", metrics=None):
-        if loss != "categorical_crossentropy":
-            raise NotImplementedError("only categorical_crossentropy (experiments_methods.py:42) is built")
+        """loss: 'categorical_crossentropy' (experiments_methods.py:42), or losses.SampledSoftmax(...) on the recurrent
+        models of HotPath: training then minimises the sampled softmax and `fit`'s history `loss` is that loss, while
+        `val_loss`, `evaluate`, ValLossHistoryCut and RankingMetrics keep the full softmax of the reference."""
+        if isinstance(loss, losses.SampledSoftmax):
+            if not isinstance(self.hot, HotPath):
+                raise NotImplementedError("sampled softmax trains the recurrent models only; the skip-branch models and "
+                                          "NoRecurrenceModel add per-item terms to the full logits")
+            self.hot.set_loss("sampled_softmax", num_sampled=loss.num_sampled, weights=loss.weights)
+        elif loss == "categorical_crossentropy":
+            if isinstance(self.hot, HotPath):
+                self.hot.set_loss("categorical_crossentropy")
+        else:
+            raise NotImplementedError("loss: categorical_crossentropy (experiments_methods.py:42) or "
+                                      "losses.SampledSoftmax(...)")
         self.loss = loss
         self.optimizer = optimizers.resolve(optimizer)
         self.metrics_names = ["loss"] + [m for m in (metrics or []) if isinstance(m, str)]
